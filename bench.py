@@ -10,11 +10,16 @@ streaming pass over the rank's shard (one kernel) + -- when N > 1 -- the NCCL al
     python bench.py --gpus N --steps K --warmup W            # our arm
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm (oracle port)
 
-Prints ONE JSON line on rank 0.  Timing: CUDA events on the launching stream, barrier +
+Prints ONE JSON result line on rank 0 (stdout); the per-kernel tables (`extras`, `roofline_by_kernel`)
+follow as a second JSON line on stderr, which keeps the result line short enough for tools that
+keep only the end of a command's output.  Timing: CUDA events on the launching stream, barrier +
 synchronize on both sides, max over ranks.  Inputs (4 GB per rank) are far larger than the 126 MB
 L2, so no explicit flush is needed between iterations.
+
+    python bench.py --dump-outputs DIR   # also writes the normal equations of the last timed pass as DIR/*.npy
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -26,6 +31,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# leave the tree as build() left it: build() never imports oracle/, so without this the first bench run would write
+# oracle/__pycache__/ into a writable checkout
+sys.dont_write_bytecode = True
 
 METRIC = "points/sec project+Jacobian (fused project + analytical Jacobian + J^T J/J^T r)"
 UNIT = "points/s"
@@ -62,14 +70,20 @@ class ClockSampler:
         except OSError:
             self.proc = None
             return
+        atexit.register(self.stop)  # also when the run ends with an exception: nvidia-smi must not outlive bench.py
         def pump():
             for line in self.proc.stdout:
                 self.samples.append((time.time(), line.strip()))
         threading.Thread(target=pump, daemon=True).start()
 
     def stop(self):
-        if self.proc:
+        if self.proc and self.proc.poll() is None:
             self.proc.terminate()
+            try:
+                self.proc.wait(timeout=5)
+            except subprocess.TimeoutExpired:
+                self.proc.kill()
+                self.proc.wait()
 
     def summary(self, t0, t1):
         rows = []
@@ -93,7 +107,8 @@ class ClockSampler:
 
 def cpu_baseline(n_sample, min_seconds, nthreads):
     """The reference's algorithm for this path on the host: per-point residual + Jacobian
-    materialised, then J^T J / J^T r (oracle port; the Rust reference cannot be built here)."""
+    materialised, then J^T J / J^T r (oracle port; the Rust reference cannot be built here).
+    Returns points/s, passes, seconds and the normal equations (H, g, cost, n_valid) of the last pass."""
     from oracle import oracle as O
     O.build()
     kb = O.make_model(O.KB, KB_SAMPLE, 512, 512)
@@ -103,12 +118,12 @@ def cpu_baseline(n_sample, min_seconds, nthreads):
     O.linearize(ds, O.RES_PIXEL, xyz[:100000], uv[:100000], nthreads=nthreads)  # warm
     reps, t0 = 0, time.perf_counter()
     while True:
-        O.linearize(ds, O.RES_PIXEL, xyz, uv, nthreads=nthreads)
+        last = O.linearize(ds, O.RES_PIXEL, xyz, uv, nthreads=nthreads)
         reps += 1
         el = time.perf_counter() - t0
         if el >= min_seconds and reps >= 1:
             break
-    return n_sample * reps / el, reps, el
+    return n_sample * reps / el, reps, el, last
 
 
 def run_reference(args):
@@ -119,17 +134,16 @@ def run_reference(args):
     vals = []
     for _ in range(max(args.warmup, 0)):
         cpu_baseline(200_000, 0.0, 1)
-    t0 = time.perf_counter()
     for _ in range(args.steps):
-        v, _, _ = cpu_baseline(n_sample, 0.0, 1)
+        v, _, _, last = cpu_baseline(n_sample, 0.0, 1)
         vals.append(v)
-        if time.perf_counter() - t0 > 150:
-            break
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *last)
     value = float(np.median(vals))
     # beside it: the same port with OpenMP over every host core -- an upper bound the single-threaded reference does not have
     ncores = os.cpu_count() or 1
     try:
-        v_all, _, _ = cpu_baseline(n_sample, 2.0, ncores)
+        v_all, _, _, _ = cpu_baseline(n_sample, 2.0, ncores)
         all_cores = {"value": v_all, "cores": ncores, "note": "OpenMP over every host core: a generous upper bound the single-threaded reference does not have"}
     except Exception as e:  # pragma: no cover
         all_cores = {"error": str(e)}
@@ -235,6 +249,8 @@ def run_ours(args):
     # --- result of the last pass (also the d2h payload of the e2e path)
     ne = N.NormalEquations()
     ctx.check(lib.acm_linearize(ctx.handle, C.byref(cam), N.RESIDUAL_PIXEL, X.handle, UV.handle, C.byref(ne)))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *unpack_normal_equations(ne))
 
     # --- e2e: host AoS buffers (nalgebra layout, pinned) through acm_linearize_host, copies inside the timed region
     e2e = None
@@ -429,36 +445,39 @@ def run_ours(args):
                 "e2e": e2e, "lm_conversion": lm, "undistort_batch": und, "check": check,
                 "last_pass": {"n_valid": int(ne.n_valid), "cost": float(ne.cost), "H00": float(ne.H[0])}}
         if world == 1 and not args.no_cpu:
-            v1, reps, el = cpu_baseline(args.cpu_points, 10.0, 1)
+            v1, reps, el, _ = cpu_baseline(args.cpu_points, 10.0, 1)
             ncores = os.cpu_count() or 1
-            vall, _, _ = cpu_baseline(args.cpu_points, 3.0, ncores)
+            vall, _, _, _ = cpu_baseline(args.cpu_points, 3.0, ncores)
             line["cpu_baseline"] = {"value": v1, "unit": UNIT, "cores": 1, "kind": "port",
                                     "sample": f"{args.cpu_points} of the 100M correspondences x {reps} passes ({el:.1f} s); oracle C port (dense J, then J^T J), 1 thread like the single-threaded reference",
                                     "all_cores": {"value": vall, "cores": ncores, "note": "OpenMP over every host core: a generous upper bound the reference does not have"}}
+        detail = None
         if extras:
-            line["extras"] = extras
+            detail = {"extras": extras}
             # one roofline entry per fused kernel (model / residual), same definition as the headline entry
-            line["roofline_by_kernel"] = {k: {"bound": "hbm", "achieved": v["gb_s"], "peak": peak, "unit": "GB/s", "frac": v["gb_s"] / peak,
-                                              "frac_of_nominal_8TBs": v["gb_s"] / 8000.0, "ms": v["ms"]}
-                                          for k, v in extras.get("linearize_100M", {}).items()}
+            detail["roofline_by_kernel"] = {k: {"bound": "hbm", "achieved": v["gb_s"], "peak": peak, "unit": "GB/s", "frac": v["gb_s"] / peak,
+                                                "frac_of_nominal_8TBs": v["gb_s"] / 8000.0, "ms": v["ms"]}
+                                            for k, v in extras.get("linearize_100M", {}).items()}
             for k, v in extras.get("linearize_100M", {}).items():
                 if v.get("sustained_ms"):
                     gb = n * 40 / v["sustained_ms"] / 1e6
-                    line["roofline_by_kernel"][k]["sustained"] = {"achieved": gb, "frac": gb / peak, "ms": v["sustained_ms"], "sm_mhz": v.get("sm_mhz"),
-                                                                  "how": "the same launch back to back for ~0.4 s; `achieved` above is a 10-launch burst"}
+                    detail["roofline_by_kernel"][k]["sustained"] = {"achieved": gb, "frac": gb / peak, "ms": v["sustained_ms"], "sm_mhz": v.get("sm_mhz"),
+                                                                    "how": "the same launch back to back for ~0.4 s; `achieved` above is a 10-launch burst"}
             # the FP64-bound ones also against the FP64 issue rate at the clock sampled during a ~0.4 s loop of that kernel
             for k, ipp in FP64_INSTR_PER_POINT.items():
                 v = extras.get("linearize_100M", {}).get(k)
                 if v and v.get("sustained_ms") and v.get("sm_mhz"):
                     rate = ipp * n / (v["sustained_ms"] * 1e-3)
-                    line["roofline_by_kernel"][k]["fp64"] = {
+                    detail["roofline_by_kernel"][k]["fp64"] = {
                         "instr_per_point": ipp, "sustained_ms": v["sustained_ms"], "sustained_gb_s": n * 40 / v["sustained_ms"] / 1e6, "sm_mhz": v["sm_mhz"],
                         "issue_frac_at_clock": rate / (FP64_LANES_PER_CLOCK * v["sm_mhz"] * 1e6),
                         "note": "FP64 lane-instructions issued per second / (148 SMs x 64 lanes x sampled SM clock); ncu shows ~75 % as the practical ceiling (math-pipe throttle)"
                                 + ("" if world == 1 else "; N > 1: the time is the slowest rank's, the clock rank 0's, so the fraction is a lower bound")}
         if check is not None and not check.get("ok", False):
             line["check_failed"] = True
-        print(json.dumps(line))
+        if detail:
+            print(json.dumps(detail), file=sys.stderr, flush=True)
+        print(json.dumps(line), flush=True)
         if check is not None and not check.get("ok", False):
             raise SystemExit("bench.py: the sharded pass disagrees with the oracle (see \"check\")")
         if lm and lm.get("vs_oracle") and not lm["vs_oracle"].get("ok", False):
@@ -466,6 +485,22 @@ def run_ours(args):
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def unpack_normal_equations(ne):
+    """acm_normal_equations -> (H (P x P), g (P), cost, n_valid)."""
+    P = ne.n_params
+    return np.array(ne.H[:P * P]).reshape(P, P), np.array(ne.g[:P]), ne.cost, ne.n_valid
+
+
+def dump_outputs(out_dir, H, g, cost, n_valid):
+    """What a caller of the timed path receives (the normal equations H, g, cost, n_valid) as float64 DIR/<name>.npy.
+    The GPU arm reads them with one more acm_linearize on the same inputs after the timed steps: the pass reduces in a
+    fixed order (no float atomics), so that equals the last timed pass bit for bit (repeat runs are compared bit for bit
+    in tests/test_gpu_parity.py)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in {"H": H, "g": g, "cost": [cost], "n_valid": [n_valid]}.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def merge_extras(per_rank, n, world):
@@ -514,11 +549,10 @@ def oracle_check(acm, N, lib, ctx, kb, cam, rank, world, dist):
     if rank == 0:
         from oracle import oracle as O
         O.build()
-        P = ne.n_params
         xyz = O.synth_points3(CHECK_SEED, 0, CHECK_POINTS, COS_MAX, False)
         uv, _ = O.project(O.make_model(O.KB, KB_SAMPLE, 512, 512), xyz, nthreads=os.cpu_count() or 1)
         Ho, go, co, no = O.linearize(O.make_model(O.DS, DS_START, 512, 512), O.RES_PIXEL, xyz, uv, nthreads=os.cpu_count() or 1)
-        H = np.array(ne.H[:P * P]).reshape(P, P); g = np.array(ne.g[:P])
+        H, g, _, _ = unpack_normal_equations(ne)
         # entry-wise relative error against the scale of the entry's row/column (g and the off-diagonals cancel)
         dH = np.abs(H - Ho) / np.sqrt(np.outer(np.diag(Ho), np.diag(Ho)))
         dg = np.abs(g - go) / np.sqrt(np.diag(Ho) * 2.0 * co)
@@ -656,7 +690,10 @@ def main():
     ap.add_argument("--no-undistort", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true")
     ap.add_argument("--no-peer", action="store_true", help="N > 1: keep the NCCL all-reduce instead of the fused NVLink exchange")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the normal equations of the last timed pass as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

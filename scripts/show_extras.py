@@ -1,5 +1,10 @@
 import json, sys
-d = json.loads([l for l in open(sys.argv[1]) if l.startswith("{")][-1])
+# bench.py prints the result line on stdout and `extras` / `roofline_by_kernel` on stderr: pass both files (or one with both)
+d = {}
+for path in sys.argv[1:]:
+    for l in open(path):
+        if l.startswith("{"):
+            d.update(json.loads(l))
 print(f"headline {d['value']/1e9:.1f} Gpts/s  {d['roofline']['achieved']:.0f} GB/s frac {d['roofline']['frac']:.3f} clocks {d['clocks']}")
 for k, v in d["extras"]["linearize_100M"].items():
     print(f"  linearize {k:28s} {v['ms']:.3f} ms {v['gb_s']:.0f} GB/s")

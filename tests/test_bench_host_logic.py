@@ -1,8 +1,12 @@
 """Host logic of bench.py that runs without a GPU: the merge of the per-rank extras (maximum over ranks of every
-timing, throughput of all ranks over that time, rank-0 samples passed through) and the constants the roofline entries
-are built from."""
+timing, throughput of all ranks over that time, rank-0 samples passed through), the constants the roofline entries
+are built from, the --dump-outputs files and the argument checks."""
 import importlib.util
 import os
+import subprocess
+import sys
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -41,3 +45,45 @@ def test_fp64_issue_constants():
     frac = 102 * 100e9 / (b.FP64_LANES_PER_CLOCK * 1.5e9)
     assert 0.71 < frac < 0.73
     assert b.BYTES_PER_POINT == 40
+
+
+def test_dump_outputs_writes_the_normal_equations_as_float64(tmp_path):
+    from apex_camera_models_b200 import _native as N
+    b = _bench()
+    ne = N.NormalEquations()
+    ne.n_params = 6
+    for i in range(36):
+        ne.H[i] = 0.5 * i
+    for i in range(6):
+        ne.g[i] = -1.0 - i
+    ne.cost, ne.n_valid = 12.25, 99_999_937
+    b.dump_outputs(str(tmp_path / "out"), *b.unpack_normal_equations(ne))
+    got = {p.stem: np.load(p) for p in (tmp_path / "out").iterdir()}
+    assert set(got) == {"H", "g", "cost", "n_valid"}
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert np.array_equal(got["H"], 0.5 * np.arange(36.0).reshape(6, 6))
+    assert np.array_equal(got["g"], -1.0 - np.arange(6.0))
+    assert got["cost"].tolist() == [12.25] and got["n_valid"].tolist() == [99_999_937.0]
+
+
+def test_steps_below_one_is_refused():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True)
+    assert r.returncode == 2 and "--steps must be at least 1" in r.stderr
+
+
+def test_reference_arm_runs_exactly_the_requested_steps_and_dumps_its_last_pass(tmp_path, O):
+    """--impl reference on the host: the JSON line reports the requested step count and --dump-outputs holds the normal
+    equations of the oracle's pass over the arm's seeded 10 M-point sample."""
+    import json
+    b = _bench()
+    out = tmp_path / "ref"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "1",
+                        "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert line["impl"] == "reference" and line["steps"] == 2
+    xyz = O.synth_points3(b.SEED, 0, 10_000_000, b.COS_MAX, False)
+    uv, _ = O.project(O.make_model(O.KB, b.KB_SAMPLE, 512, 512), xyz, nthreads=os.cpu_count() or 1)
+    H, g, cost, nv = O.linearize(O.make_model(O.DS, b.DS_START, 512, 512), O.RES_PIXEL, xyz, uv, nthreads=1)
+    assert np.array_equal(np.load(out / "H.npy"), H) and np.array_equal(np.load(out / "g.npy"), g)
+    assert np.load(out / "cost.npy").tolist() == [cost] and np.load(out / "n_valid.npy").tolist() == [float(nv)]
