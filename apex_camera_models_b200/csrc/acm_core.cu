@@ -702,8 +702,10 @@ static int32_t host_map(acm_ctx* ctx, const acm_camera* cam, const double* in_ao
         // scalar / small-batch calls (the trait's project(&p)): mapped pinned staging owned by the context, ONE kernel that
         // reads and writes host memory directly.  Single-block batches (n <= 128) do not even synchronise the stream: the
         // kernel publishes a sequence number in the staging area when its results are out and the host spins on it.
+        // staging layout, in doubles of ACM_SMALL_BATCH points: input [0, 3N), output [3N, 6N) (a ray takes 3), status bytes
+        // at 6N, the sequence flag after them
         const size_t in_dim = is_project ? 3 : 2, out_dim = is_project ? 2 : 3;
-        const size_t flag_off = (size_t)ACM_SMALL_BATCH * (5 * sizeof(double) + 8);
+        const size_t flag_off = (size_t)ACM_SMALL_BATCH * (6 * sizeof(double) + 8);
         if (!ctx->h_small) {
             ACM_CUDA(ctx, cudaHostAlloc(&ctx->h_small, flag_off + 64, cudaHostAllocMapped));
             ACM_CUDA(ctx, cudaHostGetDevicePointer(&ctx->d_small_alias, ctx->h_small, 0));
@@ -712,13 +714,13 @@ static int32_t host_map(acm_ctx* ctx, const acm_camera* cam, const double* in_ao
         }
         double* h_in = static_cast<double*>(ctx->h_small);
         double* h_out = h_in + 3 * (size_t)ACM_SMALL_BATCH;
-        uint8_t* h_st = reinterpret_cast<uint8_t*>(h_in + 5 * (size_t)ACM_SMALL_BATCH);
+        uint8_t* h_st = reinterpret_cast<uint8_t*>(h_in + 6 * (size_t)ACM_SMALL_BATCH);
         volatile unsigned long long* h_flag = reinterpret_cast<volatile unsigned long long*>(static_cast<char*>(ctx->h_small) + flag_off);
         char* d_base = static_cast<char*>(ctx->d_small_alias);
         double* d_in = reinterpret_cast<double*>(d_base);
         memcpy(h_in, in_aos, n * in_dim * sizeof(double));
         const unsigned long long seq = ++ctx->small_seq;
-        int32_t rcs = acm_small_map(ctx, cam, d_in, d_in + 3 * (size_t)ACM_SMALL_BATCH, reinterpret_cast<uint8_t*>(d_in + 5 * (size_t)ACM_SMALL_BATCH),
+        int32_t rcs = acm_small_map(ctx, cam, d_in, d_in + 3 * (size_t)ACM_SMALL_BATCH, reinterpret_cast<uint8_t*>(d_in + 6 * (size_t)ACM_SMALL_BATCH),
                                     (int)n, is_project, reinterpret_cast<unsigned long long*>(d_base + flag_off), seq);
         if (rcs) return rcs;
         bool done = false;

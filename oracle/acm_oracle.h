@@ -57,6 +57,9 @@ int orc_project_nobounds(const orc_model* m, const double X[3], double uv[2]);
 int orc_project_jacobian(const orc_model* m, const double X[3], double uv[2], double* J);
 /* 2x3 Jacobian of (u,v) w.r.t. the 3-D point, row-major Jx[2][3]; returns status (nobounds) */
 int orc_project_point_jacobian(const orc_model* m, const double X[3], double uv[2], double Jx[6]);
+/* batch forms of the two above over AoS points (J: n x 2 x P, resp. n x 2 x 3 row-major), like orc_project_batch */
+void orc_project_jacobian_batch(const orc_model* m, const double* xyz, size_t n, double* uv, double* J, uint8_t* status, int nthreads);
+void orc_project_point_jacobian_batch(const orc_model* m, const double* xyz, size_t n, double* uv, double* J, uint8_t* status, int nthreads);
 /* residual (2) and its 2xP Jacobian for either residual kind; returns status (nobounds) */
 int orc_residual_jacobian(const orc_model* m, int kind, const double X[3], const double uv_obs[2], double r[2], double* J);
 

@@ -179,6 +179,27 @@ int orc_residual_jacobian(const orc_model* m, int kind, const double X[3], const
     return ORC_OK;
 }
 
+/* batch forms of the two Jacobians over AoS points, mirroring orc_project_batch: uv (n x 2), status (n) and
+ * J row-major per point -- (n x 2 x P) for the parameter Jacobian, (n x 2 x 3) for the point Jacobian */
+void orc_project_jacobian_batch(const orc_model* m, const double* xyz, size_t n, double* uv, double* J, uint8_t* status, int nthreads) {
+    const size_t P = (size_t)m->n_params;
+    (void)nthreads;
+#ifdef _OPENMP
+#pragma omp parallel for schedule(static) num_threads(nthreads > 0 ? nthreads : 1)
+#endif
+    for (long long i = 0; i < (long long)n; ++i)
+        status[i] = (uint8_t)orc_project_jacobian(m, xyz + 3 * i, uv + 2 * i, J + 2 * P * (size_t)i);
+}
+
+void orc_project_point_jacobian_batch(const orc_model* m, const double* xyz, size_t n, double* uv, double* J, uint8_t* status, int nthreads) {
+    (void)nthreads;
+#ifdef _OPENMP
+#pragma omp parallel for schedule(static) num_threads(nthreads > 0 ? nthreads : 1)
+#endif
+    for (long long i = 0; i < (long long)n; ++i)
+        status[i] = (uint8_t)orc_project_point_jacobian(m, xyz + 3 * i, uv + 2 * i, J + 6 * (size_t)i);
+}
+
 /* Dense path: materialise r and J for the chunk, then form J^T J and J^T r.  This is what the
  * reference's generic solver does (SURVEY.md 8a row a18) and is the timed CPU baseline. */
 static void linearize_chunk(const orc_model* m, int kind, const double* xyz, const double* uv, size_t n,

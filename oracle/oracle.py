@@ -71,6 +71,9 @@ def lib():
         L.orc_unproject_batch.argtypes = [mp, dp, C.c_size_t, dp, u8p, C.c_int]; L.orc_unproject_batch.restype = None
         L.orc_project_jacobian.argtypes = [mp, dp, dp, dp]; L.orc_project_jacobian.restype = C.c_int
         L.orc_project_point_jacobian.argtypes = [mp, dp, dp, dp]; L.orc_project_point_jacobian.restype = C.c_int
+        L.orc_project_jacobian_batch.argtypes = [mp, dp, C.c_size_t, dp, dp, u8p, C.c_int]; L.orc_project_jacobian_batch.restype = None
+        L.orc_project_point_jacobian_batch.argtypes = [mp, dp, C.c_size_t, dp, dp, u8p, C.c_int]
+        L.orc_project_point_jacobian_batch.restype = None
         L.orc_residual_jacobian.argtypes = [mp, C.c_int, dp, dp, dp, dp]; L.orc_residual_jacobian.restype = C.c_int
         L.orc_linearize.argtypes = [mp, C.c_int, dp, dp, C.c_size_t, dp, dp, dp, C.POINTER(C.c_uint64), C.c_int]
         L.orc_linearize.restype = C.c_int
@@ -159,6 +162,22 @@ def project_point_jacobian1(m: Model, X):
     X = np.ascontiguousarray(X, dtype=np.float64); uv = np.empty(2); J = np.zeros((2, 3))
     st = lib().orc_project_point_jacobian(C.byref(m), _dp(X), _dp(uv), _dp(J))
     return st, uv, J
+
+
+def project_jacobian(m: Model, xyz: np.ndarray, nthreads: int = 1):
+    """Batch form of project_jacobian1: xyz (N,3) -> (uv (N,2), J (N,2,P), status (N,) uint8)."""
+    xyz = np.ascontiguousarray(xyz, dtype=np.float64); n = xyz.shape[0]
+    uv = np.empty((n, 2)); J = np.empty((n, 2, m.n_params)); st = np.empty(n, dtype=np.uint8)
+    lib().orc_project_jacobian_batch(C.byref(m), _dp(xyz), n, _dp(uv), _dp(J), _u8p(st), nthreads)
+    return uv, J, st
+
+
+def project_point_jacobian(m: Model, xyz: np.ndarray, nthreads: int = 1):
+    """Batch form of project_point_jacobian1: xyz (N,3) -> (uv (N,2), J (N,2,3), status (N,) uint8)."""
+    xyz = np.ascontiguousarray(xyz, dtype=np.float64); n = xyz.shape[0]
+    uv = np.empty((n, 2)); J = np.empty((n, 2, 3)); st = np.empty(n, dtype=np.uint8)
+    lib().orc_project_point_jacobian_batch(C.byref(m), _dp(xyz), n, _dp(uv), _dp(J), _u8p(st), nthreads)
+    return uv, J, st
 
 
 def residual_jacobian1(m: Model, kind: int, X, uv_obs):
