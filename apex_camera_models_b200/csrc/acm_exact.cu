@@ -123,17 +123,11 @@ __global__ void __launch_bounds__(256, (PuStream<PU_PROJECT, M>::PIPE ? 3 : 0)) 
 // ---------------------------------------------------------------------------------------
 // resident 256-thread blocks per SM the unproject kernel is compiled for (register cap): 3 with the pipelined stream; the Newton
 // models are bound by the latency of their dependent chains: RadTan gains 2.6 % from a 4th block (64 registers), Kannala-Brandt
-// nothing (profiles/r02_ab_unproj_occ.log; -DACM_EXP_UNPROJ_MINB_RT / _KB: A/B aid)
-#ifndef ACM_EXP_UNPROJ_MINB_RT
-#define ACM_EXP_UNPROJ_MINB_RT 4
-#endif
-#ifndef ACM_EXP_UNPROJ_MINB_KB
-#define ACM_EXP_UNPROJ_MINB_KB 3
-#endif
+// nothing (profiles/r02_ab_unproj_occ.log)
 template <int M> struct UnprojBounds { static constexpr int MINB = PuStream<PU_UNPROJECT, M>::PIPE ? 3 : 0; };
-template <> struct UnprojBounds<ACM_MODEL_RADTAN> { static constexpr int MINB = ACM_EXP_UNPROJ_MINB_RT; };
-template <> struct UnprojBounds<ACM_MODEL_KANNALA_BRANDT> { static constexpr int MINB = ACM_EXP_UNPROJ_MINB_KB; };
-template <int M, typename T, bool IEEE = ACM_TAIL_DEFAULT>
+template <> struct UnprojBounds<ACM_MODEL_RADTAN> { static constexpr int MINB = 4; };
+template <> struct UnprojBounds<ACM_MODEL_KANNALA_BRANDT> { static constexpr int MINB = 3; };
+template <int M, typename T, bool IEEE = false>
 __global__ void __launch_bounds__(256, UnprojBounds<M>::MINB) unproject_kernel(const __grid_constant__ CamParams c, const T* __restrict__ U,
                                                         const T* __restrict__ V, T* __restrict__ X, T* __restrict__ Y,
                                                         T* __restrict__ Z, uint8_t* __restrict__ S, size_t n) {
@@ -197,7 +191,7 @@ static int32_t launch_project(acm_ctx* ctx, const CamParams& c, const acm_points
     return ACM_OK;
 }
 
-template <int M, typename T, bool IEEE = ACM_TAIL_DEFAULT>
+template <int M, typename T, bool IEEE = false>
 static int32_t launch_unproject(acm_ctx* ctx, const CamParams& c, const acm_points* uv, acm_points* xyz, uint8_t* st) {
     const size_t n = uv->n;
     if (n == 0) return ACM_OK;
@@ -380,7 +374,7 @@ __device__ __forceinline__ void small_map_point(const CamParams& c, const double
         out[2 * i] = u; out[2 * i + 1] = v;
     } else {
         double x, y, z;
-        st = CamModel<M>::template unproject<ACM_TAIL_DEFAULT>(c, in[2 * i], in[2 * i + 1], x, y, z);
+        st = CamModel<M>::template unproject<false>(c, in[2 * i], in[2 * i + 1], x, y, z);
         if (st != ACM_POINT_OK) x = y = z = acm_nan();
         out[3 * i] = x; out[3 * i + 1] = y; out[3 * i + 2] = z;
     }
@@ -982,10 +976,9 @@ extern "C" int32_t acm_undistort_rgb8(acm_ctx* ctx, const acm_camera* cam, const
     const int W = (int)cam->width, H = (int)cam->height;
     dim3 grid((W + 1023) / 1024, H);
     const bool aligned = ((reinterpret_cast<uintptr_t>(d_in) & 3) == 0) && ((reinterpret_cast<uintptr_t>(d_out) & 3) == 0) && (W % 4 == 0);
-    const bool tma_ok = ((reinterpret_cast<uintptr_t>(d_in) & 15) == 0) && (W % 16 == 0) && n_frames < 0x7fffffffULL && !getenv("ACM_UNDISTORT_NO_TMA");
+    const bool tma_ok = ((reinterpret_cast<uintptr_t>(d_in) & 15) == 0) && (W % 16 == 0) && n_frames < 0x7fffffffULL;
     UndMaps map;
-    const bool generic = getenv("ACM_UNDISTORT_GENERIC") != nullptr;
-    bool have_maps = aligned && !generic && tma_ok;
+    bool have_maps = aligned && tma_ok;
     for (int r = UND_MIN_ROWS; have_maps && r <= UND_BOX_ROWS; ++r) have_maps = make_frame_tensor_map(&map.m[r - UND_MIN_ROWS], d_in, W, H, n_frames, r);
     if (have_maps) {
         dim3 fgrid((W + 63) / 64, (H + 15) / 16);
@@ -1008,7 +1001,7 @@ extern "C" int32_t acm_undistort_rgb8(acm_ctx* ctx, const acm_camera* cam, const
             ACM_CHECK_LAUNCH(ctx);
             ACM_DISPATCH_MODEL(cam->model, (undistort_list_generic_kernel<M><<<ctx->sm_count * 3, 256, 0, ctx->stream>>>(c, t[0], t[1], t[2], t[3], d_in, d_out, W, H, n_frames, interpolation, d_list, d_count)))
         }
-    } else if (interpolation == ACM_INTERP_BILINEAR && aligned && !generic) {
+    } else if (interpolation == ACM_INTERP_BILINEAR && aligned) {
         dim3 fgrid((W + 63) / 64, (H + 15) / 16);
         ACM_DISPATCH_MODEL(cam->model, (undistort_bilinear_fast_kernel<M><<<fgrid, 256, 0, ctx->stream>>>(c, t[0], t[1], t[2], t[3], d_in, d_out, W, H, n_frames)))
     } else {

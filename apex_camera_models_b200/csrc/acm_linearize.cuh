@@ -30,27 +30,17 @@
 // (Only used where the tolerance is 1e-9 relative -- never in the bit-exact project kernels.)
 // ---------------------------------------------------------------------------------------
 __device__ __forceinline__ double fast_rcp(double a) { return acm_rcp(a); }
-__device__ __forceinline__ double fast_rsqrt(double a) {
-    double y;
-    asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(a));
-    const double h = 0.5 * a;
-    y = y * fma(-h, y * y, 1.5);   // 2^-23 -> ~2^-45
-    return y * fma(-h, y * y, 1.5);  // -> full double precision
-}
 // sqrt(a) with 1/sqrt(a) as a by-product.
 // REFINE_INV = false: one Newton step on the seed (inv accurate to ~2^-44, enough for a Jacobian
 // entry), then a Heron correction with the exact fma residual, which squares the error: s <= 1 ulp.
 // REFINE_INV = true (inv feeds a residual): two coupled Goldschmidt iterations on g ~ sqrt(a),
 // h ~ 1/(2 sqrt(a)) -- r = 1/2 - g h, g += g r, h += h r -- take both from 2^-23 to full precision in
 // 2 DMUL + 6 DFMA + 1 DADD (the separate Newton + Heron form needed 11).
-#ifndef ACM_AB_OLD_SQRT
-#define ACM_AB_OLD_SQRT 0
-#endif
 template <bool REFINE_INV = false>
 __device__ __forceinline__ double fast_sqrt(double a, double& inv) {
     double y;
     asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(a));
-    if (REFINE_INV && !ACM_AB_OLD_SQRT) {
+    if (REFINE_INV) {
         double g = a * y, h = 0.5 * y;
         double r = fma(-g, h, 0.5);
         g = fma(g, r, g); h = fma(h, r, h);
@@ -82,16 +72,7 @@ struct LinParams {
     double fx, fy, cx, cy;
     double d[5];
     double k0;  // validity constant: UCM w, EUCM (a-1)/(2a-1), DS w2, FOV tan(w/2)
-    unsigned atab;  // shared-memory address of the atan table (acm_atan_tab_init), set by the streaming kernel for KB / FOV
 };
-
-// -DACM_LIN_ATAN_TAB=1 builds the KB / FOV passes with the table-driven atan2 of acm_math.cuh (16 FP64 instructions instead
-// of 25).  Measured SLOWER on the same box (KB 4453 vs 4780 GB/s, FOV 4920 vs 5245): the index computation, the LDS and
-// the clamps add ~18 non-FP64 instructions per point to loops whose issue slots are as full as their FP64 pipe
-// (KB: 362 instructions per trip against 2 x 186 FP64 issue cycles).  Kept as an A/B aid.
-#ifndef ACM_LIN_ATAN_TAB
-#define ACM_LIN_ATAN_TAB 0
-#endif
 
 __host__ __device__ inline void lin_derive(int model, LinParams& p) {
     const double alpha = p.d[0];
@@ -266,8 +247,6 @@ template <> struct Lin<ACM_MODEL_DOUBLE_SPHERE, ACM_RESIDUAL_ALGEBRAIC> : LinUni
 
 template <> struct Lin<ACM_MODEL_FOV, ACM_RESIDUAL_PIXEL> {
     static constexpr int ND = 1; static constexpr bool UNIT_C = true;
-    // TAB: table-driven atan2 (needs p.atab: only the streaming kernel provides it)
-    template <bool TAB = false>
     static __device__ __forceinline__ bool eval(const LinParams& p, double x, double y, double z, double u, double v,
                                                 double& ru, double& rv, double* au, double* av) {
         // branch-free: the r2 < sqrt(EPS) case (fov.rs:203-207, constant rd) is a select at the end
@@ -280,7 +259,7 @@ template <> struct Lin<ACM_MODEL_FOV, ACM_RESIDUAL_PIXEL> {
         const double r2s = small ? 1.0 : r2;
         double ir;
         const double r = fast_sqrt<true>(r2s, ir);
-        const double a = TAB ? acm_atan2_q1_tab(t2 * r, z, p.atab) : fast_atan2_q1(t2 * r, z);
+        const double a = fast_atan2_q1(t2 * r, z);
         const double da = z * r * tt1 * fast_rcp(fma(t2 * t2, r2s, z * z));
         const double irw = iw * ir;
         double rd = a * irw;
@@ -343,46 +322,6 @@ __device__ __forceinline__ void lin_accumulate_masked(double* acc, bool ok, doub
     acc[L::COUNT] += ok ? 1.0 : 0.0;
 }
 
-template <int ND, bool UNIT_C>
-__device__ __forceinline__ void lin_accumulate(double* acc, double ru, double rv, const double* au, const double* av) {
-    using L = AccLayout<ND>;
-    acc[L::HFF + 0] = fma(au[0], au[0], acc[L::HFF + 0]);
-    acc[L::HFF + 1] = fma(av[0], av[0], acc[L::HFF + 1]);
-    acc[L::GF + 0] = fma(au[0], ru, acc[L::GF + 0]);
-    acc[L::GF + 1] = fma(av[0], rv, acc[L::GF + 1]);
-    if (UNIT_C) {
-        acc[L::HFC + 0] += au[0];
-        acc[L::HFC + 1] += av[0];
-        acc[L::GC + 0] += ru;
-        acc[L::GC + 1] += rv;
-    } else {
-        acc[L::HFC + 0] = fma(au[0], au[1], acc[L::HFC + 0]);
-        acc[L::HFC + 1] = fma(av[0], av[1], acc[L::HFC + 1]);
-        acc[L::HCC + 0] = fma(au[1], au[1], acc[L::HCC + 0]);
-        acc[L::HCC + 1] = fma(av[1], av[1], acc[L::HCC + 1]);
-        acc[L::GC + 0] = fma(au[1], ru, acc[L::GC + 0]);
-        acc[L::GC + 1] = fma(av[1], rv, acc[L::GC + 1]);
-    }
-#pragma unroll
-    for (int k = 0; k < ND; ++k) {
-        acc[L::HFD + k] = fma(au[0], au[2 + k], acc[L::HFD + k]);
-        acc[L::HFD + ND + k] = fma(av[0], av[2 + k], acc[L::HFD + ND + k]);
-        if (UNIT_C) {
-            acc[L::HCD + k] += au[2 + k];
-            acc[L::HCD + ND + k] += av[2 + k];
-        } else {
-            acc[L::HCD + k] = fma(au[1], au[2 + k], acc[L::HCD + k]);
-            acc[L::HCD + ND + k] = fma(av[1], av[2 + k], acc[L::HCD + ND + k]);
-        }
-        acc[L::GD + k] = fma(au[2 + k], ru, fma(av[2 + k], rv, acc[L::GD + k]));
-#pragma unroll
-        for (int j = 0; j <= k; ++j)
-            acc[L::HDD + L::tri(j, k)] = fma(au[2 + j], au[2 + k], fma(av[2 + j], av[2 + k], acc[L::HDD + L::tri(j, k)]));
-    }
-    acc[L::COST] = fma(ru, ru, fma(rv, rv, acc[L::COST]));
-    acc[L::COUNT] += 1.0;
-}
-
 // Reduced accumulator vector -> dense symmetric H (P x P), g, cost, count.
 // FULL = false (the LM step): only the structurally non-zero entries of the UPPER triangle are written -- the caller zeroed H
 // once and mirrors while it copies -- so the serial part of the step is ~25 independent load/store pairs (__restrict__ lets
@@ -419,9 +358,7 @@ template <int M, int KIND> struct LinOps {
     static constexpr int NACC = L::N, COST = L::COST, COUNT = L::COUNT;
     static __device__ __forceinline__ void point(double* acc, const LinParams& p, double x, double y, double z, double u, double v) {
         double ru, rv, au[2 + ND], av[2 + ND];
-        bool ok;
-        if constexpr (M == ACM_MODEL_FOV && ACM_LIN_ATAN_TAB) ok = E::template eval<true>(p, x, y, z, u, v, ru, rv, au, av);
-        else ok = E::eval(p, x, y, z, u, v, ru, rv, au, av);
+        const bool ok = E::eval(p, x, y, z, u, v, ru, rv, au, av);
         lin_accumulate_masked<ND, E::UNIT_C>(acc, ok, ru, rv, au, av);
     }
     // `x` = the parameter vector the pass was evaluated at (unused here: fx, fy are folded in during the pass)
@@ -446,7 +383,7 @@ template <> struct LinOps<ACM_MODEL_KANNALA_BRANDT, ACM_RESIDUAL_PIXEL> {
         double r = fast_sqrt<true>(x * x + y * y, ir);
         const bool on_axis = !(r >= LIN_EPS);
         r = on_axis ? 0.0 : r;
-        const double th = ACM_LIN_ATAN_TAB ? acm_atan2_q1_tab(r, ok ? z : 1.0, p.atab) : fast_atan2_q1(r, ok ? z : 1.0);
+        const double th = fast_atan2_q1(r, ok ? z : 1.0);
         const double xr = on_axis ? 0.0 : x * ir, yr = on_axis ? 0.0 : y * ir;
         const double t2 = th * th, t3 = t2 * th, t5 = t3 * t2, t7 = t5 * t2, t9 = t7 * t2;
         const double thd = fma(p.d[3], t9, fma(p.d[2], t7, fma(p.d[1], t5, fma(p.d[0], t3, th))));

@@ -115,45 +115,3 @@ __device__ __forceinline__ double acm_atan2_q1(double a, double b) {
     at = hi ? __dadd_rn(ACM_ATAN_C[11], at) : at;
     return swap ? __dsub_rn(ACM_ATAN_C[12], at) : at;
 }
-
-// ---------------------------------------------------------------------------------------
-// Table-driven atan2 for the solver kernels (first quadrant, a >= 0, b > 0), 16 FP64 instructions instead of 25 and a
-// dependent chain of ~12 instead of ~20:  t = min/max in [0, 1];  with c = i/64 the table point nearest to t,
-//   atan(t) = atan(c) + atan(x),   x = (t - c) / (1 + t c) = (min - c max) / (max + c min),   |x| <= 1/128 (+ index slack),
-// so ONE reciprocal serves the division and the reduction, and x - x^3/3 + x^5/5 - x^7/7 is exact to 1.6e-18 relative
-// (checked with mpmath over 2e5 random t).  The index comes from a float estimate of t built from the operands' high
-// words (ALU / FP32 / MUFU work, nothing on the FP64 pipe); a wrong neighbour only widens |x| slightly, and i = 0 is exact
-// for tiny t (x = min / max).  The table {c_i, atan(c_i)} (65 x 16 B) sits in shared memory: per-lane indices would
-// serialise in the constant cache.  Total error <= ~1.5 ulp like acm_atan2_q1.
-// ---------------------------------------------------------------------------------------
-static __device__ const double ACM_ATAN_TAB64[65] = {
-    0x0.0p+0, 0x1.fff555bbb729bp-7, 0x1.ffd55bba97625p-6, 0x1.7fb818430da2ap-5, 0x1.ff55bb72cfdeap-5, 0x1.3f59f0e7c559dp-4, 0x1.7ee182602f10fp-4, 0x1.be39ebe6f07c3p-4, 0x1.fd5ba9aac2f6ep-4, 0x1.1e1fafb043727p-3, 0x1.3d6eee8c6626cp-3, 0x1.5c9811e3ec26ap-3, 0x1.7b97b4bce5b02p-3, 0x1.9a6a8e96c8626p-3, 0x1.b90d7529260a2p-3, 0x1.d77d5df205736p-3, 0x1.f5b75f92c80ddp-3, 0x1.09dc597d86362p-2, 0x1.18bf5a30bf178p-2, 0x1.278372057ef46p-2, 0x1.362773707ebccp-2, 0x1.44aa436c2af0ap-2, 0x1.530ad9951cd4ap-2, 0x1.614840309cfe2p-2, 0x1.6f61941e4def1p-2, 0x1.7d5604b63b3f7p-2, 0x1.8b24d394a1b25p-2, 0x1.98cd5454d6b18p-2, 0x1.a64eec3cc23fdp-2, 0x1.b3a911da65c6cp-2, 0x1.c0db4c94ec9f0p-2, 0x1.cde53432c1351p-2, 0x1.dac670561bb4fp-2, 0x1.e77eb7f175a34p-2, 0x1.f40dd0b541418p-2, 0x1.0039c73c1a40cp-1, 0x1.0657e94db30d0p-1, 0x1.0c6145b5b43dap-1, 0x1.1255d9bfbd2a9p-1, 0x1.1835a88be7c13p-1, 0x1.1e00babdefeb4p-1, 0x1.23b71e2cc9e6ap-1, 0x1.2958e59308e31p-1, 0x1.2ee628406cbcap-1, 0x1.345f01cce37bbp-1, 0x1.39c391cd4171ap-1, 0x1.3f13fb89e96f4p-1, 0x1.445065b795b56p-1, 0x1.4978fa3269ee1p-1, 0x1.4e8de5bb6ec04p-1, 0x1.538f57b89061fp-1, 0x1.587d81f732fbbp-1, 0x1.5d58987169b18p-1, 0x1.6220d115d7b8ep-1, 0x1.66d663923e087p-1, 0x1.6b798920b3d99p-1, 0x1.700a7c5784634p-1, 0x1.748978fba8e0fp-1, 0x1.78f6bbd5d315ep-1, 0x1.7d528289fa093p-1, 0x1.819d0b7158a4dp-1, 0x1.85d69576cc2c5p-1, 0x1.89ff5ff57f1f8p-1, 0x1.8e17aa99cc05ep-1, 0x1.921fb54442d18p-1};
-#define ACM_ATAN_TAB_BYTES (65 * 16)
-
-// fill the shared-memory table (call with all threads of the block, then __syncthreads())
-__device__ __forceinline__ void acm_atan_tab_init(double* tab_smem) {
-    for (int i = threadIdx.x; i < 65; i += blockDim.x) { tab_smem[2 * i] = (double)i * 0.015625; tab_smem[2 * i + 1] = ACM_ATAN_TAB64[i]; }
-}
-
-// float with ~20 correct bits from the high word of a non-negative double (0 below 2^-126, 3e38 above 2^127)
-__device__ __forceinline__ float acm_approx_f32(double v) {
-    const unsigned hi = (unsigned)__double2hiint(v);
-    const float f = __uint_as_float((hi << 3) - 0x38000000u);
-    return hi < 0x38100000u ? 0.0f : (hi >= 0x47f00000u ? 3.0e38f : f);
-}
-
-__device__ __forceinline__ double acm_atan2_q1_tab(double a, double b, unsigned tab_smem_addr) {
-    const bool swap = a > b;
-    const double mn = swap ? b : a, mx = swap ? a : b;
-    int i = __float2int_rn(__fdividef(acm_approx_f32(mn), acm_approx_f32(mx)) * 64.0f);
-    i = min(max(i, 0), 64);
-    double c, ac;
-    asm("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(c), "=d"(ac) : "r"(tab_smem_addr + 16u * (unsigned)i));
-    const double num = __fma_rn(-c, mx, mn), den = __fma_rn(c, mn, mx);
-    const double x = __dmul_rn(num, acm_rcp(den));
-    const double x2 = __dmul_rn(x, x);
-    double p = __fma_rn(x2, -1.0 / 7.0, 0.2);
-    p = __fma_rn(x2, p, -1.0 / 3.0);
-    const double at = __dadd_rn(ac, __fma_rn(__dmul_rn(x, x2), p, x));
-    return swap ? __dsub_rn(1.5707963267948966, at) : at;
-}

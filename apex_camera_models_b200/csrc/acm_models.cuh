@@ -34,13 +34,7 @@ __device__ __forceinline__ void acm_normalize_ieee(double x, double y, double z,
 // correctly rounded sqrt.  What follows the last test only has to meet the 1e-9 relative bar of the
 // values; there the IEEE divisions and square roots (three divisions in normalize() alone) become a
 // MUFU-seeded reciprocal / rsqrt (<= 2 ulp, acm_math.cuh).  unproject<true> keeps IEEE tails: sample_points uses it, so the
-// correspondences handed to the solver stay bit-identical to the reference's for the arithmetic-only models;
-// -DACM_IEEE_TAILS makes it the default everywhere (A/B aid).
-#ifdef ACM_IEEE_TAILS
-#define ACM_TAIL_DEFAULT true
-#else
-#define ACM_TAIL_DEFAULT false
-#endif
+// correspondences handed to the solver stay bit-identical to the reference's for the arithmetic-only models.
 template <bool IEEE>
 __device__ __forceinline__ void acm_normalize(double x, double y, double z, double& ox, double& oy, double& oz) {
     if (IEEE) { acm_normalize_ieee(x, y, z, ox, oy, oz); return; }
@@ -79,7 +73,7 @@ template <> struct CamModel<ACM_MODEL_PINHOLE> {
         if (BOUNDS && acm_outside(c, u, v)) return ACM_PROJECTION_OUTSIDE_IMAGE;
         return ACM_POINT_OK;
     }
-    template <bool IEEE = ACM_TAIL_DEFAULT>
+    template <bool IEEE = false>
     static __device__ __forceinline__ int unproject(const CamParams& c, double u, double v, double& rx, double& ry, double& rz) {
         if (acm_outside(c, u, v)) return ACM_POINT_IS_OUTSIDE_IMAGE;
         double mx = acm_mx(c, u), my = acm_my(c, v);
@@ -160,7 +154,7 @@ template <> struct CamModel<ACM_MODEL_RADTAN> {
         return -1;   // 100 steps without a stop: let the IEEE loop give the verdict
     }
 
-    template <bool IEEE = ACM_TAIL_DEFAULT>
+    template <bool IEEE = false>
     static __device__ int unproject(const CamParams& c, double u, double v, double& rx, double& ry, double& rz) {
         if (acm_outside(c, u, v)) return ACM_POINT_IS_OUTSIDE_IMAGE;
         const double k1 = c.d[0], k2 = c.d[1], p1 = c.d[2], p2 = c.d[3], k3 = c.d[4];
@@ -235,7 +229,7 @@ template <> struct CamModel<ACM_MODEL_KANNALA_BRANDT> {
         v = c.fy * thd * yr + c.cy;
         return ACM_POINT_OK;  // no image-bounds test in the reference
     }
-    template <bool IEEE = ACM_TAIL_DEFAULT>
+    template <bool IEEE = false>
     static __device__ int unproject(const CamParams& c, double u, double v, double& rx, double& ry, double& rz) {
         if (c.has_resolution && acm_outside(c, u, v)) return ACM_POINT_IS_OUTSIDE_IMAGE;
         const double k1 = c.d[0], k2 = c.d[1], k3 = c.d[2], k4 = c.d[3];
@@ -327,7 +321,7 @@ template <> struct CamModel<ACM_MODEL_UCM> {
         v = c.fy * (y / den) + c.cy;
         return ACM_POINT_OK;
     }
-    template <bool IEEE = ACM_TAIL_DEFAULT>
+    template <bool IEEE = false>
     static __device__ __forceinline__ int unproject(const CamParams& c, double u, double v, double& rx, double& ry, double& rz) {
         const double alpha = c.d[0];
         double gamma = 1.0 - alpha;
@@ -359,7 +353,7 @@ template <> struct CamModel<ACM_MODEL_EUCM> {
         v = c.fy * (y / den) + c.cy;
         return ACM_POINT_OK;
     }
-    template <bool IEEE = ACM_TAIL_DEFAULT>
+    template <bool IEEE = false>
     static __device__ __forceinline__ int unproject(const CamParams& c, double u, double v, double& rx, double& ry, double& rz) {
         const double alpha = c.d[0], beta = c.d[1];
         double mx = acm_mx(c, u), my = acm_my(c, v);
@@ -393,7 +387,7 @@ template <> struct CamModel<ACM_MODEL_DOUBLE_SPHERE> {
         v = c.fy * (y / den) + c.cy;
         return ACM_POINT_OK;
     }
-    template <bool IEEE = ACM_TAIL_DEFAULT>
+    template <bool IEEE = false>
     static __device__ __forceinline__ int unproject(const CamParams& c, double u, double v, double& rx, double& ry, double& rz) {
         const double alpha = c.d[0], xi = c.d[1];
         double gamma = 1.0 - alpha;
@@ -442,7 +436,7 @@ template <> struct CamModel<ACM_MODEL_FOV> {
         v = c.fy * my + c.cy;
         return ACM_POINT_OK;
     }
-    template <bool IEEE = ACM_TAIL_DEFAULT>
+    template <bool IEEE = false>
     static __device__ __forceinline__ int unproject(const CamParams& c, double u, double v, double& rx, double& ry, double& rz) {
         const double w = c.d[0];
         double mul2 = c.k0 * 2.0;

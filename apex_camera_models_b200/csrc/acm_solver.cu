@@ -415,20 +415,17 @@ __device__ __forceinline__ double warp_peer_exchange(const PeerArgs& peer, unsig
 //   DS 5.88 -> 6.24 TB/s (3 deep), EUCM 5.63 -> 5.79, UCM 5.83 -> 6.47 (2 deep), FOV 4.50 -> 4.97
 //   (3 deep, 128 threads), RadTan 4.09 -> 4.25 (2 deep; 5.1 with the structured accumulation; 128-thread blocks capped at 168
 //   registers for 12 warps/SM measured 4.2-4.8); Pinhole (already at 7.1 TB/s) is faster without the ring.
-// MIN_BLOCKS > 1 caps the registers through __launch_bounds__.
 // PTS = points evaluated per loop trip and thread (2 = one 16-byte packet per array, 4 = two packets: four independent
 // evaluation chains for the scheduler to interleave; needs an even DEPTH >= 2).
-template <int M> struct LinStreamDefault { static constexpr int DEPTH = 0, BLOCK = 256, MIN_BLOCKS = 0, PTS = 2; };
-#ifndef ACM_LIN_NO_RING  // A/B aid: -DACM_LIN_NO_RING builds every model with the register prefetch
-template <> struct LinStreamDefault<ACM_MODEL_DOUBLE_SPHERE> { static constexpr int DEPTH = 3, BLOCK = 256, MIN_BLOCKS = 0, PTS = 2; };
-template <> struct LinStreamDefault<ACM_MODEL_EUCM> { static constexpr int DEPTH = 3, BLOCK = 256, MIN_BLOCKS = 0, PTS = 2; };
-template <> struct LinStreamDefault<ACM_MODEL_UCM> { static constexpr int DEPTH = 2, BLOCK = 256, MIN_BLOCKS = 0, PTS = 2; };
-template <> struct LinStreamDefault<ACM_MODEL_FOV> { static constexpr int DEPTH = 4, BLOCK = 256, MIN_BLOCKS = 0, PTS = 4; };
-template <> struct LinStreamDefault<ACM_MODEL_RADTAN> { static constexpr int DEPTH = 3, BLOCK = 256, MIN_BLOCKS = 0, PTS = 2; };
-#endif
+template <int M> struct LinStream { static constexpr int DEPTH = 0, BLOCK = 256, PTS = 2; };
+template <> struct LinStream<ACM_MODEL_DOUBLE_SPHERE> { static constexpr int DEPTH = 3, BLOCK = 256, PTS = 2; };
+template <> struct LinStream<ACM_MODEL_EUCM> { static constexpr int DEPTH = 3, BLOCK = 256, PTS = 2; };
+template <> struct LinStream<ACM_MODEL_UCM> { static constexpr int DEPTH = 2, BLOCK = 256, PTS = 2; };
+template <> struct LinStream<ACM_MODEL_FOV> { static constexpr int DEPTH = 4, BLOCK = 256, PTS = 4; };
+template <> struct LinStream<ACM_MODEL_RADTAN> { static constexpr int DEPTH = 3, BLOCK = 256, PTS = 2; };
 // KB (37 accumulators, 166 registers): 3 blocks of 128 threads.  Same-box A/B (scripts/ab_lin.sh; boxes of the pool differ by
 // up to 40 % on this FP64-bound kernel, so only same-box comparisons count): register prefetch 4.42 TB/s, ring 1 deep 3.95,
-// 2 deep 4.51, 3 deep 4.59; capped at 128 registers (MIN_BLOCKS = 4, 36-byte spill) 4.19.
+// 2 deep 4.51, 3 deep 4.59; capped at 128 registers (4 blocks per SM, 36-byte spill) 4.19.
 // Round 2, same-box A/B (profiles/r02_ab_pts4.log): four points per trip, FOV 5262 -> 5463 GB/s (2 deep), KB 4789 -> 4861 (4 deep);
 // RadTan loses (5348 -> 5139 / 4255) and keeps two.  FOV in 256-thread blocks (the compiler then takes 126 registers instead of
 // 96, two blocks per SM): 5365 -> 5667 GB/s 4 deep, 5535 2 deep (profiles/r02_ab_fov_occ*.log); capping the registers for more
@@ -436,14 +433,7 @@ template <> struct LinStreamDefault<ACM_MODEL_RADTAN> { static constexpr int DEP
 // 256-thread block per SM, long_scoreboard 0.56 per issue with the ring 2 deep): 3 deep 5345 -> 5560, 4 deep 5561; two 128-thread
 // blocks 4876 (profiles/r02_ab_radtan_ring.log).  Double Sphere (the headline kernel) does not move: 3 deep x 2 points 5931-5939, 4 deep x 4
 // points 5941, 4 deep x 2 points 5926-5952 GB/s over 200 launches (profiles/r02_ab_ds_headline.log).
-template <> struct LinStreamDefault<ACM_MODEL_KANNALA_BRANDT> { static constexpr int DEPTH = 4, BLOCK = 128, MIN_BLOCKS = 0, PTS = 4; };
-template <int M> struct LinStream : LinStreamDefault<M> {};
-#ifdef ACM_EXP_MODEL  // tuning aid: -DACM_EXP_MODEL=<id> -DACM_EXP_DEPTH= -DACM_EXP_BLOCK= -DACM_EXP_MINB= overrides one model
-#ifndef ACM_EXP_PTS
-#define ACM_EXP_PTS 2
-#endif
-template <> struct LinStream<ACM_EXP_MODEL> { static constexpr int DEPTH = ACM_EXP_DEPTH, BLOCK = ACM_EXP_BLOCK, MIN_BLOCKS = ACM_EXP_MINB, PTS = ACM_EXP_PTS; };
-#endif
+template <> struct LinStream<ACM_MODEL_KANNALA_BRANDT> { static constexpr int DEPTH = 4, BLOCK = 128, PTS = 4; };
 
 // The solve form of the kernel (128-thread blocks) has its own ring depth / points per trip / register cap: it carries the trial
 // parameters in registers (the one-pass form reads them from the constant bank) and peaks at 152-168 registers outside the
@@ -452,8 +442,7 @@ template <> struct LinStream<ACM_EXP_MODEL> { static constexpr int DEPTH = ACM_E
 // 1.25 M / 10 M correspondences): Double Sphere 15.1 -> 13.9 / 67.7 -> 66.4 (taken); EUCM 13.7 -> 12.7 / 63.4 -> 64.3 and UCM
 // 11.4 -> 10.4 / 62.2 -> 70.3 (better from L2, worse from HBM: kept at three); FOV worse at both.  Four points per trip fit
 // 166 registers for Double Sphere but gain nothing (15.2 / 70.0).
-// -DACM_EXP_SOLVE_MODEL=<id> -DACM_EXP_SOLVE_DEPTH= -DACM_EXP_SOLVE_PTS= -DACM_EXP_SOLVE_MINB= overrides one model.
-template <int M> struct SolveStreamDefault {
+template <int M> struct SolveStream {
     // Ring depth / points per trip of the solve, measured on their own (us per pass at 10 M correspondences,
     // profiles/r02_ab_lm_fov.log, r02_ab_lm_kb_rt.log): FOV with four points per trip spilled under the 170-register cap (20
     // bytes): two points, 3 deep = 95.7 -> 80.0; KB two points 3 deep (238 registers) 102.8 -> 98.6; RadTan 3 deep 94.0 -> 90.9
@@ -467,13 +456,6 @@ template <int M> struct SolveStreamDefault {
     // 10-15 % at 10 M, EUCM gains 0.5 % (profiles/r02_ab_lm_stream2.log, _stream3.log).  0 = never.
     static constexpr size_t WIDE_BLOCK_FROM = (M == ACM_MODEL_DOUBLE_SPHERE) ? 4000000 : 0;
 };
-template <int M> struct SolveStream : SolveStreamDefault<M> {};
-#ifdef ACM_EXP_SOLVE_MODEL
-template <> struct SolveStream<ACM_EXP_SOLVE_MODEL> {
-    static constexpr int DEPTH = ACM_EXP_SOLVE_DEPTH, PTS = ACM_EXP_SOLVE_PTS, MIN_BLOCKS = ACM_EXP_SOLVE_MINB;
-    static constexpr size_t WIDE_BLOCK_FROM = 0;
-};
-#endif
 template <int M, bool SOLVE> struct StreamCfg { static constexpr int DEPTH = LinStream<M>::DEPTH, PTS = LinStream<M>::PTS; };
 template <int M> struct StreamCfg<M, true> { static constexpr int DEPTH = SolveStream<M>::DEPTH, PTS = SolveStream<M>::PTS; };
 
@@ -507,11 +489,6 @@ __device__ __forceinline__ void lin_stream_pass(const LinKernelArgs& a, const Li
     extern __shared__ double2 lin_ring[];
     LinParams p = p_in;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    if constexpr ((M == ACM_MODEL_KANNALA_BRANDT || M == ACM_MODEL_FOV) && ACM_LIN_ATAN_TAB) {
-        __shared__ __align__(16) double lin_atab[2 * 65];
-        if (!primed) { acm_atan_tab_init(lin_atab); __syncthreads(); }   // a solve fills it in its first pass
-        p.atab = (unsigned)__cvta_generic_to_shared(lin_atab);
-    }
     const int nb = (int)gridDim.x;
     const size_t npairs = a.n >> 1;
     const size_t stride = (size_t)nb * BS;
@@ -800,7 +777,7 @@ __device__ __forceinline__ bool lin_pass(const LinKernelArgs& a, LmState* sh, Lm
 }
 
 template <int M, int KIND, int BS, bool SOLVE>
-__global__ void __launch_bounds__(BS, (SOLVE ? (BS == 128 ? SolveStream<M>::MIN_BLOCKS : 0) : (BS == LinStream<M>::BLOCK ? LinStream<M>::MIN_BLOCKS : 0))) lin_kernel(const __grid_constant__ LinKernelArgs a) {
+__global__ void __launch_bounds__(BS, (SOLVE && BS == 128) ? SolveStream<M>::MIN_BLOCKS : 0) lin_kernel(const __grid_constant__ LinKernelArgs a) {
     static_assert(LinOps<M, KIND>::NACC <= 64, "hand-off layout assumes <= 64 accumulators");
     constexpr int NSTATE = sizeof(LmState) / sizeof(double);
     __shared__ LmState sh;
@@ -849,10 +826,10 @@ static int32_t ensure_ll(acm_ctx* ctx, size_t blocks) {
     return ACM_OK;
 }
 
-template <int M, int KIND, int BS>
+template <int M, int KIND, int BS, bool SOLVE>
 static int32_t launch_lin_bs(acm_ctx* ctx, LinKernelArgs& a, const acm_points* xyz, const acm_points* uv) {
-    const size_t ring_bytes = (size_t)(a.mode == 2 ? StreamCfg<M, true>::DEPTH : StreamCfg<M, false>::DEPTH) * 5 * BS * sizeof(double2);
-    const void* fn = a.mode == 2 ? reinterpret_cast<const void*>(&lin_kernel<M, KIND, BS, true>) : reinterpret_cast<const void*>(&lin_kernel<M, KIND, BS, false>);
+    const size_t ring_bytes = (size_t)StreamCfg<M, SOLVE>::DEPTH * 5 * BS * sizeof(double2);
+    const void* fn = reinterpret_cast<const void*>(&lin_kernel<M, KIND, BS, SOLVE>);
     int bps = 0;
     int32_t rc = acm_kernel_blocks_per_sm(ctx, fn, BS, ring_bytes, &bps);
     if (rc) return rc;
@@ -860,7 +837,7 @@ static int32_t launch_lin_bs(acm_ctx* ctx, LinKernelArgs& a, const acm_points* x
     int grid = grid_for(ctx, (n >> 1) + 1, BS, bps);
     // the solve gives every sum its own reducer block (a few hundred correspondences would otherwise queue all sums on the
     // warps of one or two blocks: 6.4 k of the 15 k cycles of a pass at n = 450); blocks without points contribute zeros
-    if (a.mode == 2 && grid < LinOps<M, KIND>::NACC) grid = LinOps<M, KIND>::NACC;
+    if (SOLVE && grid < LinOps<M, KIND>::NACC) grid = LinOps<M, KIND>::NACC;
     rc = ensure_ll(ctx, (size_t)ctx->sm_count * 16);
     if (rc) return rc;
     ACM_REQUIRE(ctx, (size_t)grid <= (size_t)ctx->sm_count * 16, "linearize: grid larger than the hand-off buffer");
@@ -872,15 +849,14 @@ static int32_t launch_lin_bs(acm_ctx* ctx, LinKernelArgs& a, const acm_points* x
     a.out = ctx->d_reduce;
     // tags: one per pass, never reused
     a.tag0 = ctx->lm_tag + 1;
-    ctx->lm_tag += (a.mode == 2 ? (unsigned long long)a.max_passes : 1ULL) + 1ULL;
+    ctx->lm_tag += (SOLVE ? (unsigned long long)a.max_passes : 1ULL) + 1ULL;
     void* args[] = {&a};
     if (ctx->coop_launch) {
         ACM_CUDA(ctx, cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(BS), args, ring_bytes, ctx->stream));
         ctx->launches++;
     } else {
         // no cooperative launch on this device / configuration: the grid never exceeds the resident capacity computed above
-        if (a.mode == 2) lin_kernel<M, KIND, BS, true><<<grid, BS, ring_bytes, ctx->stream>>>(a);
-        else lin_kernel<M, KIND, BS, false><<<grid, BS, ring_bytes, ctx->stream>>>(a);
+        lin_kernel<M, KIND, BS, SOLVE><<<grid, BS, ring_bytes, ctx->stream>>>(a);
         ACM_CHECK_LAUNCH(ctx);
     }
     return ACM_OK;
@@ -888,15 +864,14 @@ static int32_t launch_lin_bs(acm_ctx* ctx, LinKernelArgs& a, const acm_points* x
 
 // Block size per model: the accumulators of the wide models (KB: 37 doubles) push the
 // kernel past 128 registers/thread; 128-thread blocks then pack one more block per SM.
-// ACM_LIN_BLOCK=128|256 overrides (tuning aid).
+// The solve runs 128-thread blocks, or 256 from SolveStream<M>::WIDE_BLOCK_FROM correspondences on.
 template <int M, int KIND>
 static int32_t launch_lin(acm_ctx* ctx, LinKernelArgs& a, const acm_points* xyz, const acm_points* uv) {
-    int bs = LinStream<M>::BLOCK;
-    if (a.mode == 2) bs = (SolveStream<M>::WIDE_BLOCK_FROM != 0 && xyz->n >= SolveStream<M>::WIDE_BLOCK_FROM) ? 256 : 128;
-    const char* e = getenv("ACM_LIN_BLOCK");
-    if (e && (atoi(e) == 128 || atoi(e) == 256)) bs = atoi(e);
-    if (bs == 128) return launch_lin_bs<M, KIND, 128>(ctx, a, xyz, uv);
-    return launch_lin_bs<M, KIND, 256>(ctx, a, xyz, uv);
+    if (a.mode != 2) return launch_lin_bs<M, KIND, LinStream<M>::BLOCK, false>(ctx, a, xyz, uv);
+    if constexpr (SolveStream<M>::WIDE_BLOCK_FROM != 0) {
+        if (xyz->n >= SolveStream<M>::WIDE_BLOCK_FROM) return launch_lin_bs<M, KIND, 256, true>(ctx, a, xyz, uv);
+    }
+    return launch_lin_bs<M, KIND, 128, true>(ctx, a, xyz, uv);
 }
 
 #define ACM_DISPATCH_LIN(model, kind, ...)                                                                       \
@@ -940,7 +915,7 @@ static void make_lin_params(const acm_camera* cam, LinParams* p) {
     lin_derive(cam->model, *p);
 }
 
-static bool peers_usable(const acm_ctx* ctx) { return ctx->peer_n > 1 && !getenv("ACM_NO_PEER_EXCHANGE"); }
+static bool peers_usable(const acm_ctx* ctx) { return ctx->peer_n > 1; }
 
 // A peer exchange that timed out leaves the ranks' exchange counters out of step: refuse to go on
 // until the host has re-attached the peers (acm_peer_detach + acm_peer_attach / acm_comm_init_all).

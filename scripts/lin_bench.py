@@ -1,5 +1,5 @@
 """Times acm_linearize_async for every model on 100 M synthetic correspondences (inputs > L2).
-ACM_LIN_BLOCK=128|256 overrides the block size; MODELS=5,2,... selects model ids; REPS sets the launches."""
+MODELS=5,2,... selects model ids; REPS sets the launches."""
 import ctypes as C, os, sys
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -27,4 +27,4 @@ for mid in models:
         ctx.sync(); ctx.timer_start()
         for _ in range(reps): f()
         ms = ctx.timer_stop() / reps
-        print(f"{names[mid]:15s} kind={kind} block={os.environ.get('ACM_LIN_BLOCK', 'default')}: {ms:.3f} ms  {n / ms / 1e6:.1f} Gpts/s  {n * 40 / ms / 1e6:.0f} GB/s", flush=True)
+        print(f"{names[mid]:15s} kind={kind}: {ms:.3f} ms  {n / ms / 1e6:.1f} Gpts/s  {n * 40 / ms / 1e6:.0f} GB/s", flush=True)

@@ -968,10 +968,12 @@ def test_reprojection_error_matches_oracle(acm, ctx, O, cameras, name):
 
 
 @pytest.mark.parametrize("name,W,H", [("kannala_brandt", 512, 512), ("double_sphere", 752, 480), ("pinhole", 752, 480),
-                                      ("rad_tan", 752, 480), ("fov", 320, 200), ("ucm", 1920, 1080), ("kannala_brandt", 37, 29)])
+                                      ("rad_tan", 752, 480), ("fov", 320, 200), ("ucm", 1920, 1080), ("kannala_brandt", 37, 29),
+                                      ("double_sphere", 756, 480)])
 def test_undistort_bytes_and_remap_indices(acm, ctx, O, cameras, name, W, H):
     """undistort.rs:14-105: output bytes and remap indices are bit-exact (KB / FOV depend on the
-    device atan2: count index flips, expected 0)."""
+    device atan2: count index flips, expected 0).  Widths that are multiples of 16 take the TMA kernel, 756 (a multiple
+    of 4 only) the whole-image gather kernel when bilinear, 37 the generic one."""
     cam = dict(cameras[name]); cam["width"], cam["height"] = W, H
     if name in ("ucm", "fov"):  # keep the principal point inside the test image
         cam["params"] = list(cam["params"]); cam["params"][2] = W / 2.0 + 0.3; cam["params"][3] = H / 2.0 - 0.2

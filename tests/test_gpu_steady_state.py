@@ -27,7 +27,6 @@ pytestmark = pytest.mark.gpu
 NT = min(os.cpu_count() or 1, 16)   # oracle threads (per-point results do not depend on it)
 PAIRS = [(name, 0) for name in MODELS] + [(name, 1) for name in MODELS if name in UNIFIED]
 PAIR_IDS = [f"{n}-{'algebraic' if k else 'pixel'}" for n, k in PAIRS]
-DEFAULT_LIN_BLOCK = {"kannala_brandt": 128}   # LinStream<M>::BLOCK of the one-pass kernel; 256 for the others
 
 
 @pytest.fixture(scope="module")
@@ -249,11 +248,6 @@ def assert_normal_equations_match(H, g, c, nv, Ho, go, co, nvo):
     assert np.array_equal(H, H.T)
 
 
-def block_shapes(name):
-    d = DEFAULT_LIN_BLOCK.get(name, 256)
-    return [None, 384 - d]   # the default shape, then the other one through ACM_LIN_BLOCK
-
-
 def linearize_once(ctx, cost):
     before = ctx.kernel_launches()
     out = cost.linearize()
@@ -262,14 +256,14 @@ def linearize_once(ctx, cost):
 
 
 @pytest.mark.parametrize("name,kind", PAIRS, ids=PAIR_IDS)
-def test_linearize_at_steady_state(acm, ctx, O, cameras, sizes, monkeypatch, name, kind):
+def test_linearize_at_steady_state(acm, ctx, O, cameras, sizes, name, kind):
     """lin_kernel<M, KIND, BS, false> (one pass, one launch) at n = 12*T + 75.
 
     The grid is min(ceil(pairs / BS), S * blocks_per_sm) <= T / BS blocks, so every thread streams at least
     (n / 2) / T >= 6 packets: more than the deepest ring (4), so every stage of every ring is reused; the four-point
     loop of KB / FOV runs at least two trips, and as the packet count per thread is 6 or 7 at full occupancy the
-    odd-packet tail runs too.  n is odd: block 0 / thread 0 adds the last point.  Both block shapes (128 and 256
-    threads) are run against the same oracle sums; a repeat call is bit-identical."""
+    odd-packet tail runs too.  n is odd: block 0 / thread 0 adds the last point.  The block shape is the model's
+    (128 threads for KB, 256 for the others); a repeat call is bit-identical."""
     cam = cameras[name]
     m, om = gpu_model(acm, ctx, cam), oracle_model(O, cam)
     n = sizes["lin"]
@@ -278,15 +272,10 @@ def test_linearize_at_steady_state(acm, ctx, O, cameras, sizes, monkeypatch, nam
     assert n - nvo >= n // 100, (n, nvo)   # the rejected points are there
     X, UV = acm.Points.from_numpy(ctx, xyz), acm.Points.from_numpy(ctx, obs)
     cost = acm.OptimizationCost(m, X, UV, residual_kind=kind)
-    for bs in block_shapes(name):
-        if bs is None:
-            monkeypatch.delenv("ACM_LIN_BLOCK", raising=False)
-        else:
-            monkeypatch.setenv("ACM_LIN_BLOCK", str(bs))
-        H, g, c, nv = linearize_once(ctx, cost)
-        assert_normal_equations_match(H, g, c, nv, Ho, go, co, nvo)
-        H2, g2, c2, nv2 = linearize_once(ctx, cost)
-        assert np.array_equal(H, H2) and np.array_equal(g, g2) and c == c2 and nv == nv2, bs
+    H, g, c, nv = linearize_once(ctx, cost)
+    assert_normal_equations_match(H, g, c, nv, Ho, go, co, nvo)
+    H2, g2, c2, nv2 = linearize_once(ctx, cost)
+    assert np.array_equal(H, H2) and np.array_equal(g, g2) and c == c2 and nv == nv2
     X.free(); UV.free()
 
 
@@ -302,12 +291,12 @@ def valid_points(O, om, name, n, seed, cos_max=None):
 
 
 @pytest.mark.parametrize("name", MODELS)
-def test_linearize_census_at_steady_state(acm, ctx, O, cameras, sizes, monkeypatch, name):
+def test_linearize_census_at_steady_state(acm, ctx, O, cameras, sizes, name):
     """Pixel residual at n = 12*T + 75 (the size of test_linearize_at_steady_state): every point is valid and observed
     at the oracle's projection, except K markers observed 1 px to the right, at indices 0..63, n-64..n-1 (the odd last
     point is block 0 / thread 0's) and 4096 random ones.  The markers carry the whole cost and gradient, so cost / c0
     (c0: the oracle's cost of one marker) and |g[cx]| must round to exactly K: a dropped or doubled packet, or one read
-    from a stale ring slot, moves them by a whole unit whatever the tolerance.  Both block shapes."""
+    from a stale ring slot, moves them by a whole unit whatever the tolerance."""
     cam = cameras[name]
     m, om = gpu_model(acm, ctx, cam), oracle_model(O, cam)
     n = sizes["lin"]
@@ -321,15 +310,10 @@ def test_linearize_census_at_steady_state(acm, ctx, O, cameras, sizes, monkeypat
     assert nv0 == 1 and 0.49 < c0 < 0.51
     X, UV = acm.Points.from_numpy(ctx, xyz), acm.Points.from_numpy(ctx, obs)
     cost = acm.OptimizationCost(m, X, UV, residual_kind=0)
-    for bs in block_shapes(name):
-        if bs is None:
-            monkeypatch.delenv("ACM_LIN_BLOCK", raising=False)
-        else:
-            monkeypatch.setenv("ACM_LIN_BLOCK", str(bs))
-        H, g, c, nv = linearize_once(ctx, cost)
-        assert nv == n, (bs, nv - n)
-        assert round(c / c0) == K, (bs, c / c0 - K)
-        assert round(abs(g[2])) == K, (bs, abs(g[2]) - K)
+    H, g, c, nv = linearize_once(ctx, cost)
+    assert nv == n, nv - n
+    assert round(c / c0) == K, c / c0 - K
+    assert round(abs(g[2])) == K, abs(g[2]) - K
     X.free(); UV.free()
 
 
@@ -379,25 +363,18 @@ def assert_same_solve(r, oo, ores, what):
 
 
 @pytest.mark.parametrize("name,kind", PAIRS, ids=PAIR_IDS)
-def test_lm_solve_at_steady_state(acm, ctx, O, cameras, sizes, monkeypatch, name, kind):
+def test_lm_solve_at_steady_state(acm, ctx, O, cameras, sizes, name, kind):
     """lin_kernel<M, KIND, BS, true> (the whole solve in one cooperative launch) at n = 12*T + 75, with the converter's
     configuration and bounds (Pinhole: none).  Below WIDE_BLOCK_FROM the solve runs 128-thread blocks, at most T / 128
-    of them, so every thread streams at least 6 packets per pass and the solve ring (2-4 deep) wraps within each pass;
-    ACM_LIN_BLOCK = 256 runs the other block shape.  Each must walk the oracle's trajectory: status, iterations and
-    passes equal, n_valid exact, parameters and final cost within 1e-9."""
+    of them, so every thread streams at least 6 packets per pass and the solve ring (2-4 deep) wraps within each pass.
+    It must walk the oracle's trajectory: status, iterations and passes equal, n_valid exact, parameters and final cost
+    within 1e-9."""
     n = sizes["lin"]
     m, om, X, UV, xyz, uv, lo, hi = solve_problem(acm, ctx, O, cameras, name, n, 0xACE50019 + MODELS.index(name))
-    start = m.params().copy()
     oo, ores = O.lm_solve(om, kind, xyz, uv, lo, hi, nthreads=NT)
     cost = acm.OptimizationCost(m, X, UV, residual_kind=kind)
-    for bs in (None, 128, 256):
-        if bs is None:
-            monkeypatch.delenv("ACM_LIN_BLOCK", raising=False)
-        else:
-            monkeypatch.setenv("ACM_LIN_BLOCK", str(bs))
-        m.set_params(start)
-        r = solve_once(ctx, cost, bounds="converter" if lo is not None else None)
-        assert_same_solve(r, oo, ores, (name, kind, bs))
+    r = solve_once(ctx, cost, bounds="converter" if lo is not None else None)
+    assert_same_solve(r, oo, ores, (name, kind))
     X.free(); UV.free()
 
 
