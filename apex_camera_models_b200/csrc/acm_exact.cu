@@ -460,7 +460,7 @@ __global__ void __launch_bounds__(256) undistort_kernel(const __grid_constant__ 
     const int seg_px = min(1024, W - blockIdx.x * 1024);  // pixels of this block's segment
     const int seg_bytes = seg_px * 3;
     const size_t seg_off = ((size_t)row * W + (size_t)blockIdx.x * 1024) * 3;
-    const bool vec_ok = ((seg_off & 15) == 0) && ((frame_bytes & 15) == 0);
+    const bool vec_ok = ((seg_off & 15) == 0) && ((frame_bytes & 15) == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
     for (size_t f = 0; f < n_frames; ++f) {
         const uint8_t* src = in + f * frame_bytes;
         uint8_t o[12];
@@ -498,7 +498,7 @@ __global__ void __launch_bounds__(256) undistort_kernel(const __grid_constant__ 
 }
 
 // ---------------------------------------------------------------------------------------
-// Fast bilinear path (W % 4 == 0, 4-byte aligned frames).  Byte-exact by construction:
+// Per-pixel work of the TMA and gather kernels below.  Byte-exact by construction:
 //  * The reference blends in f64 (undistort.rs:92-99) and rounds half away from zero.  Here the
 //    four tap weights are quantised once per output pixel to 24-bit fixed point
 //    (W_i = rn(w_i * 2^24), sum <= 2^24 + 2, so sum p_i W_i fits 32 bits).
@@ -506,142 +506,182 @@ __global__ void __launch_bounds__(256) undistort_kernel(const __grid_constant__ 
 //    reference moves the value by < 1e-12, so whenever the fractional part of S + 0.5 is farther
 //    than E = 640 / 2^24 = 3.8e-5 from an integer both round to the same byte.  Otherwise
 //    (probability 7.6e-5 per channel) the pixel is redone with the reference's exact f64
-//    expression, as are pixels with a weight of exactly 1 or whose window would leave the frame.
-//  * Instruction diet (the first version of this kernel was issue-bound at 151 instr/pixel):
-//    each 6-byte tap run is three aligned 32-bit loads + two PRMT with a per-pixel selector;
-//    five more PRMT gather the four taps of each channel into one register; the blend is three
-//    dp4a per channel against the weights split into byte planes (W = hi<<16 | mid<<8 | lo).
-// ---------------------------------------------------------------------------------------
-__device__ __forceinline__ void blend_exact_px(const uint8_t* p, int row_stride, double wx, double wy, uint8_t* o) {
-    const uint8_t* q = p + row_stride;
-    const double wxi = 1.0 - wx, wyi = 1.0 - wy;
-    o[0] = blend(__ldg(p), __ldg(p + 3), __ldg(q), __ldg(q + 3), wx, wy, wxi, wyi);
-    o[1] = blend(__ldg(p + 1), __ldg(p + 4), __ldg(q + 1), __ldg(q + 4), wx, wy, wxi, wyi);
-    o[2] = blend(__ldg(p + 2), __ldg(p + 5), __ldg(q + 2), __ldg(q + 5), wx, wy, wxi, wyi);
-}
-
+//    expression, as are pixels with a weight of exactly 1.
+//  * Instruction diet (the first gather kernel was issue-bound at 151 instr/pixel): each 6-byte tap
+//    run is three aligned 32-bit words + two PRMT with a per-pixel selector; five more PRMT gather the
+//    four taps of each channel into one register; the blend is S = (dp2a(hi16) << 8) + dp4a(lo8) + 2^23
+//    per channel: the upper 16 bits of the weights pairwise through dp2a, the low byte plane through dp4a.
 // Thread <-> pixel mapping: a warp owns a 32-wide, 4-tall output patch, lane = x.  Neighbouring
 // lanes then read neighbouring source pixels (3 bytes apart), so one warp-wide 32-bit load touches
 // ~4 sectors instead of the ~17 of a "4 consecutive pixels per thread" mapping (ncu: the first
-// mapping was bound by L1 sector look-ups, 444 M per 8 frames).  The 96 output bytes of a patch row
-// are exchanged with two shuffles so that 24 lanes store one aligned word each.
-template <int M>
-__device__ __forceinline__ void undistort_patch_gather(const CamParams& c, double tfx, double tfy, double tcx, double tcy,
-                                                       const uint8_t* __restrict__ in, uint8_t* __restrict__ out, int W, int H,
-                                                       size_t n_frames, const int x0, const int y0) {
-    constexpr uint32_t TIE_E = 640u;
-    const int lane = threadIdx.x & 31;
-    const int uo = x0 + lane;
-    const size_t frame_bytes = (size_t)W * H * 3;
-    const int row_stride = 3 * W;
-    int off[4], offa[4], mode[4];          // mode: 0 black, 1 fast, 2 exact only, 3 redo this frame exactly
-    uint32_t sel[4], wlo[4], wmid[4], whi[4];
-    double wx[4], wy[4];
+// mapping was bound by L1 sector look-ups, 444 M per 8 frames).
+// ---------------------------------------------------------------------------------------
+constexpr uint32_t UND_TIE_E = 640u;
+
+// One output pixel, set up once and reused for every frame.
+struct FixedTap {
+    Tap t;
+    uint32_t sel;            // PRMT selector of the sample's bytes in its 4-byte-aligned window
+    uint32_t wlo, w01, w23;  // 24-bit weights, tap order [00, 10, 01, 11]: low byte plane for dp4a, upper 16 bits pairwise
+                             // for dp2a.  All zero without a sample: the blend is then 2^23 >> 24 = 0 (black) and can never
+                             // look like a tie, so the frame loops need no per-pixel mode test.
+    bool slow;               // bilinear with a weight of exactly 1: always takes the exact f64 expression
+};
+
+template <int M, bool NEAREST>
+__device__ __forceinline__ FixedTap setup_tap(const CamParams& c, double tfx, double tfy, double tcx, double tcy, int uo, int vo, int W,
+                                              int H) {
+    const double xn = ((double)uo - tcx) / tfx;  // outside the branch: the 4 pixels of a lane share it
+    double sx = 0.0, sy = 0.0;
+    int st = ACM_POINT_IS_OUTSIDE_IMAGE;
+    if (uo < W && vo < H) {
+        const double yn = ((double)vo - tcy) / tfy;
+        st = CamModel<M>::template project<true>(c, xn, yn, 1.0, sx, sy);
+    }
+    FixedTap p;
+    p.t = make_tap(sx, sy, st, W, H, NEAREST ? ACM_INTERP_NEAREST : ACM_INTERP_BILINEAR);
+    const double wxi = 1.0 - p.t.wx, wyi = 1.0 - p.t.wy;
+    uint32_t w00 = __double2uint_rn(wxi * wyi * 16777216.0), w10 = __double2uint_rn(p.t.wx * wyi * 16777216.0);
+    uint32_t w01 = __double2uint_rn(wxi * p.t.wy * 16777216.0), w11 = __double2uint_rn(p.t.wx * p.t.wy * 16777216.0);
+    if (!p.t.ok) w00 = w10 = w01 = w11 = 0u;
+    p.slow = !NEAREST && ((w00 | w10 | w01 | w11) >> 24) != 0u;
+    p.wlo = (w00 & 0xFF) | ((w10 & 0xFF) << 8) | ((w01 & 0xFF) << 16) | ((w11 & 0xFF) << 24);
+    p.w01 = ((w00 >> 8) & 0xFFFF) | (((w10 >> 8) & 0xFFFF) << 16);
+    p.w23 = ((w01 >> 8) & 0xFFFF) | (((w11 >> 8) & 0xFFFF) << 16);
+    p.sel = 0x3210u + 0x1111u * (uint32_t)(p.t.off00 & 3);
+    return p;
+}
+
+// Bilinear blend from the aligned 12-byte windows of the two tap rows (a0..a2, b0..b2) with the selector and weights
+// of setup_tap.  Returns [R G B 0] and in `tz` the distance of the three channel sums to a rounding tie (see tie_bits).
+__device__ __forceinline__ uint32_t blend_fixed(uint32_t a0, uint32_t a1, uint32_t a2, uint32_t b0, uint32_t b1, uint32_t b2, uint32_t sel,
+                                                uint32_t wlo, uint32_t w01, uint32_t w23, uint32_t& tz) {
+    const uint32_t A = __byte_perm(a0, a1, sel), B = __byte_perm(a1, a2, sel);         // [r0 g0 b0 r1] [g1 b1 . .]
+    const uint32_t A2 = __byte_perm(b0, b1, sel), B2 = __byte_perm(b1, b2, sel);
+    const uint32_t PR = __byte_perm(A, A2, 0x7430);                                    // [r00 r10 r01 r11]
+    const uint32_t T0 = __byte_perm(A, B, 0x5241), T1 = __byte_perm(A2, B2, 0x5241);   // [g0 g1 b0 b1]
+    const uint32_t PG = __byte_perm(T0, T1, 0x5410), PB = __byte_perm(T0, T1, 0x7632);
+    const uint32_t sr = (__dp2a_hi(w23, PR, __dp2a_lo(w01, PR, 0u)) << 8) + __dp4a(PR, wlo, 1u << 23);
+    const uint32_t sg = (__dp2a_hi(w23, PG, __dp2a_lo(w01, PG, 0u)) << 8) + __dp4a(PG, wlo, 1u << 23);
+    const uint32_t sb = (__dp2a_hi(w23, PB, __dp2a_lo(w01, PB, 0u)) << 8) + __dp4a(PB, wlo, 1u << 23);
+    // distance of the 24-bit fraction to a rounding tie, scaled by 2^8 so that the 32-bit wrap does the
+    // masking: ((s + E) mod 2^24) < 2E  <=>  (s * 2^8 + E * 2^8) mod 2^32 < 2E * 2^8
+    tz = min(min(sr * 256u + UND_TIE_E * 256u, sg * 256u + UND_TIE_E * 256u), sb * 256u + UND_TIE_E * 256u);
+    return __byte_perm(__byte_perm(sr, sg, 0x4473), sb, 0x4710);                       // [sr.3 sg.3 sb.3 .]
+}
+
+// bit k: pixel k of blend_fixed is too close to a rounding tie and must be redone exactly
+__device__ __forceinline__ uint32_t tie_bits(const uint32_t tz[4]) {
+    uint32_t bits = 0u;
+    if (min(min(tz[0], tz[1]), min(tz[2], tz[3])) < 2u * UND_TIE_E * 256u) {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) bits |= (tz[k] < 2u * UND_TIE_E * 256u ? 1u : 0u) << k;
+    }
+    return bits;
+}
+
+// nearest: the sample is the pixel itself (undistort.rs:79-90), 3 bytes out of two aligned words
+__device__ __forceinline__ uint32_t pick_nearest(uint32_t a0, uint32_t a1, uint32_t sel) { return __byte_perm(a0, a1, sel) & 0xFFFFFFu; }
+
+// the reference's f64 expression for one pixel, p = its p00 in global memory; returns [R G B 0]
+__device__ __forceinline__ uint32_t blend_exact_px(const uint8_t* p, int row_stride, double wx, double wy) {
+    const uint8_t* q = p + row_stride;
+    const double wxi = 1.0 - wx, wyi = 1.0 - wy;
+    const uint32_t r = blend(__ldg(p), __ldg(p + 3), __ldg(q), __ldg(q + 3), wx, wy, wxi, wyi);
+    const uint32_t g = blend(__ldg(p + 1), __ldg(p + 4), __ldg(q + 1), __ldg(q + 4), wx, wy, wxi, wyi);
+    const uint32_t b = blend(__ldg(p + 2), __ldg(p + 5), __ldg(q + 2), __ldg(q + 5), wx, wy, wxi, wyi);
+    return r | (g << 8) | (b << 16);
+}
+
+// Stores a finished patch: px[k] = [R G B .] of this lane's pixel in row k.  The 96 output bytes of a patch row are
+// exchanged with two shuffles so that lane j < 24 stores word j (bytes of pixels 4j/3 and 4j/3 + 1) at dst + 4j.
+// dst: word 0 of row 0 plus 4 * lane; n_rows: rows this lane stores.
+__device__ __forceinline__ void store_patch(const uint32_t px[4], uint8_t* dst, int row_stride, int n_rows) {
+    const int lane = threadIdx.x & 31, src_lane = (4 * lane) / 3;
+    const uint32_t out_sel = (lane % 3 == 0) ? 0x4210u : (lane % 3 == 1) ? 0x5421u : 0x6542u;
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-        const int vo = y0 + k;
-        double sx = 0.0, sy = 0.0;
-        int st = ACM_POINT_IS_OUTSIDE_IMAGE;
-        if (uo < W && vo < H) {
-            const double xn = ((double)uo - tcx) / tfx;
-            const double yn = ((double)vo - tcy) / tfy;
-            st = CamModel<M>::template project<true>(c, xn, yn, 1.0, sx, sy);
-        }
-        const Tap t = make_tap(sx, sy, st, W, H, ACM_INTERP_BILINEAR);
-        off[k] = t.off00; wx[k] = t.wx; wy[k] = t.wy;
-        mode[k] = t.ok ? 1 : 0;
-        const double wxi = 1.0 - t.wx, wyi = 1.0 - t.wy;
-        const uint32_t w00 = __double2uint_rn(wxi * wyi * 16777216.0), w10 = __double2uint_rn(t.wx * wyi * 16777216.0);
-        const uint32_t w01 = __double2uint_rn(wxi * t.wy * 16777216.0), w11 = __double2uint_rn(t.wx * t.wy * 16777216.0);
-        if (t.ok && ((size_t)t.off00 + (size_t)row_stride + 16 > frame_bytes || ((w00 | w10 | w01 | w11) >> 24))) mode[k] = 2;
-        // byte planes, tap order [00, 10, 01, 11]
-        wlo[k] = (w00 & 0xFF) | ((w10 & 0xFF) << 8) | ((w01 & 0xFF) << 16) | ((w11 & 0xFF) << 24);
-        wmid[k] = ((w00 >> 8) & 0xFF) | (((w10 >> 8) & 0xFF) << 8) | (((w01 >> 8) & 0xFF) << 16) | (((w11 >> 8) & 0xFF) << 24);
-        whi[k] = ((w00 >> 16) & 0xFF) | (((w10 >> 16) & 0xFF) << 8) | (((w01 >> 16) & 0xFF) << 16) | (((w11 >> 16) & 0xFF) << 24);
-        sel[k] = 0x3210u + 0x1111u * (uint32_t)(t.off00 & 3);
-        // invalid pixels load from offset 0 (always inside the frame): the 24 tap loads of a thread
-        // are issued back to back, ahead of any math or branch
-        offa[k] = mode[k] == 1 ? (t.off00 & ~3) : 0;
+        const uint32_t pa = __shfl_sync(0xffffffffu, px[k], src_lane);
+        const uint32_t pb = __shfl_sync(0xffffffffu, px[k], (src_lane + 1) & 31);
+        if (k < n_rows) __stcs(reinterpret_cast<uint32_t*>(dst + (size_t)k * row_stride), __byte_perm(pa, pb, out_sel));
     }
-    const bool has_slow = (mode[0] == 2) | (mode[1] == 2) | (mode[2] == 2) | (mode[3] == 2);
-    // output exchange: lane j < 24 stores word j of the 96-byte patch row = bytes of pixels p, p+1
-    const int src_lane = (4 * lane) / 3;
-    const uint32_t out_sel = (lane % 3 == 0) ? 0x4210u : (lane % 3 == 1) ? 0x5421u : 0x6542u;
-    const int valid_px = min(32, W - x0);                     // multiple of 4 because W % 4 == 0
-    const bool store_lane = (lane < 24) && (4 * lane + 3 < 3 * valid_px);
-    for (size_t f = 0; f < n_frames; ++f) {
-        const uint8_t* src = in + f * frame_bytes;
-        uint32_t ta[4][3], tb[4][3];
+}
+
+// ---------------------------------------------------------------------------------------
+// Gather path (W % 4 == 0, 4-byte aligned frames): the taps come from global memory through L1, 3 x LDG.32 per tap row
+// (2 for nearest).  With list == nullptr the grid covers the image: block = 64 x 16 pixels, warp w owns the patch at
+// (w & 1, w >> 1).  Otherwise the warps stride over the patches the TMA kernel below listed (source box larger than its
+// tile).
+// ---------------------------------------------------------------------------------------
+template <int M, bool NEAREST>
+__global__ void __launch_bounds__(256, 3) undistort_gather_kernel(const __grid_constant__ CamParams c, double tfx, double tfy, double tcx,
+                                                               double tcy, const uint8_t* __restrict__ in, uint8_t* __restrict__ out,
+                                                               int W, int H, size_t n_frames, const uint32_t* __restrict__ list,
+                                                               const uint32_t* __restrict__ list_count) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const size_t frame_bytes = (size_t)W * H * 3;
+    const int row_stride = 3 * W;
+    const uint32_t npx = (uint32_t)(W + 31) / 32u;
+    const uint32_t n = list ? *list_count : 1u;  // whole image: one patch per warp, the stride ends the loop
+    for (uint32_t e = list ? blockIdx.x * 8u + warp : 0u; e < n; e += gridDim.x * 8u) {
+        const int x0 = list ? (int)(list[e] % npx) * 32 : blockIdx.x * 64 + (warp & 1) * 32;
+        const int y0 = list ? (int)(list[e] / npx) * 4 : blockIdx.y * 16 + (warp >> 1) * 4;
+        FixedTap tap[4];
+        int offa[4];  // aligned window of the taps
+        uint32_t valid = 0u, slow = 0u;
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
-            const uint32_t* r0 = reinterpret_cast<const uint32_t*>(src + offa[k]);
-            const uint32_t* r1 = reinterpret_cast<const uint32_t*>(src + offa[k] + row_stride);
-            ta[k][0] = __ldg(r0); ta[k][1] = __ldg(r0 + 1); ta[k][2] = __ldg(r0 + 2);
-            tb[k][0] = __ldg(r1); tb[k][1] = __ldg(r1 + 1); tb[k][2] = __ldg(r1 + 2);
+            tap[k] = setup_tap<M, NEAREST>(c, tfx, tfy, tcx, tcy, x0 + lane, y0 + k, W, H);
+            // a window that would read past the end of the frame (the last frame's end for the last pixels) is not read:
+            // the pixel takes the exact path
+            const bool exact = tap[k].slow || (tap[k].t.ok && (size_t)tap[k].t.off00 + (size_t)row_stride + 16 > frame_bytes);
+            valid |= (uint32_t)tap[k].t.ok << k;
+            slow |= (uint32_t)exact << k;
+            // pixels without a sample or taken exactly load from offset 0 (always inside the frame): the tap loads of a
+            // thread are issued back to back, ahead of any math or branch
+            offa[k] = (tap[k].t.ok && !exact) ? (tap[k].t.off00 & ~3) : 0;
         }
-        uint32_t px[4];  // [R G B .] per pixel
-        bool any_tie = false;
+        const int valid_px = min(32, W - x0);  // multiple of 4 because W % 4 == 0
+        const int n_rows = (lane < 24 && 4 * lane + 3 < 3 * valid_px) ? min(4, H - y0) : 0;  // rows this lane stores
+        uint8_t* dst = out + ((size_t)y0 * W + x0) * 3 + 4 * lane;
+        for (size_t f = 0; f < n_frames; ++f, dst += frame_bytes) {
+            const uint8_t* src = in + f * frame_bytes;
+            uint32_t px[4];  // [R G B .] per pixel
+            uint32_t redo = slow;
+            if (NEAREST) {
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const uint32_t A = __byte_perm(ta[k][0], ta[k][1], sel[k]), B = __byte_perm(ta[k][1], ta[k][2], sel[k]);    // [r0 g0 b0 r1] [g1 b1 . .]
-            const uint32_t A2 = __byte_perm(tb[k][0], tb[k][1], sel[k]), B2 = __byte_perm(tb[k][1], tb[k][2], sel[k]);
-            const uint32_t PR = __byte_perm(A, A2, 0x7430);                                       // [r00 r10 r01 r11]
-            const uint32_t T0 = __byte_perm(A, B, 0x5241), T1 = __byte_perm(A2, B2, 0x5241);      // [g0 g1 b0 b1]
-            const uint32_t PG = __byte_perm(T0, T1, 0x5410), PB = __byte_perm(T0, T1, 0x7632);
-            const uint32_t sr = (__dp4a(PR, whi[k], 0u) << 16) + (__dp4a(PR, wmid[k], 0u) << 8) + __dp4a(PR, wlo[k], 1u << 23);
-            const uint32_t sg = (__dp4a(PG, whi[k], 0u) << 16) + (__dp4a(PG, wmid[k], 0u) << 8) + __dp4a(PG, wlo[k], 1u << 23);
-            const uint32_t sb = (__dp4a(PB, whi[k], 0u) << 16) + (__dp4a(PB, wmid[k], 0u) << 8) + __dp4a(PB, wlo[k], 1u << 23);
-            const uint32_t rgb = __byte_perm(__byte_perm(sr, sg, 0x4473), sb, 0x4710);            // [sr.3 sg.3 sb.3 .]
-            const bool tie = (((sr + TIE_E) & 0xFFFFFFu) < 2u * TIE_E) | (((sg + TIE_E) & 0xFFFFFFu) < 2u * TIE_E) |
-                             (((sb + TIE_E) & 0xFFFFFFu) < 2u * TIE_E);
-            px[k] = mode[k] == 1 ? rgb : 0u;
-            if (tie && mode[k] == 1) { any_tie = true; mode[k] = 3; }
-        }
-        if (any_tie || has_slow) {
+                for (int k = 0; k < 4; ++k) {
+                    const uint32_t* r0 = reinterpret_cast<const uint32_t*>(src + offa[k]);
+                    px[k] = ((valid >> k) & 1u) ? pick_nearest(__ldg(r0), __ldg(r0 + 1), tap[k].sel) : 0u;
+                }
+            } else {
+                uint32_t ta[4][3], tb[4][3], tz[4];
 #pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                if (mode[k] >= 2) {
-                    uint8_t o[3];
-                    blend_exact_px(src + off[k], row_stride, wx[k], wy[k], o);
-                    px[k] = o[0] | (o[1] << 8) | ((uint32_t)o[2] << 16);
-                    if (mode[k] == 3) mode[k] = 1;
+                for (int k = 0; k < 4; ++k) {
+                    const uint32_t* r0 = reinterpret_cast<const uint32_t*>(src + offa[k]);
+                    const uint32_t* r1 = reinterpret_cast<const uint32_t*>(src + offa[k] + row_stride);
+                    ta[k][0] = __ldg(r0); ta[k][1] = __ldg(r0 + 1); ta[k][2] = __ldg(r0 + 2);
+                    tb[k][0] = __ldg(r1); tb[k][1] = __ldg(r1 + 1); tb[k][2] = __ldg(r1 + 2);
+                }
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    px[k] = blend_fixed(ta[k][0], ta[k][1], ta[k][2], tb[k][0], tb[k][1], tb[k][2], tap[k].sel, tap[k].wlo, tap[k].w01,
+                                        tap[k].w23, tz[k]);
+                }
+                redo |= tie_bits(tz);
+            }
+            if (redo) {  // rare: these pixels byte by byte from global memory, bilinear with the reference's f64 expression
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    if ((redo >> k) & 1u) {
+                        const uint8_t* p = src + tap[k].t.off00;
+                        px[k] = NEAREST ? (__ldg(p) | (__ldg(p + 1) << 8) | ((uint32_t)__ldg(p + 2) << 16))
+                                        : blend_exact_px(p, row_stride, tap[k].t.wx, tap[k].t.wy);
+                    }
                 }
             }
+            store_patch(px, dst, row_stride, n_rows);
         }
-        uint8_t* dst = out + f * frame_bytes;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const uint32_t pa = __shfl_sync(0xffffffffu, px[k], src_lane);
-            const uint32_t pb = __shfl_sync(0xffffffffu, px[k], (src_lane + 1) & 31);
-            if (store_lane && y0 + k < H) {
-                uint32_t* d32 = reinterpret_cast<uint32_t*>(dst + ((size_t)(y0 + k) * W + x0) * 3) + lane;
-                __stcs(d32, __byte_perm(pa, pb, out_sel));
-            }
-        }
-    }
-}
-
-
-// grid-mapped: block = 64 x 16 output pixels, warp w owns the patch at (w & 1, w >> 1)
-template <int M>
-__global__ void __launch_bounds__(256, 3) undistort_bilinear_fast_kernel(const __grid_constant__ CamParams c, double tfx, double tfy,
-                                                                      double tcx, double tcy, const uint8_t* __restrict__ in,
-                                                                      uint8_t* __restrict__ out, int W, int H, size_t n_frames) {
-    const int warp = threadIdx.x >> 5;
-    undistort_patch_gather<M>(c, tfx, tfy, tcx, tcy, in, out, W, H, n_frames, blockIdx.x * 64 + (warp & 1) * 32, blockIdx.y * 16 + (warp >> 1) * 4);
-}
-
-// list-driven: the patches the TMA kernel below could not stage (source box larger than its tile)
-template <int M>
-__global__ void __launch_bounds__(256, 3) undistort_bilinear_list_kernel(const __grid_constant__ CamParams c, double tfx, double tfy,
-                                                                      double tcx, double tcy, const uint8_t* __restrict__ in,
-                                                                      uint8_t* __restrict__ out, int W, int H, size_t n_frames,
-                                                                      const uint32_t* __restrict__ list, const uint32_t* __restrict__ list_count) {
-    const uint32_t total = *list_count;
-    const uint32_t npx = (uint32_t)(W + 31) / 32u;
-    for (uint32_t e = blockIdx.x * 8u + (threadIdx.x >> 5); e < total; e += gridDim.x * 8u) {
-        const uint32_t pid = list[e];
-        undistort_patch_gather<M>(c, tfx, tfy, tcx, tcy, in, out, W, H, n_frames, (int)(pid % npx) * 32, (int)(pid / npx) * 4);
     }
 }
 
@@ -655,23 +695,17 @@ __global__ void __launch_bounds__(256, 3) undistort_bilinear_list_kernel(const _
 // has no global loads and no address arithmetic left.  The warp is producer and consumer of its
 // own ring, hence no "empty" barriers: the shuffles that exchange the finished pixels order every
 // lane's tile reads before lane 0 re-arms the stage.  Patches whose box does not fit are appended
-// to a list and handled by `undistort_bilinear_list_kernel`.
-// The blend also drops one instruction per channel: the upper 16 bits of the 24-bit weights go
-// through dp2a, the low byte plane through dp4a:  S = (dp2a(hi16) << 8) + dp4a(lo8) + 2^23.
+// to a list and handled by `undistort_gather_kernel`.
 // ---------------------------------------------------------------------------------------
-#define UND_BOX_W 128
-#define UND_BOX_ROWS 10      // tallest box (the shared-memory tile holds this many rows)
-#define UND_MIN_ROWS 4       // one tensor map per box height UND_MIN_ROWS .. UND_BOX_ROWS: a warp fetches only the rows it needs
+constexpr int UND_BOX_W = 128;
+constexpr int UND_BOX_ROWS = 10;  // tallest box (the shared-memory tile holds this many rows)
+constexpr int UND_MIN_ROWS = 4;   // one tensor map per box height UND_MIN_ROWS .. UND_BOX_ROWS: a warp fetches only the rows it needs
 // Round 2, same-box A/B (4096^2, 32 frames): 4 stages x 1 frame 39.2 / 23.9 us per frame (bilinear / nearest), 2 stages x 2
 // frames 38.4 / 21.6 (one barrier wait and one re-arm per two frames), 3 x 2 and 6 x 1 slower (shared memory costs a resident
 // block).  Addressing the output rows as a warp-uniform frame base + 32-bit lane offsets instead of a per-lane pointer
 // that is advanced per frame cost 18 % in the bilinear kernel (46.3 us) -- kept out.
-#ifndef UND_STAGES
-#define UND_STAGES 2       // ring depth in stages
-#endif
-#ifndef UND_FPS
-#define UND_FPS 2          // frames per stage: one TMA box {UND_BOX_W, rows, UND_FPS}, one barrier wait and one re-arm per UND_FPS frames
-#endif
+constexpr int UND_STAGES = 2;  // ring depth in stages
+constexpr int UND_FPS = 2;     // frames per stage: one TMA box {UND_BOX_W, rows, UND_FPS}, one barrier wait and one re-arm per UND_FPS frames
 
 struct UndMaps { CUtensorMap m[UND_BOX_ROWS - UND_MIN_ROWS + 1]; };
 
@@ -694,12 +728,10 @@ __device__ __forceinline__ void und_tma_load_3d(uint32_t dst, const void* map, u
 }
 
 template <int M, bool NEAREST>
-__global__ void __launch_bounds__(256, 3) undistort_bilinear_tma_kernel(const __grid_constant__ CamParams c, double tfx, double tfy,
-                                                                     double tcx, double tcy, const __grid_constant__ UndMaps in_maps,
-                                                                     const uint8_t* __restrict__ in, uint8_t* __restrict__ out, int W,
-                                                                     int H, int n_frames, uint32_t* __restrict__ list,
-                                                                     uint32_t* __restrict__ list_count) {
-    constexpr uint32_t TIE_E = 640u;
+__global__ void __launch_bounds__(256, 3) undistort_tma_kernel(const __grid_constant__ CamParams c, double tfx, double tfy, double tcx,
+                                                            double tcy, const __grid_constant__ UndMaps in_maps,
+                                                            const uint8_t* __restrict__ in, uint8_t* __restrict__ out, int W, int H,
+                                                            int n_frames, uint32_t* __restrict__ list, uint32_t* __restrict__ list_count) {
     constexpr int TILE = UND_FPS * UND_BOX_W * UND_BOX_ROWS;   // one stage = UND_FPS frames of the box
     // dynamic shared memory: tiles[8 warps][STAGES][TILE] | mbarriers[8][STAGES] | wx[4][256] | wy[4][256]
     // (the f64 weights are only read by the rare exact re-blend; keeping them out of registers is what
@@ -713,46 +745,24 @@ __global__ void __launch_bounds__(256, 3) undistort_bilinear_tma_kernel(const __
     const int x0 = blockIdx.x * 64 + (warp & 1) * 32;        // patch origin
     const int y0 = blockIdx.y * 16 + (warp >> 1) * 4;
     if (x0 >= W || y0 >= H) return;                          // warp-uniform; nothing block-wide follows
-    const int uo = x0 + lane;
     const size_t frame_bytes = (size_t)W * H * 3;
     const int row_stride = 3 * W;
-    // Pixels without a sample keep all-zero weights: their blend is 2^23 >> 24 = 0 (black) and can never
-    // look like a tie, so the frame loop needs no per-pixel mode test.  `slow` marks the pixels that must
-    // always take the exact f64 expression (a weight of exactly 1).
     int off[4];
     uint32_t sel[4], wlo[4], w01[4], w23[4];
     uint32_t valid = 0u, slow = 0u;
     int bx_min = 0x7fffffff, bx_max = -1, by_min = 0x7fffffff, by_max = -1;
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-        const int vo = y0 + k;
-        double sx = 0.0, sy = 0.0;
-        int st = ACM_POINT_IS_OUTSIDE_IMAGE;
-        if (uo < W && vo < H) {
-            const double xn = ((double)uo - tcx) / tfx;
-            const double yn = ((double)vo - tcy) / tfy;
-            st = CamModel<M>::template project<true>(c, xn, yn, 1.0, sx, sy);
-        }
-        const Tap t = make_tap(sx, sy, st, W, H, NEAREST ? ACM_INTERP_NEAREST : ACM_INTERP_BILINEAR);
-        off[k] = t.off00;
-        if (!NEAREST) { s_wx[k * 256 + threadIdx.x] = t.wx; s_wy[k * 256 + threadIdx.x] = t.wy; }
-        const double wxi = 1.0 - t.wx, wyi = 1.0 - t.wy;
-        uint32_t w00 = __double2uint_rn(wxi * wyi * 16777216.0), w10 = __double2uint_rn(t.wx * wyi * 16777216.0);
-        uint32_t w01_ = __double2uint_rn(wxi * t.wy * 16777216.0), w11 = __double2uint_rn(t.wx * t.wy * 16777216.0);
-        if (t.ok) {
+        const FixedTap p = setup_tap<M, NEAREST>(c, tfx, tfy, tcx, tcy, x0 + lane, y0 + k, W, H);
+        off[k] = p.t.off00; sel[k] = p.sel; wlo[k] = p.wlo; w01[k] = p.w01; w23[k] = p.w23;
+        if (!NEAREST) { s_wx[k * 256 + threadIdx.x] = p.t.wx; s_wy[k * 256 + threadIdx.x] = p.t.wy; }
+        slow |= (uint32_t)p.slow << k;
+        if (p.t.ok) {
             valid |= 1u << k;
-            if (!NEAREST && ((w00 | w10 | w01_ | w11) >> 24)) slow |= 1u << k;
-            const int ty = t.off00 / row_stride, tb = t.off00 - ty * row_stride;
+            const int ty = p.t.off00 / row_stride, tb = p.t.off00 - ty * row_stride;
             bx_min = min(bx_min, tb); bx_max = max(bx_max, tb + (NEAREST ? 2 : 5));
             by_min = min(by_min, ty); by_max = max(by_max, ty + (NEAREST ? 0 : 1));
-        } else {
-            w00 = w10 = w01_ = w11 = 0u;
         }
-        // tap order [00, 10, 01, 11]: low byte plane for dp4a, upper 16 bits pairwise for dp2a
-        wlo[k] = (w00 & 0xFF) | ((w10 & 0xFF) << 8) | ((w01_ & 0xFF) << 16) | ((w11 & 0xFF) << 24);
-        w01[k] = ((w00 >> 8) & 0xFFFF) | (((w10 >> 8) & 0xFFFF) << 16);
-        w23[k] = ((w01_ >> 8) & 0xFFFF) | (((w11 >> 8) & 0xFFFF) << 16);
-        sel[k] = 0x3210u + 0x1111u * (uint32_t)(t.off00 & 3);
     }
     bx_min = __reduce_min_sync(0xffffffffu, bx_min); bx_max = __reduce_max_sync(0xffffffffu, bx_max);
     by_min = __reduce_min_sync(0xffffffffu, by_min); by_max = __reduce_max_sync(0xffffffffu, by_max);
@@ -774,8 +784,6 @@ __global__ void __launch_bounds__(256, 3) undistort_bilinear_tma_kernel(const __
         const int ty = off[k] / row_stride, tb = off[k] - ty * row_stride;
         so[k] = tile0 + (((valid >> k) & 1u) ? (uint32_t)((ty - box_y) * UND_BOX_W + ((tb - box_x) & ~3)) : 0u);
     }
-    const int src_lane = (4 * lane) / 3;
-    const uint32_t out_sel = (lane % 3 == 0) ? 0x4210u : (lane % 3 == 1) ? 0x5421u : 0x6542u;
     const int valid_px = min(32, W - x0);                     // multiple of 4 because W % 16 == 0
     const int n_rows = (lane < 24 && 4 * lane + 3 < 3 * valid_px) ? min(4, H - y0) : 0;  // rows this lane stores
     if (lane == 0) {
@@ -816,16 +824,16 @@ __global__ void __launch_bounds__(256, 3) undistort_bilinear_tma_kernel(const __
             if (any_valid) {
                 const uint32_t tile_off = stage_off + (uint32_t)h * frame_stride;
                 uint32_t redo = slow;
-                uint32_t tz[4];
-                if (NEAREST) {  // the sample is the pixel itself (undistort.rs:79-90): 3 bytes out of two aligned words
+                if (NEAREST) {
 #pragma unroll
                     for (int k = 0; k < 4; ++k) {
                         uint32_t a0, a1;
                         const uint32_t addr = so[k] + tile_off;
                         asm volatile("ld.shared.u32 %0, [%2];\n ld.shared.u32 %1, [%2+4];" : "=r"(a0), "=r"(a1) : "r"(addr));
-                        px[k] = ((valid >> k) & 1u) ? (__byte_perm(a0, a1, sel[k]) & 0xFFFFFFu) : 0u;
+                        px[k] = ((valid >> k) & 1u) ? pick_nearest(a0, a1, sel[k]) : 0u;
                     }
                 } else {
+                    uint32_t tz[4];
 #pragma unroll
                     for (int k = 0; k < 4; ++k) {
                         uint32_t a0, a1, a2, b0, b1, b2;
@@ -833,23 +841,9 @@ __global__ void __launch_bounds__(256, 3) undistort_bilinear_tma_kernel(const __
                         asm volatile("ld.shared.u32 %0, [%6];\n ld.shared.u32 %1, [%6+4];\n ld.shared.u32 %2, [%6+8];\n"
                                      "ld.shared.u32 %3, [%6+128];\n ld.shared.u32 %4, [%6+132];\n ld.shared.u32 %5, [%6+136];"
                                      : "=r"(a0), "=r"(a1), "=r"(a2), "=r"(b0), "=r"(b1), "=r"(b2) : "r"(addr));
-                        const uint32_t A = __byte_perm(a0, a1, sel[k]), B = __byte_perm(a1, a2, sel[k]);     // [r0 g0 b0 r1] [g1 b1 . .]
-                        const uint32_t A2 = __byte_perm(b0, b1, sel[k]), B2 = __byte_perm(b1, b2, sel[k]);
-                        const uint32_t PR = __byte_perm(A, A2, 0x7430);                                       // [r00 r10 r01 r11]
-                        const uint32_t T0 = __byte_perm(A, B, 0x5241), T1 = __byte_perm(A2, B2, 0x5241);      // [g0 g1 b0 b1]
-                        const uint32_t PG = __byte_perm(T0, T1, 0x5410), PB = __byte_perm(T0, T1, 0x7632);
-                        const uint32_t sr = (__dp2a_hi(w23[k], PR, __dp2a_lo(w01[k], PR, 0u)) << 8) + __dp4a(PR, wlo[k], 1u << 23);
-                        const uint32_t sg = (__dp2a_hi(w23[k], PG, __dp2a_lo(w01[k], PG, 0u)) << 8) + __dp4a(PG, wlo[k], 1u << 23);
-                        const uint32_t sb = (__dp2a_hi(w23[k], PB, __dp2a_lo(w01[k], PB, 0u)) << 8) + __dp4a(PB, wlo[k], 1u << 23);
-                        px[k] = __byte_perm(__byte_perm(sr, sg, 0x4473), sb, 0x4710);                         // [sr.3 sg.3 sb.3 .]
-                        // distance of the 24-bit fraction to a rounding tie, scaled by 2^8 so that the 32-bit wrap does the
-                        // masking: ((s + E) mod 2^24) < 2E  <=>  (s * 2^8 + E * 2^8) mod 2^32 < 2E * 2^8
-                        tz[k] = min(min(sr * 256u + TIE_E * 256u, sg * 256u + TIE_E * 256u), sb * 256u + TIE_E * 256u);
+                        px[k] = blend_fixed(a0, a1, a2, b0, b1, b2, sel[k], wlo[k], w01[k], w23[k], tz[k]);
                     }
-                    if (min(min(tz[0], tz[1]), min(tz[2], tz[3])) < 2u * TIE_E * 256u) {
-#pragma unroll
-                        for (int k = 0; k < 4; ++k) redo |= (tz[k] < 2u * TIE_E * 256u ? 1u : 0u) << k;
-                    }
+                    redo |= tie_bits(tz);
                 }
                 if (redo) {  // rare: redo these pixels with the reference's f64 expression from global memory
                     const uint8_t* src = in + (size_t)f * frame_bytes;
@@ -859,19 +853,12 @@ __global__ void __launch_bounds__(256, 3) undistort_bilinear_tma_kernel(const __
                             // rebuild the byte offset of p00 from the tile address and the byte selector
                             const uint32_t rel = so[k] - tile0;
                             const int o00 = (box_y + (int)(rel / UND_BOX_W)) * row_stride + box_x + (int)(rel % UND_BOX_W) + (int)(sel[k] & 3u);
-                            uint8_t o[3];
-                            blend_exact_px(src + o00, row_stride, s_wx[k * 256 + threadIdx.x], s_wy[k * 256 + threadIdx.x], o);
-                            px[k] = o[0] | (o[1] << 8) | ((uint32_t)o[2] << 16);
+                            px[k] = blend_exact_px(src + o00, row_stride, s_wx[k * 256 + threadIdx.x], s_wy[k * 256 + threadIdx.x]);
                         }
                     }
                 }
             }
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                const uint32_t pa = __shfl_sync(0xffffffffu, px[k], src_lane);
-                const uint32_t pb = __shfl_sync(0xffffffffu, px[k], (src_lane + 1) & 31);
-                if (k < n_rows) __stcs(reinterpret_cast<uint32_t*>(dst + (size_t)k * row_stride), __byte_perm(pa, pb, out_sel));
-            }
+            store_patch(px, dst, row_stride, n_rows);
             dst += frame_bytes;
         }
         // every lane's tile reads of this stage have been consumed by the shuffles above
@@ -880,36 +867,6 @@ __global__ void __launch_bounds__(256, 3) undistort_bilinear_tma_kernel(const __
             und_tma_load_3d(tile0 + stage * TILE, in_map, bar0 + 8 * stage, box_x, box_y, f0 + UND_STAGES * UND_FPS);
         }
         if (++stage == UND_STAGES) { stage = 0; parity ^= 1u; }
-    }
-}
-
-// nearest-neighbour leftovers of the TMA kernel (patches whose source box does not fit its tile):
-// one warp per listed patch, byte loads / stores -- never on the hot path
-template <int M>
-__global__ void __launch_bounds__(256) undistort_list_generic_kernel(const __grid_constant__ CamParams c, double tfx, double tfy, double tcx,
-                                                                     double tcy, const uint8_t* __restrict__ in, uint8_t* __restrict__ out,
-                                                                     int W, int H, size_t n_frames, int interp,
-                                                                     const uint32_t* __restrict__ list, const uint32_t* __restrict__ list_count) {
-    const uint32_t total = *list_count;
-    const uint32_t npx = (uint32_t)(W + 31) / 32u;
-    const int lane = threadIdx.x & 31;
-    const size_t frame_bytes = (size_t)W * H * 3;
-    for (uint32_t e = blockIdx.x * 8u + (threadIdx.x >> 5); e < total; e += gridDim.x * 8u) {
-        const uint32_t pid = list[e];
-        const int uo = (int)(pid % npx) * 32 + lane, y0 = (int)(pid / npx) * 4;
-        for (int k = 0; k < 4; ++k) {
-            const int vo = y0 + k;
-            if (uo >= W || vo >= H) continue;
-            double sx = 0.0, sy = 0.0;
-            const double xn = ((double)uo - tcx) / tfx, yn = ((double)vo - tcy) / tfy;
-            const int st = CamModel<M>::template project<true>(c, xn, yn, 1.0, sx, sy);
-            const Tap t = make_tap(sx, sy, st, W, H, interp);
-            for (size_t f = 0; f < n_frames; ++f) {
-                uint8_t* d = out + f * frame_bytes + ((size_t)vo * W + uo) * 3;
-                const uint8_t* p = in + f * frame_bytes + t.off00;
-                d[0] = t.ok ? __ldg(p) : 0; d[1] = t.ok ? __ldg(p + 1) : 0; d[2] = t.ok ? __ldg(p + 2) : 0;
-            }
-        }
     }
 }
 
@@ -961,6 +918,32 @@ static int32_t check_undistort_args(acm_ctx* ctx, const acm_camera* cam, const d
     return ACM_OK;
 }
 
+// maps != nullptr: the TMA kernel, then the gather over the patches it lists (list = d_count + 64);
+// gather: the gather over the whole image; otherwise the generic byte kernel
+template <int M, bool NEAREST>
+static int32_t launch_undistort(acm_ctx* ctx, const CamParams& c, const double* t, const UndMaps* maps, bool gather, const uint8_t* d_in,
+                                uint8_t* d_out, int W, int H, size_t n_frames, uint32_t* d_count) {
+    const dim3 patch_grid((W + 63) / 64, (H + 15) / 16);  // block = 64 x 16 output pixels
+    if (maps) {
+        constexpr int smem = 8 * UND_STAGES * UND_FPS * UND_BOX_W * UND_BOX_ROWS + 8 * UND_STAGES * 8 + 2 * 4 * 256 * 8;
+        uint32_t* const d_list = d_count + 64;
+        cudaFuncSetAttribute(undistort_tma_kernel<M, NEAREST>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        undistort_tma_kernel<M, NEAREST><<<patch_grid, 256, smem, ctx->stream>>>(c, t[0], t[1], t[2], t[3], *maps, d_in, d_out, W, H, (int)n_frames,
+                                                                               d_list, d_count);
+        ACM_CHECK_LAUNCH(ctx);
+        undistort_gather_kernel<M, NEAREST><<<ctx->sm_count * 3, 256, 0, ctx->stream>>>(c, t[0], t[1], t[2], t[3], d_in, d_out, W, H, n_frames,
+                                                                                       d_list, d_count);
+    } else if (gather) {
+        undistort_gather_kernel<M, NEAREST><<<patch_grid, 256, 0, ctx->stream>>>(c, t[0], t[1], t[2], t[3], d_in, d_out, W, H, n_frames, nullptr,
+                                                                               nullptr);
+    } else {
+        undistort_kernel<M><<<dim3((W + 1023) / 1024, H), 256, 0, ctx->stream>>>(c, t[0], t[1], t[2], t[3], d_in, d_out, W, H, n_frames,
+                                                                                NEAREST ? ACM_INTERP_NEAREST : ACM_INTERP_BILINEAR);
+    }
+    ACM_CHECK_LAUNCH(ctx);
+    return ACM_OK;
+}
+
 extern "C" int32_t acm_undistort_rgb8(acm_ctx* ctx, const acm_camera* cam, const double* target_intrinsics, const uint8_t* d_in,
                                       uint8_t* d_out, size_t n_frames, int32_t interpolation) {
     ACM_ENTER(ctx);
@@ -974,40 +957,24 @@ extern "C" int32_t acm_undistort_rgb8(acm_ctx* ctx, const acm_camera* cam, const
     rc = acm_make_cam_params(ctx, cam, &c);
     if (rc) return rc;
     const int W = (int)cam->width, H = (int)cam->height;
-    dim3 grid((W + 1023) / 1024, H);
-    const bool aligned = ((reinterpret_cast<uintptr_t>(d_in) & 3) == 0) && ((reinterpret_cast<uintptr_t>(d_out) & 3) == 0) && (W % 4 == 0);
-    const bool tma_ok = ((reinterpret_cast<uintptr_t>(d_in) & 15) == 0) && (W % 16 == 0) && n_frames < 0x7fffffffULL;
-    UndMaps map;
-    bool have_maps = aligned && tma_ok;
-    for (int r = UND_MIN_ROWS; have_maps && r <= UND_BOX_ROWS; ++r) have_maps = make_frame_tensor_map(&map.m[r - UND_MIN_ROWS], d_in, W, H, n_frames, r);
-    if (have_maps) {
-        dim3 fgrid((W + 63) / 64, (H + 15) / 16);
+    const uintptr_t in_addr = reinterpret_cast<uintptr_t>(d_in), out_addr = reinterpret_cast<uintptr_t>(d_out);
+    const bool gather = W % 4 == 0 && (in_addr & 3) == 0 && (out_addr & 3) == 0;
+    UndMaps maps;
+    bool tma = gather && W % 16 == 0 && (in_addr & 15) == 0 && n_frames < 0x7fffffffULL;
+    for (int r = UND_MIN_ROWS; tma && r <= UND_BOX_ROWS; ++r) tma = make_frame_tensor_map(&maps.m[r - UND_MIN_ROWS], d_in, W, H, n_frames, r);
+    uint32_t* d_count = nullptr;
+    if (tma) {
         // leftover list: [count][patch ids], one id per 32 x 4 patch at most
         const size_t n_patches = (size_t)((W + 31) / 32) * (size_t)((H + 3) / 4);
         rc = acm_ensure_scratch(ctx, 256 + n_patches * sizeof(uint32_t));
         if (rc) return rc;
-        uint32_t* d_count = static_cast<uint32_t*>(ctx->d_scratch);
-        uint32_t* d_list = d_count + 64;
+        d_count = static_cast<uint32_t*>(ctx->d_scratch);
         ACM_CUDA(ctx, cudaMemsetAsync(d_count, 0, sizeof(uint32_t), ctx->stream));
-        constexpr int und_smem_bytes = 8 * UND_STAGES * UND_FPS * UND_BOX_W * UND_BOX_ROWS + 8 * UND_STAGES * 8 + 2 * 4 * 256 * 8;
-        if (interpolation == ACM_INTERP_BILINEAR) {
-            ACM_DISPATCH_MODEL(cam->model, (cudaFuncSetAttribute(undistort_bilinear_tma_kernel<M, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, und_smem_bytes)))
-            ACM_DISPATCH_MODEL(cam->model, (undistort_bilinear_tma_kernel<M, false><<<fgrid, 256, und_smem_bytes, ctx->stream>>>(c, t[0], t[1], t[2], t[3], map, d_in, d_out, W, H, (int)n_frames, d_list, d_count)))
-            ACM_CHECK_LAUNCH(ctx);
-            ACM_DISPATCH_MODEL(cam->model, (undistort_bilinear_list_kernel<M><<<ctx->sm_count * 3, 256, 0, ctx->stream>>>(c, t[0], t[1], t[2], t[3], d_in, d_out, W, H, n_frames, d_list, d_count)))
-        } else {
-            ACM_DISPATCH_MODEL(cam->model, (cudaFuncSetAttribute(undistort_bilinear_tma_kernel<M, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, und_smem_bytes)))
-            ACM_DISPATCH_MODEL(cam->model, (undistort_bilinear_tma_kernel<M, true><<<fgrid, 256, und_smem_bytes, ctx->stream>>>(c, t[0], t[1], t[2], t[3], map, d_in, d_out, W, H, (int)n_frames, d_list, d_count)))
-            ACM_CHECK_LAUNCH(ctx);
-            ACM_DISPATCH_MODEL(cam->model, (undistort_list_generic_kernel<M><<<ctx->sm_count * 3, 256, 0, ctx->stream>>>(c, t[0], t[1], t[2], t[3], d_in, d_out, W, H, n_frames, interpolation, d_list, d_count)))
-        }
-    } else if (interpolation == ACM_INTERP_BILINEAR && aligned) {
-        dim3 fgrid((W + 63) / 64, (H + 15) / 16);
-        ACM_DISPATCH_MODEL(cam->model, (undistort_bilinear_fast_kernel<M><<<fgrid, 256, 0, ctx->stream>>>(c, t[0], t[1], t[2], t[3], d_in, d_out, W, H, n_frames)))
-    } else {
-        ACM_DISPATCH_MODEL(cam->model, (undistort_kernel<M><<<grid, 256, 0, ctx->stream>>>(c, t[0], t[1], t[2], t[3], d_in, d_out, W, H, n_frames, interpolation)))
     }
-    ACM_CHECK_LAUNCH(ctx);
+    const UndMaps* const tma_maps = tma ? &maps : nullptr;
+    ACM_DISPATCH_MODEL(cam->model, return interpolation == ACM_INTERP_NEAREST
+                                              ? launch_undistort<M, true>(ctx, c, t, tma_maps, gather, d_in, d_out, W, H, n_frames, d_count)
+                                              : launch_undistort<M, false>(ctx, c, t, tma_maps, gather, d_in, d_out, W, H, n_frames, d_count))
     return ACM_OK;
 }
 

@@ -972,8 +972,9 @@ def test_reprojection_error_matches_oracle(acm, ctx, O, cameras, name):
                                       ("double_sphere", 756, 480)])
 def test_undistort_bytes_and_remap_indices(acm, ctx, O, cameras, name, W, H):
     """undistort.rs:14-105: output bytes and remap indices are bit-exact (KB / FOV depend on the
-    device atan2: count index flips, expected 0).  Widths that are multiples of 16 take the TMA kernel, 756 (a multiple
-    of 4 only) the whole-image gather kernel when bilinear, 37 the generic one."""
+    device atan2: count index flips, expected 0).  Widths that are multiples of 16 take the TMA kernel (and the gather
+    kernel for the patches of the 0.6x target it lists), 756 (a multiple of 4 only) the whole-image gather kernel, 37 the
+    generic one."""
     cam = dict(cameras[name]); cam["width"], cam["height"] = W, H
     if name in ("ucm", "fov"):  # keep the principal point inside the test image
         cam["params"] = list(cam["params"]); cam["params"][2] = W / 2.0 + 0.3; cam["params"][3] = H / 2.0 - 0.2
@@ -1002,8 +1003,34 @@ def test_undistort_bytes_and_remap_indices(acm, ctx, O, cameras, name, W, H):
         acm.undistort_image(np.zeros((H + 1, W, 3), np.uint8), m)
 
 
+@pytest.mark.parametrize("in_shift,out_shift", [(1, 1), (1, 0), (0, 1)])
+def test_undistort_unaligned_device_buffers(acm, ctx, O, cameras, in_shift, out_shift):
+    """Frame buffers 1 byte off their allocation at a width that is a multiple of 16: neither the TMA nor the gather
+    kernel may take them (both read aligned words), the generic byte kernel does.  Bytes equal the oracle's."""
+    from apex_camera_models_b200 import _native as N
+    cam = dict(cameras["kannala_brandt"]); W, H, F = 512, 512, 3
+    m, om = gpu_model(acm, ctx, cam), oracle_model(O, cam)
+    blk = m.camera_block()
+    frames = O.synth_bytes(0xACE50007, 0, F * W * H * 3).reshape(F, H, W, 3)
+    nb = frames.nbytes
+    d_in, d_out = ctx.device_alloc(nb + 16), ctx.device_alloc(nb + 16)
+    try:
+        ctx.h2d(d_in + in_shift, frames)
+        for target in (None, [cam["params"][0] * 0.6, cam["params"][1] * 0.6, W / 2.0, H / 2.0]):
+            t = cam["params"][:4] if target is None else target
+            for interp in (acm.InterpolationMethod.Bilinear, acm.InterpolationMethod.Nearest):
+                ctx.check(N.lib.acm_undistort_rgb8(ctx.handle, C.byref(blk), None if target is None else (C.c_double * 4)(*target),
+                                                   C.c_void_p(d_in + in_shift), C.c_void_p(d_out + out_shift), F, int(interp)))
+                out = np.empty_like(frames); ctx.d2h(out, d_out + out_shift); ctx.sync()
+                for f in range(F):
+                    ref = O.undistort_rgb8(om, t, frames[f], int(interp), nthreads=4)
+                    assert np.array_equal(out[f], ref), f"frame {f} interp {interp} target {target}: {(out[f] != ref).sum()} bytes differ"
+    finally:
+        ctx.device_free(d_in); ctx.device_free(d_out)
+
+
 def test_undistort_many_frames_ring_wraparound(acm, ctx, O, cameras):
-    """The TMA path keeps 4 frames in flight per warp: 11 frames take every stage through three
+    """The TMA path keeps 2 stages x 2 frames in flight per warp: 11 frames take every stage through three
     phases of its mbarrier; the bytes of every frame must still equal the oracle's."""
     cam = dict(cameras["kannala_brandt"]); W, H = 512, 512
     m, om = gpu_model(acm, ctx, cam), oracle_model(O, cam)
