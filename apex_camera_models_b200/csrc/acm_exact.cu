@@ -8,6 +8,8 @@
 // per thread (2 f64 or 4 f32 points), grid-stride loop over a grid of sm_count * k blocks.
 #include <stdlib.h>
 
+#include <new>
+
 #include <cuda.h>
 
 #include "acm_models.cuh"
@@ -396,11 +398,8 @@ int32_t acm_small_map(acm_ctx* ctx, const acm_camera* cam, const double* d_in, d
 
 // ---------------------------------------------------------------------------------------
 // undistort_image: per output pixel  ray = ((u-cx_t)/fx_t, (v-cy_t)/fy_t, 1) -> project ->
-// bilinear / nearest sample (undistort.rs:33-46, :51-105).  One thread owns 4 horizontally
-// adjacent output pixels: it evaluates their source coordinates once, then loops over the
-// frames of the batch (the map is never stored), gathers the taps through the read-only
-// path and stages the 12 output bytes in shared memory so that the block writes the row
-// segment with 16-byte coalesced stores.
+// bilinear / nearest sample (undistort.rs:33-46, :51-105).  Remap plans: the same sample at a
+// source coordinate computed once per plan (acm_remap_plan below).
 // ---------------------------------------------------------------------------------------
 struct Tap {
     int ok;        // sample exists
@@ -434,35 +433,156 @@ __device__ __forceinline__ uint8_t blend(uint8_t p00, uint8_t p10, uint8_t p01, 
     return (uint8_t)r;
 }
 
-template <int M>
-__global__ void __launch_bounds__(256) undistort_kernel(const __grid_constant__ CamParams c, double tfx, double tfy, double tcx,
-                                                        double tcy, const uint8_t* __restrict__ in, uint8_t* __restrict__ out,
-                                                        int W, int H, size_t n_frames, int interp) {
+// ---------------------------------------------------------------------------------------
+// Per-pixel work of the TMA and gather kernels below.  Byte-exact by construction:
+//  * The reference blends in f64 (undistort.rs:92-99) and rounds half away from zero.  Here the
+//    four tap weights are quantised once per output pixel to 24-bit fixed point
+//    (W_i = rn(w_i * 2^24), sum <= 2^24 + 2, so sum p_i W_i fits 32 bits).
+//    |S / 2^24 - sum p_i w_i| <= 4 * 255 * 2^-25 = 3.04e-5 and the f64 evaluation order of the
+//    reference moves the value by < 1e-12, so whenever the fractional part of S + 0.5 is farther
+//    than E = 640 / 2^24 = 3.8e-5 from an integer both round to the same byte.  Otherwise
+//    (probability 7.6e-5 per channel) the pixel is redone with the reference's exact f64
+//    expression, as are pixels with a weight of exactly 1.
+//  * Instruction diet (the first gather kernel was issue-bound at 151 instr/pixel): each 6-byte tap
+//    run is three aligned 32-bit words + two PRMT with a per-pixel selector; five more PRMT gather the
+//    four taps of each channel into one register; the blend is S = (dp2a(hi16) << 8) + dp4a(lo8) + 2^23
+//    per channel: the upper 16 bits of the weights pairwise through dp2a, the low byte plane through dp4a.
+// Thread <-> pixel mapping: a warp owns a 32-wide, 4-tall output patch, lane = x.  Neighbouring
+// lanes then read neighbouring source pixels (3 bytes apart), so one warp-wide 32-bit load touches
+// ~4 sectors instead of the ~17 of a "4 consecutive pixels per thread" mapping (ncu: the first
+// mapping was bound by L1 sector look-ups, 444 M per 8 frames).
+// ---------------------------------------------------------------------------------------
+constexpr uint32_t UND_TIE_E = 640u;
+
+// One output pixel, set up once and reused for every frame.
+struct FixedTap {
+    Tap t;
+    uint32_t sel;            // PRMT selector of the sample's bytes in its 4-byte-aligned window
+    uint32_t wlo, w01, w23;  // 24-bit weights, tap order [00, 10, 01, 11]: low byte plane for dp4a, upper 16 bits pairwise
+                             // for dp2a.  All zero without a sample: the blend is then 2^23 >> 24 = 0 (black) and can never
+                             // look like a tie, so the frame loops need no per-pixel mode test.
+    bool slow;               // bilinear with a weight of exactly 1: always takes the exact f64 expression
+};
+
+// The tap of a source coordinate (sx, sy) on a W x H input, `st` the status of the step that produced it.  The model source
+// below calls it per launch, remap_pack_kernel once per plan: both give the same bits.
+template <bool NEAREST>
+__device__ __forceinline__ FixedTap tap_from_coord(double sx, double sy, int st, int W, int H) {
+    FixedTap p;
+    p.t = make_tap(sx, sy, st, W, H, NEAREST ? ACM_INTERP_NEAREST : ACM_INTERP_BILINEAR);
+    const double wxi = 1.0 - p.t.wx, wyi = 1.0 - p.t.wy;
+    uint32_t w00 = __double2uint_rn(wxi * wyi * 16777216.0), w10 = __double2uint_rn(p.t.wx * wyi * 16777216.0);
+    uint32_t w01 = __double2uint_rn(wxi * p.t.wy * 16777216.0), w11 = __double2uint_rn(p.t.wx * p.t.wy * 16777216.0);
+    if (!p.t.ok) w00 = w10 = w01 = w11 = 0u;
+    p.slow = !NEAREST && ((w00 | w10 | w01 | w11) >> 24) != 0u;
+    p.wlo = (w00 & 0xFF) | ((w10 & 0xFF) << 8) | ((w01 & 0xFF) << 16) | ((w11 & 0xFF) << 24);
+    p.w01 = ((w00 >> 8) & 0xFFFF) | (((w10 >> 8) & 0xFFFF) << 16);
+    p.w23 = ((w01 >> 8) & 0xFFFF) | (((w11 >> 8) & 0xFFFF) << 16);
+    p.sel = 0x3210u + 0x1111u * (uint32_t)(p.t.off00 & 3);
+    return p;
+}
+
+// Where the frame kernels get their taps.  W x H is the output grid.
+//  * ModelSrc<M>: undistort_image computes each pixel's source coordinate per launch (the ray through the target pinhole,
+//    then CamModel<M>::project, undistort.rs:33-46); input and output grids are the camera's.
+//  * PlanSrc: an acm_remap_plan's record (remap_pack_kernel) per pixel on any Wi x Hi input.  The plan's f64 map is read
+//    only where the f64 weights are needed: by the byte kernel and by the rare exact re-blend.
+// coord(): source coordinate and status; tap(): FixedTap; in_w / in_h: the input grid.
+template <int M> struct ModelSrc {
+    static constexpr bool PLAN = false;
+    CamParams c;
+    double tfx, tfy, tcx, tcy;  // target intrinsics
+    __device__ __forceinline__ int in_w(int W) const { return W; }
+    __device__ __forceinline__ int in_h(int H) const { return H; }
+    __device__ __forceinline__ int coord(int uo, int vo, int W, int H, double& sx, double& sy) const {
+        const double xn = ((double)uo - tcx) / tfx;  // outside the branch: the 4 pixels of a lane share it
+        sx = 0.0; sy = 0.0;
+        int st = ACM_POINT_IS_OUTSIDE_IMAGE;
+        if (uo < W && vo < H) {
+            const double yn = ((double)vo - tcy) / tfy;
+            st = CamModel<M>::template project<true>(c, xn, yn, 1.0, sx, sy);
+        }
+        return st;
+    }
+    template <bool NEAREST> __device__ __forceinline__ FixedTap tap(int uo, int vo, int W, int H) const {
+        double sx, sy;
+        const int st = coord(uo, vo, W, H, sx, sy);
+        return tap_from_coord<NEAREST>(sx, sy, st, W, H);
+    }
+};
+
+// Plan record, one per output pixel (16 B): x = input pixel index of the tap (bits 0-29; 3 * Wi * Hi < 2^31) | slow << 30 |
+// valid << 31, then wlo, w01, w23 of FixedTap.
+struct PlanSrc {
+    static constexpr bool PLAN = true;
+    const uint4* rec;
+    const double2* map;  // (sx, sy) per output pixel, NaN where there is no sample
+    int Wi, Hi;
+    __device__ __forceinline__ int in_w(int) const { return Wi; }
+    __device__ __forceinline__ int in_h(int) const { return Hi; }
+    __device__ __forceinline__ int coord(int uo, int vo, int W, int H, double& sx, double& sy) const {
+        sx = 0.0; sy = 0.0;
+        if (uo >= W || vo >= H) return ACM_POINT_IS_OUTSIDE_IMAGE;
+        const double2 s = __ldg(map + (size_t)vo * W + uo);
+        sx = s.x; sy = s.y;
+        return ACM_POINT_OK;  // NaN: make_tap finds no sample
+    }
+    template <bool NEAREST> __device__ __forceinline__ FixedTap tap(int uo, int vo, int W, int H) const {
+        FixedTap p;
+        uint4 r = make_uint4(0u, 0u, 0u, 0u);
+        if (uo < W && vo < H) r = __ldg(rec + (size_t)vo * W + uo);
+        p.t.ok = (int)(r.x >> 31);
+        p.t.off00 = 3 * (int)(r.x & 0x3FFFFFFFu);
+        p.t.wx = 0.0; p.t.wy = 0.0;  // the exact re-blend takes them from the map (exact_w)
+        p.slow = ((r.x >> 30) & 1u) != 0u;
+        p.wlo = r.y; p.w01 = r.z; p.w23 = r.w;
+        p.sel = 0x3210u + 0x1111u * (uint32_t)(p.t.off00 & 3);
+        return p;
+    }
+    // the reference's bilinear weights (undistort.rs:94): wx = x - floor(x), wy = y - floor(y)
+    __device__ __forceinline__ void exact_w(int uo, int vo, int W, double& wx, double& wy) const {
+        const double2 s = __ldg(map + (size_t)vo * W + uo);
+        wx = s.x - floor(s.x); wy = s.y - floor(s.y);
+    }
+};
+
+// f64 map -> plan records, with the quantisation of the frame kernels (tap_from_coord).  Model-independent.
+template <bool NEAREST>
+__global__ void __launch_bounds__(256) remap_pack_kernel(const double2* __restrict__ map, uint4* __restrict__ rec, size_t n, int Wi, int Hi) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const double2 s = map[i];
+    const FixedTap p = tap_from_coord<NEAREST>(s.x, s.y, ACM_POINT_OK, Wi, Hi);
+    rec[i] = make_uint4((uint32_t)(p.t.off00 / 3) | ((uint32_t)p.slow << 30) | ((uint32_t)p.t.ok << 31), p.wlo, p.w01, p.w23);
+}
+
+// Generic byte kernel (any width and alignment): one thread owns 4 horizontally adjacent output pixels: it finds their
+// source coordinates once, then loops over the frames of the batch, gathers the taps through the read-only path, blends
+// with the reference's f64 expression and stages the 12 output bytes in shared memory so that the block writes the row
+// segment with 16-byte coalesced stores where the output allows.
+template <class Src>
+__global__ void __launch_bounds__(256) undistort_kernel(const __grid_constant__ Src source, const uint8_t* __restrict__ in,
+                                                        uint8_t* __restrict__ out, int W, int H, size_t n_frames, int interp) {
     // block = 256 threads x 4 pixels = 1024 pixels of one image row (W is padded by the guard)
     __shared__ __align__(16) uint8_t sm[256 * 12];
     const int row = blockIdx.y;
     const int px0 = (blockIdx.x * 256 + threadIdx.x) * 4;
-    const size_t frame_bytes = (size_t)W * H * 3;
+    const int Wi = source.in_w(W), Hi = source.in_h(H);
+    const size_t in_frame_bytes = (size_t)Wi * Hi * 3, frame_bytes = (size_t)W * H * 3;
     Tap taps[4];
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-        int uo = px0 + k;
-        double sx = 0.0, sy = 0.0;
-        int st = ACM_POINT_IS_OUTSIDE_IMAGE;
-        if (uo < W) {
-            double xn = ((double)uo - tcx) / tfx;
-            double yn = ((double)row - tcy) / tfy;
-            st = CamModel<M>::template project<true>(c, xn, yn, 1.0, sx, sy);
-        }
-        taps[k] = make_tap(sx, sy, st, W, H, interp);
+        double sx, sy;
+        const int st = source.coord(px0 + k, row, W, H, sx, sy);
+        taps[k] = make_tap(sx, sy, st, Wi, Hi, interp);
     }
-    const int row_stride = 3 * W;
+    const int row_stride = 3 * Wi;  // input
     const int seg_px = min(1024, W - blockIdx.x * 1024);  // pixels of this block's segment
     const int seg_bytes = seg_px * 3;
     const size_t seg_off = ((size_t)row * W + (size_t)blockIdx.x * 1024) * 3;
     const bool vec_ok = ((seg_off & 15) == 0) && ((frame_bytes & 15) == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
     for (size_t f = 0; f < n_frames; ++f) {
-        const uint8_t* src = in + f * frame_bytes;
+        const uint8_t* src = in + f * in_frame_bytes;
         uint8_t o[12];
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
@@ -495,61 +615,6 @@ __global__ void __launch_bounds__(256) undistort_kernel(const __grid_constant__ 
         }
         __syncthreads();
     }
-}
-
-// ---------------------------------------------------------------------------------------
-// Per-pixel work of the TMA and gather kernels below.  Byte-exact by construction:
-//  * The reference blends in f64 (undistort.rs:92-99) and rounds half away from zero.  Here the
-//    four tap weights are quantised once per output pixel to 24-bit fixed point
-//    (W_i = rn(w_i * 2^24), sum <= 2^24 + 2, so sum p_i W_i fits 32 bits).
-//    |S / 2^24 - sum p_i w_i| <= 4 * 255 * 2^-25 = 3.04e-5 and the f64 evaluation order of the
-//    reference moves the value by < 1e-12, so whenever the fractional part of S + 0.5 is farther
-//    than E = 640 / 2^24 = 3.8e-5 from an integer both round to the same byte.  Otherwise
-//    (probability 7.6e-5 per channel) the pixel is redone with the reference's exact f64
-//    expression, as are pixels with a weight of exactly 1.
-//  * Instruction diet (the first gather kernel was issue-bound at 151 instr/pixel): each 6-byte tap
-//    run is three aligned 32-bit words + two PRMT with a per-pixel selector; five more PRMT gather the
-//    four taps of each channel into one register; the blend is S = (dp2a(hi16) << 8) + dp4a(lo8) + 2^23
-//    per channel: the upper 16 bits of the weights pairwise through dp2a, the low byte plane through dp4a.
-// Thread <-> pixel mapping: a warp owns a 32-wide, 4-tall output patch, lane = x.  Neighbouring
-// lanes then read neighbouring source pixels (3 bytes apart), so one warp-wide 32-bit load touches
-// ~4 sectors instead of the ~17 of a "4 consecutive pixels per thread" mapping (ncu: the first
-// mapping was bound by L1 sector look-ups, 444 M per 8 frames).
-// ---------------------------------------------------------------------------------------
-constexpr uint32_t UND_TIE_E = 640u;
-
-// One output pixel, set up once and reused for every frame.
-struct FixedTap {
-    Tap t;
-    uint32_t sel;            // PRMT selector of the sample's bytes in its 4-byte-aligned window
-    uint32_t wlo, w01, w23;  // 24-bit weights, tap order [00, 10, 01, 11]: low byte plane for dp4a, upper 16 bits pairwise
-                             // for dp2a.  All zero without a sample: the blend is then 2^23 >> 24 = 0 (black) and can never
-                             // look like a tie, so the frame loops need no per-pixel mode test.
-    bool slow;               // bilinear with a weight of exactly 1: always takes the exact f64 expression
-};
-
-template <int M, bool NEAREST>
-__device__ __forceinline__ FixedTap setup_tap(const CamParams& c, double tfx, double tfy, double tcx, double tcy, int uo, int vo, int W,
-                                              int H) {
-    const double xn = ((double)uo - tcx) / tfx;  // outside the branch: the 4 pixels of a lane share it
-    double sx = 0.0, sy = 0.0;
-    int st = ACM_POINT_IS_OUTSIDE_IMAGE;
-    if (uo < W && vo < H) {
-        const double yn = ((double)vo - tcy) / tfy;
-        st = CamModel<M>::template project<true>(c, xn, yn, 1.0, sx, sy);
-    }
-    FixedTap p;
-    p.t = make_tap(sx, sy, st, W, H, NEAREST ? ACM_INTERP_NEAREST : ACM_INTERP_BILINEAR);
-    const double wxi = 1.0 - p.t.wx, wyi = 1.0 - p.t.wy;
-    uint32_t w00 = __double2uint_rn(wxi * wyi * 16777216.0), w10 = __double2uint_rn(p.t.wx * wyi * 16777216.0);
-    uint32_t w01 = __double2uint_rn(wxi * p.t.wy * 16777216.0), w11 = __double2uint_rn(p.t.wx * p.t.wy * 16777216.0);
-    if (!p.t.ok) w00 = w10 = w01 = w11 = 0u;
-    p.slow = !NEAREST && ((w00 | w10 | w01 | w11) >> 24) != 0u;
-    p.wlo = (w00 & 0xFF) | ((w10 & 0xFF) << 8) | ((w01 & 0xFF) << 16) | ((w11 & 0xFF) << 24);
-    p.w01 = ((w00 >> 8) & 0xFFFF) | (((w10 >> 8) & 0xFFFF) << 16);
-    p.w23 = ((w01 >> 8) & 0xFFFF) | (((w11 >> 8) & 0xFFFF) << 16);
-    p.sel = 0x3210u + 0x1111u * (uint32_t)(p.t.off00 & 3);
-    return p;
 }
 
 // Bilinear blend from the aligned 12-byte windows of the two tap rows (a0..a2, b0..b2) with the selector and weights
@@ -608,19 +673,19 @@ __device__ __forceinline__ void store_patch(const uint32_t px[4], uint8_t* dst, 
 }
 
 // ---------------------------------------------------------------------------------------
-// Gather path (W % 4 == 0, 4-byte aligned frames): the taps come from global memory through L1, 3 x LDG.32 per tap row
+// Gather path (Wi % 4 == 0 and W % 4 == 0, 4-byte aligned frames; W x H the output, Wi x Hi the input grid): the taps come from global memory through L1, 3 x LDG.32 per tap row
 // (2 for nearest).  With list == nullptr the grid covers the image: block = 64 x 16 pixels, warp w owns the patch at
 // (w & 1, w >> 1).  Otherwise the warps stride over the patches the TMA kernel below listed (source box larger than its
 // tile).
 // ---------------------------------------------------------------------------------------
-template <int M, bool NEAREST>
-__global__ void __launch_bounds__(256, 3) undistort_gather_kernel(const __grid_constant__ CamParams c, double tfx, double tfy, double tcx,
-                                                               double tcy, const uint8_t* __restrict__ in, uint8_t* __restrict__ out,
-                                                               int W, int H, size_t n_frames, const uint32_t* __restrict__ list,
-                                                               const uint32_t* __restrict__ list_count) {
+template <class Src, bool NEAREST>
+__global__ void __launch_bounds__(256, 3) undistort_gather_kernel(const __grid_constant__ Src source, const uint8_t* __restrict__ in,
+                                                               uint8_t* __restrict__ out, int W, int H, size_t n_frames,
+                                                               const uint32_t* __restrict__ list, const uint32_t* __restrict__ list_count) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const size_t frame_bytes = (size_t)W * H * 3;
-    const int row_stride = 3 * W;
+    const int Wi = source.in_w(W), Hi = source.in_h(H);
+    const size_t in_frame_bytes = (size_t)Wi * Hi * 3, frame_bytes = (size_t)W * H * 3;
+    const int in_stride = 3 * Wi, row_stride = 3 * W;
     const uint32_t npx = (uint32_t)(W + 31) / 32u;
     const uint32_t n = list ? *list_count : 1u;  // whole image: one patch per warp, the stride ends the loop
     for (uint32_t e = list ? blockIdx.x * 8u + warp : 0u; e < n; e += gridDim.x * 8u) {
@@ -631,10 +696,10 @@ __global__ void __launch_bounds__(256, 3) undistort_gather_kernel(const __grid_c
         uint32_t valid = 0u, slow = 0u;
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
-            tap[k] = setup_tap<M, NEAREST>(c, tfx, tfy, tcx, tcy, x0 + lane, y0 + k, W, H);
+            tap[k] = source.template tap<NEAREST>(x0 + lane, y0 + k, W, H);
             // a window that would read past the end of the frame (the last frame's end for the last pixels) is not read:
             // the pixel takes the exact path
-            const bool exact = tap[k].slow || (tap[k].t.ok && (size_t)tap[k].t.off00 + (size_t)row_stride + 16 > frame_bytes);
+            const bool exact = tap[k].slow || (tap[k].t.ok && (size_t)tap[k].t.off00 + (size_t)in_stride + 16 > in_frame_bytes);
             valid |= (uint32_t)tap[k].t.ok << k;
             slow |= (uint32_t)exact << k;
             // pixels without a sample or taken exactly load from offset 0 (always inside the frame): the tap loads of a
@@ -645,7 +710,7 @@ __global__ void __launch_bounds__(256, 3) undistort_gather_kernel(const __grid_c
         const int n_rows = (lane < 24 && 4 * lane + 3 < 3 * valid_px) ? min(4, H - y0) : 0;  // rows this lane stores
         uint8_t* dst = out + ((size_t)y0 * W + x0) * 3 + 4 * lane;
         for (size_t f = 0; f < n_frames; ++f, dst += frame_bytes) {
-            const uint8_t* src = in + f * frame_bytes;
+            const uint8_t* src = in + f * in_frame_bytes;
             uint32_t px[4];  // [R G B .] per pixel
             uint32_t redo = slow;
             if (NEAREST) {
@@ -659,7 +724,7 @@ __global__ void __launch_bounds__(256, 3) undistort_gather_kernel(const __grid_c
 #pragma unroll
                 for (int k = 0; k < 4; ++k) {
                     const uint32_t* r0 = reinterpret_cast<const uint32_t*>(src + offa[k]);
-                    const uint32_t* r1 = reinterpret_cast<const uint32_t*>(src + offa[k] + row_stride);
+                    const uint32_t* r1 = reinterpret_cast<const uint32_t*>(src + offa[k] + in_stride);
                     ta[k][0] = __ldg(r0); ta[k][1] = __ldg(r0 + 1); ta[k][2] = __ldg(r0 + 2);
                     tb[k][0] = __ldg(r1); tb[k][1] = __ldg(r1 + 1); tb[k][2] = __ldg(r1 + 2);
                 }
@@ -675,8 +740,10 @@ __global__ void __launch_bounds__(256, 3) undistort_gather_kernel(const __grid_c
                 for (int k = 0; k < 4; ++k) {
                     if ((redo >> k) & 1u) {
                         const uint8_t* p = src + tap[k].t.off00;
+                        double wx = tap[k].t.wx, wy = tap[k].t.wy;
+                        if constexpr (Src::PLAN) { if (!NEAREST) source.exact_w(x0 + lane, y0 + k, W, wx, wy); }
                         px[k] = NEAREST ? (__ldg(p) | (__ldg(p + 1) << 8) | ((uint32_t)__ldg(p + 2) << 16))
-                                        : blend_exact_px(p, row_stride, tap[k].t.wx, tap[k].t.wy);
+                                        : blend_exact_px(p, in_stride, wx, wy);
                     }
                 }
             }
@@ -686,7 +753,7 @@ __global__ void __launch_bounds__(256, 3) undistort_gather_kernel(const __grid_c
 }
 
 // ---------------------------------------------------------------------------------------
-// TMA path (W % 16 == 0, 16-byte aligned frames): the gathers above are bound by load latency and L1
+// TMA path (Wi % 16 == 0, 16-byte aligned input; W % 4 == 0, 4-byte aligned output): the gathers above are bound by load latency and L1
 // sector look-ups (ncu: long_scoreboard 4.6 per issue, 60 % of the LSU wavefront budget).  Here
 // every warp stages the SOURCE BOX of its 32 x 4 output patch -- UND_BOX_W bytes x UND_BOX_ROWS
 // rows, found once from the taps -- in shared memory with one `cp.async.bulk.tensor.3d` per frame
@@ -727,15 +794,14 @@ __device__ __forceinline__ void und_tma_load_3d(uint32_t dst, const void* map, u
                  ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2) : "memory");
 }
 
-template <int M, bool NEAREST>
-__global__ void __launch_bounds__(256, 3) undistort_tma_kernel(const __grid_constant__ CamParams c, double tfx, double tfy, double tcx,
-                                                            double tcy, const __grid_constant__ UndMaps in_maps,
+template <class Src, bool NEAREST>
+__global__ void __launch_bounds__(256, 3) undistort_tma_kernel(const __grid_constant__ Src source, const __grid_constant__ UndMaps in_maps,
                                                             const uint8_t* __restrict__ in, uint8_t* __restrict__ out, int W, int H,
                                                             int n_frames, uint32_t* __restrict__ list, uint32_t* __restrict__ list_count) {
     constexpr int TILE = UND_FPS * UND_BOX_W * UND_BOX_ROWS;   // one stage = UND_FPS frames of the box
     // dynamic shared memory: tiles[8 warps][STAGES][TILE] | mbarriers[8][STAGES] | wx[4][256] | wy[4][256]
     // (the f64 weights are only read by the rare exact re-blend; keeping them out of registers is what
-    // lets three blocks stay resident)
+    // lets three blocks stay resident; a plan source takes them from its map instead)
     extern __shared__ __align__(128) uint8_t und_smem[];
     uint8_t* const tiles = und_smem;
     unsigned long long* const bars = reinterpret_cast<unsigned long long*>(und_smem + 8 * UND_STAGES * TILE);
@@ -745,21 +811,22 @@ __global__ void __launch_bounds__(256, 3) undistort_tma_kernel(const __grid_cons
     const int x0 = blockIdx.x * 64 + (warp & 1) * 32;        // patch origin
     const int y0 = blockIdx.y * 16 + (warp >> 1) * 4;
     if (x0 >= W || y0 >= H) return;                          // warp-uniform; nothing block-wide follows
-    const size_t frame_bytes = (size_t)W * H * 3;
-    const int row_stride = 3 * W;
+    const int Wi = source.in_w(W), Hi = source.in_h(H);
+    const size_t in_frame_bytes = (size_t)Wi * Hi * 3, frame_bytes = (size_t)W * H * 3;
+    const int in_stride = 3 * Wi, row_stride = 3 * W;
     int off[4];
     uint32_t sel[4], wlo[4], w01[4], w23[4];
     uint32_t valid = 0u, slow = 0u;
     int bx_min = 0x7fffffff, bx_max = -1, by_min = 0x7fffffff, by_max = -1;
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-        const FixedTap p = setup_tap<M, NEAREST>(c, tfx, tfy, tcx, tcy, x0 + lane, y0 + k, W, H);
+        const FixedTap p = source.template tap<NEAREST>(x0 + lane, y0 + k, W, H);
         off[k] = p.t.off00; sel[k] = p.sel; wlo[k] = p.wlo; w01[k] = p.w01; w23[k] = p.w23;
-        if (!NEAREST) { s_wx[k * 256 + threadIdx.x] = p.t.wx; s_wy[k * 256 + threadIdx.x] = p.t.wy; }
+        if (!NEAREST && !Src::PLAN) { s_wx[k * 256 + threadIdx.x] = p.t.wx; s_wy[k * 256 + threadIdx.x] = p.t.wy; }
         slow |= (uint32_t)p.slow << k;
         if (p.t.ok) {
             valid |= 1u << k;
-            const int ty = p.t.off00 / row_stride, tb = p.t.off00 - ty * row_stride;
+            const int ty = p.t.off00 / in_stride, tb = p.t.off00 - ty * in_stride;
             bx_min = min(bx_min, tb); bx_max = max(bx_max, tb + (NEAREST ? 2 : 5));
             by_min = min(by_min, ty); by_max = max(by_max, ty + (NEAREST ? 0 : 1));
         }
@@ -781,10 +848,10 @@ __global__ void __launch_bounds__(256, 3) undistort_tma_kernel(const __grid_cons
     uint32_t so[4];  // shared-memory address of the aligned tap window in stage 0
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-        const int ty = off[k] / row_stride, tb = off[k] - ty * row_stride;
+        const int ty = off[k] / in_stride, tb = off[k] - ty * in_stride;
         so[k] = tile0 + (((valid >> k) & 1u) ? (uint32_t)((ty - box_y) * UND_BOX_W + ((tb - box_x) & ~3)) : 0u);
     }
-    const int valid_px = min(32, W - x0);                     // multiple of 4 because W % 16 == 0
+    const int valid_px = min(32, W - x0);                     // multiple of 4 because W % 4 == 0
     const int n_rows = (lane < 24 && 4 * lane + 3 < 3 * valid_px) ? min(4, H - y0) : 0;  // rows this lane stores
     if (lane == 0) {
 #pragma unroll
@@ -846,14 +913,17 @@ __global__ void __launch_bounds__(256, 3) undistort_tma_kernel(const __grid_cons
                     redo |= tie_bits(tz);
                 }
                 if (redo) {  // rare: redo these pixels with the reference's f64 expression from global memory
-                    const uint8_t* src = in + (size_t)f * frame_bytes;
+                    const uint8_t* src = in + (size_t)f * in_frame_bytes;
 #pragma unroll
                     for (int k = 0; k < 4; ++k) {
                         if ((redo >> k) & 1u) {
                             // rebuild the byte offset of p00 from the tile address and the byte selector
                             const uint32_t rel = so[k] - tile0;
-                            const int o00 = (box_y + (int)(rel / UND_BOX_W)) * row_stride + box_x + (int)(rel % UND_BOX_W) + (int)(sel[k] & 3u);
-                            px[k] = blend_exact_px(src + o00, row_stride, s_wx[k * 256 + threadIdx.x], s_wy[k * 256 + threadIdx.x]);
+                            const int o00 = (box_y + (int)(rel / UND_BOX_W)) * in_stride + box_x + (int)(rel % UND_BOX_W) + (int)(sel[k] & 3u);
+                            double wx, wy;
+                            if constexpr (Src::PLAN) source.exact_w(x0 + lane, y0 + k, W, wx, wy);
+                            else { wx = s_wx[k * 256 + threadIdx.x]; wy = s_wy[k * 256 + threadIdx.x]; }
+                            px[k] = blend_exact_px(src + o00, in_stride, wx, wy);
                         }
                     }
                 }
@@ -919,28 +989,42 @@ static int32_t check_undistort_args(acm_ctx* ctx, const acm_camera* cam, const d
 }
 
 // maps != nullptr: the TMA kernel, then the gather over the patches it lists (list = d_count + 64);
-// gather: the gather over the whole image; otherwise the generic byte kernel
-template <int M, bool NEAREST>
-static int32_t launch_undistort(acm_ctx* ctx, const CamParams& c, const double* t, const UndMaps* maps, bool gather, const uint8_t* d_in,
-                                uint8_t* d_out, int W, int H, size_t n_frames, uint32_t* d_count) {
+// gather: the gather over the whole image; otherwise the generic byte kernel.  W x H: the output grid.
+template <class Src, bool NEAREST>
+static int32_t launch_undistort(acm_ctx* ctx, const Src& source, const UndMaps* maps, bool gather, const uint8_t* d_in, uint8_t* d_out,
+                                int W, int H, size_t n_frames, uint32_t* d_count) {
     const dim3 patch_grid((W + 63) / 64, (H + 15) / 16);  // block = 64 x 16 output pixels
     if (maps) {
         constexpr int smem = 8 * UND_STAGES * UND_FPS * UND_BOX_W * UND_BOX_ROWS + 8 * UND_STAGES * 8 + 2 * 4 * 256 * 8;
         uint32_t* const d_list = d_count + 64;
-        cudaFuncSetAttribute(undistort_tma_kernel<M, NEAREST>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        undistort_tma_kernel<M, NEAREST><<<patch_grid, 256, smem, ctx->stream>>>(c, t[0], t[1], t[2], t[3], *maps, d_in, d_out, W, H, (int)n_frames,
-                                                                               d_list, d_count);
+        cudaFuncSetAttribute(undistort_tma_kernel<Src, NEAREST>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        undistort_tma_kernel<Src, NEAREST><<<patch_grid, 256, smem, ctx->stream>>>(source, *maps, d_in, d_out, W, H, (int)n_frames, d_list,
+                                                                                 d_count);
         ACM_CHECK_LAUNCH(ctx);
-        undistort_gather_kernel<M, NEAREST><<<ctx->sm_count * 3, 256, 0, ctx->stream>>>(c, t[0], t[1], t[2], t[3], d_in, d_out, W, H, n_frames,
-                                                                                       d_list, d_count);
+        undistort_gather_kernel<Src, NEAREST><<<ctx->sm_count * 3, 256, 0, ctx->stream>>>(source, d_in, d_out, W, H, n_frames, d_list, d_count);
     } else if (gather) {
-        undistort_gather_kernel<M, NEAREST><<<patch_grid, 256, 0, ctx->stream>>>(c, t[0], t[1], t[2], t[3], d_in, d_out, W, H, n_frames, nullptr,
-                                                                               nullptr);
+        undistort_gather_kernel<Src, NEAREST><<<patch_grid, 256, 0, ctx->stream>>>(source, d_in, d_out, W, H, n_frames, nullptr, nullptr);
     } else {
-        undistort_kernel<M><<<dim3((W + 1023) / 1024, H), 256, 0, ctx->stream>>>(c, t[0], t[1], t[2], t[3], d_in, d_out, W, H, n_frames,
-                                                                                NEAREST ? ACM_INTERP_NEAREST : ACM_INTERP_BILINEAR);
+        undistort_kernel<Src><<<dim3((W + 1023) / 1024, H), 256, 0, ctx->stream>>>(source, d_in, d_out, W, H, n_frames,
+                                                                                  NEAREST ? ACM_INTERP_NEAREST : ACM_INTERP_BILINEAR);
     }
     ACM_CHECK_LAUNCH(ctx);
+    return ACM_OK;
+}
+
+// Tensor maps of the TMA path over a Wi x Hi input batch, and the leftover list ([count][patch ids], one id per 32 x 4
+// patch of the W x H output at most) in the context's scratch.  *tma (in: the path rule allows TMA) turns false when the
+// driver refuses a tensor map: the caller then gathers.
+static int32_t prepare_tma(acm_ctx* ctx, UndMaps* maps, const uint8_t* d_in, int Wi, int Hi, int W, int H, size_t n_frames, bool* tma,
+                           uint32_t** d_count) {
+    *d_count = nullptr;
+    for (int r = UND_MIN_ROWS; *tma && r <= UND_BOX_ROWS; ++r) *tma = make_frame_tensor_map(&maps->m[r - UND_MIN_ROWS], d_in, Wi, Hi, n_frames, r);
+    if (!*tma) return ACM_OK;
+    const size_t n_patches = (size_t)((W + 31) / 32) * (size_t)((H + 3) / 4);
+    int32_t rc = acm_ensure_scratch(ctx, 256 + n_patches * sizeof(uint32_t));
+    if (rc) return rc;
+    *d_count = static_cast<uint32_t*>(ctx->d_scratch);
+    ACM_CUDA(ctx, cudaMemsetAsync(*d_count, 0, sizeof(uint32_t), ctx->stream));
     return ACM_OK;
 }
 
@@ -961,20 +1045,22 @@ extern "C" int32_t acm_undistort_rgb8(acm_ctx* ctx, const acm_camera* cam, const
     const bool gather = W % 4 == 0 && (in_addr & 3) == 0 && (out_addr & 3) == 0;
     UndMaps maps;
     bool tma = gather && W % 16 == 0 && (in_addr & 15) == 0 && n_frames < 0x7fffffffULL;
-    for (int r = UND_MIN_ROWS; tma && r <= UND_BOX_ROWS; ++r) tma = make_frame_tensor_map(&maps.m[r - UND_MIN_ROWS], d_in, W, H, n_frames, r);
-    uint32_t* d_count = nullptr;
-    if (tma) {
-        // leftover list: [count][patch ids], one id per 32 x 4 patch at most
-        const size_t n_patches = (size_t)((W + 31) / 32) * (size_t)((H + 3) / 4);
-        rc = acm_ensure_scratch(ctx, 256 + n_patches * sizeof(uint32_t));
-        if (rc) return rc;
-        d_count = static_cast<uint32_t*>(ctx->d_scratch);
-        ACM_CUDA(ctx, cudaMemsetAsync(d_count, 0, sizeof(uint32_t), ctx->stream));
-    }
+    uint32_t* d_count;
+    rc = prepare_tma(ctx, &maps, d_in, W, H, W, H, n_frames, &tma, &d_count);
+    if (rc) return rc;
     const UndMaps* const tma_maps = tma ? &maps : nullptr;
-    ACM_DISPATCH_MODEL(cam->model, return interpolation == ACM_INTERP_NEAREST
-                                              ? launch_undistort<M, true>(ctx, c, t, tma_maps, gather, d_in, d_out, W, H, n_frames, d_count)
-                                              : launch_undistort<M, false>(ctx, c, t, tma_maps, gather, d_in, d_out, W, H, n_frames, d_count))
+    ACM_DISPATCH_MODEL(cam->model, {
+        const ModelSrc<M> source{c, t[0], t[1], t[2], t[3]};
+        return interpolation == ACM_INTERP_NEAREST ? launch_undistort<ModelSrc<M>, true>(ctx, source, tma_maps, gather, d_in, d_out, W, H, n_frames, d_count)
+                                                   : launch_undistort<ModelSrc<M>, false>(ctx, source, tma_maps, gather, d_in, d_out, W, H, n_frames, d_count);
+    })
+    return ACM_OK;
+}
+
+static int32_t launch_undistort_map(acm_ctx* ctx, const CamParams& c, const double* t, double* d_src_xy, int W, int H) {
+    const int grid = (int)(((size_t)W * H + 255) / 256);
+    ACM_DISPATCH_MODEL(c.model, (undistort_map_kernel<M><<<grid, 256, 0, ctx->stream>>>(c, t[0], t[1], t[2], t[3], d_src_xy, W, H)))
+    ACM_CHECK_LAUNCH(ctx);
     return ACM_OK;
 }
 
@@ -987,12 +1073,187 @@ extern "C" int32_t acm_undistort_map(acm_ctx* ctx, const acm_camera* cam, const 
     CamParams c;
     rc = acm_make_cam_params(ctx, cam, &c);
     if (rc) return rc;
-    const int W = (int)cam->width, H = (int)cam->height;
-    size_t n = (size_t)W * H;
-    int grid = (int)((n + 255) / 256);
-    ACM_DISPATCH_MODEL(cam->model, (undistort_map_kernel<M><<<grid, 256, 0, ctx->stream>>>(c, t[0], t[1], t[2], t[3], d_src_xy, W, H)))
+    return launch_undistort_map(ctx, c, t, d_src_xy, (int)cam->width, (int)cam->height);
+}
+
+// ---------------------------------------------------------------------------------------
+// Remap between two camera models (beyond the reference, composed of its functions): output pixel (u, v) of the output
+// camera's grid -> ray = output.unproject((u, v)) (with its pixel-bounds test) -> src = input.project(ray) -> the
+// interpolate_pixel of undistort.rs:51-105 on the input frame; black where a step fails.  Both steps keep their IEEE
+// forms (unproject<true> as acm_unproject_ieee, the non-FAST project<true> as undistort), so the map of the five
+// arithmetic-only models is bit-identical to the oracle's.
+// ---------------------------------------------------------------------------------------
+template <int MI, int MO>
+__global__ void __launch_bounds__(256) remap_map_kernel(const __grid_constant__ CamParams ci, const __grid_constant__ CamParams co,
+                                                        double* __restrict__ src_xy, int W, int H) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)W * H) return;
+    const int uo = (int)(i % W), vo = (int)(i / W);
+    double x, y, z, sx, sy;
+    int st = CamModel<MO>::template unproject<true>(co, (double)uo, (double)vo, x, y, z);
+    if (st == ACM_POINT_OK) st = CamModel<MI>::template project<true>(ci, x, y, z, sx, sy);
+    if (st != ACM_POINT_OK) sx = sy = acm_nan();
+    reinterpret_cast<double2*>(src_xy)[i] = make_double2(sx, sy);
+}
+
+template <int MO>
+static int32_t launch_remap_map(acm_ctx* ctx, const CamParams& ci, const CamParams& co, double* d_src_xy, int W, int H) {
+    const int grid = (int)(((size_t)W * H + 255) / 256);
+    ACM_DISPATCH_MODEL(ci.model, (remap_map_kernel<M, MO><<<grid, 256, 0, ctx->stream>>>(ci, co, d_src_xy, W, H)))
     ACM_CHECK_LAUNCH(ctx);
     return ACM_OK;
+}
+
+static int32_t check_frame_camera(acm_ctx* ctx, const acm_camera* cam, const char* side) {
+    if (!cam) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "remap: null %s camera", side);
+    if (cam->width == 0 || cam->height == 0)
+        return acm_fail(ctx, ACM_ERR_INVALID_ARG, "remap: %s camera resolution must be set (frames have the camera's resolution)", side);
+    if ((uint64_t)cam->width * cam->height * 3 >= 0x7fffffffULL)
+        return acm_fail(ctx, ACM_ERR_INVALID_ARG, "remap: %s frame larger than 2 GiB is not supported", side);
+    return ACM_OK;
+}
+
+// source coordinates of every pixel of output_cam's grid: the remap map of input_cam -> output_cam
+static int32_t remap_map(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam, double* d_src_xy) {
+    CamParams ci, co;
+    int32_t rc = acm_make_cam_params(ctx, input_cam, &ci);
+    if (!rc) rc = acm_make_cam_params(ctx, output_cam, &co);
+    if (rc) return rc;
+    const int W = (int)output_cam->width, H = (int)output_cam->height;
+    ACM_DISPATCH_MODEL(co.model, return launch_remap_map<M>(ctx, ci, co, d_src_xy, W, H))
+    return ACM_OK;
+}
+
+extern "C" int32_t acm_remap_map(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam, double* d_src_xy) {
+    ACM_ENTER(ctx);
+    int32_t rc = check_frame_camera(ctx, input_cam, "input");
+    if (!rc) rc = check_frame_camera(ctx, output_cam, "output");
+    if (rc) return rc;
+    ACM_REQUIRE(ctx, d_src_xy, "remap_map: null output");
+    return remap_map(ctx, input_cam, output_cam, d_src_xy);
+}
+
+// A plan: the f64 map (16 B per output pixel, read by the byte kernel and the exact re-blend) and the packed records
+// (16 B per output pixel, read by the TMA and gather kernels): 32 B per output pixel, 537 MB for a 4096 x 4096 output.
+struct acm_remap_plan {
+    acm_ctx* ctx;
+    int Wi, Hi, Wo, Ho;
+    int32_t interpolation;
+    double2* d_map;
+    uint4* d_rec;
+};
+
+static int32_t launch_remap_pack(acm_ctx* ctx, acm_remap_plan* p) {
+    const size_t n = (size_t)p->Wo * p->Ho;
+    const int grid = (int)((n + 255) / 256);
+    if (p->interpolation == ACM_INTERP_NEAREST) remap_pack_kernel<true><<<grid, 256, 0, ctx->stream>>>(p->d_map, p->d_rec, n, p->Wi, p->Hi);
+    else remap_pack_kernel<false><<<grid, 256, 0, ctx->stream>>>(p->d_map, p->d_rec, n, p->Wi, p->Hi);
+    ACM_CHECK_LAUNCH(ctx);
+    return ACM_OK;
+}
+
+static void free_plan(acm_remap_plan* p) {
+    if (p->d_map) cudaFree(p->d_map);
+    if (p->d_rec) cudaFree(p->d_rec);
+    delete p;
+}
+
+extern "C" int32_t acm_remap_plan_create(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam,
+                                         const double* target_intrinsics, int32_t interpolation, acm_remap_plan** out) {
+    ACM_ENTER(ctx);
+    ACM_REQUIRE(ctx, out, "remap_plan: null output");
+    *out = nullptr;
+    ACM_REQUIRE(ctx, !(output_cam && target_intrinsics), "remap_plan: give either an output camera or target intrinsics, not both");
+    int32_t rc = check_frame_camera(ctx, input_cam, "input");
+    if (!rc && output_cam) rc = check_frame_camera(ctx, output_cam, "output");
+    if (rc) return rc;
+    ACM_REQUIRE(ctx, interpolation == ACM_INTERP_NEAREST || interpolation == ACM_INTERP_BILINEAR, "remap_plan: unknown interpolation");
+    CamParams ci;
+    rc = acm_make_cam_params(ctx, input_cam, &ci);
+    if (rc) return rc;
+    acm_remap_plan* p = new (std::nothrow) acm_remap_plan{ctx, (int)input_cam->width, (int)input_cam->height, 0, 0, interpolation, nullptr,
+                                                          nullptr};
+    if (!p) return acm_fail(ctx, ACM_ERR_CUDA, "remap_plan: out of host memory");
+    const acm_camera* const grid_cam = output_cam ? output_cam : input_cam;
+    p->Wo = (int)grid_cam->width; p->Ho = (int)grid_cam->height;
+    const size_t n = (size_t)p->Wo * p->Ho;
+    rc = acm_device_malloc(ctx, reinterpret_cast<void**>(&p->d_map), n * sizeof(double2));
+    if (!rc) rc = acm_device_malloc(ctx, reinterpret_cast<void**>(&p->d_rec), n * sizeof(uint4));
+    if (!rc && output_cam) {
+        rc = remap_map(ctx, input_cam, output_cam, reinterpret_cast<double*>(p->d_map));
+    } else if (!rc) {  // undistort_image semantics: the map of acm_undistort_map
+        double t[4];
+        for (int i = 0; i < 4; ++i) t[i] = target_intrinsics ? target_intrinsics[i] : input_cam->params[i];
+        rc = launch_undistort_map(ctx, ci, t, reinterpret_cast<double*>(p->d_map), p->Wo, p->Ho);
+    }
+    if (!rc) rc = launch_remap_pack(ctx, p);
+    if (rc) {
+        cudaStreamSynchronize(ctx->stream);  // no kernel may still write to the buffers that are freed
+        free_plan(p);
+        return rc;
+    }
+    *out = p;
+    return ACM_OK;
+}
+
+extern "C" int32_t acm_remap_plan_destroy(acm_ctx* ctx, acm_remap_plan* plan) {
+    ACM_ENTER(ctx);
+    if (!plan) return ACM_OK;
+    ACM_REQUIRE(ctx, plan->ctx == ctx, "remap_plan: the plan belongs to another context");
+    ACM_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    free_plan(plan);
+    return ACM_OK;
+}
+
+// Path rule: TMA + leftover gather when Wi % 16 == 0, the input is 16-byte and the output 4-byte aligned, Wo % 4 == 0 and the
+// tensor maps encode; the whole-image gather when Wi % 4 == 0, Wo % 4 == 0 and both buffers are 4-byte aligned; the byte
+// kernel otherwise.
+extern "C" int32_t acm_remap_rgb8(acm_ctx* ctx, const acm_remap_plan* plan, const uint8_t* d_in, uint8_t* d_out, size_t n_frames) {
+    ACM_ENTER(ctx);
+    ACM_REQUIRE(ctx, plan, "remap: null plan");
+    ACM_REQUIRE(ctx, plan->ctx == ctx, "remap: the plan belongs to another context");
+    ACM_REQUIRE(ctx, d_in && d_out, "remap: null frame buffer");
+    if (n_frames == 0) return ACM_OK;
+    const int Wi = plan->Wi, Hi = plan->Hi, W = plan->Wo, H = plan->Ho;
+    const uintptr_t in_addr = reinterpret_cast<uintptr_t>(d_in), out_addr = reinterpret_cast<uintptr_t>(d_out);
+    const bool gather = Wi % 4 == 0 && W % 4 == 0 && (in_addr & 3) == 0 && (out_addr & 3) == 0;
+    UndMaps maps;
+    bool tma = gather && Wi % 16 == 0 && (in_addr & 15) == 0 && n_frames < 0x7fffffffULL;
+    uint32_t* d_count;
+    int32_t rc = prepare_tma(ctx, &maps, d_in, Wi, Hi, W, H, n_frames, &tma, &d_count);
+    if (rc) return rc;
+    const PlanSrc source{plan->d_rec, plan->d_map, Wi, Hi};
+    const UndMaps* const tma_maps = tma ? &maps : nullptr;
+    return plan->interpolation == ACM_INTERP_NEAREST
+               ? launch_undistort<PlanSrc, true>(ctx, source, tma_maps, gather, d_in, d_out, W, H, n_frames, d_count)
+               : launch_undistort<PlanSrc, false>(ctx, source, tma_maps, gather, d_in, d_out, W, H, n_frames, d_count);
+}
+
+extern "C" int32_t acm_remap_rgb8_host(acm_ctx* ctx, const acm_remap_plan* plan, const uint8_t* frames_in, uint8_t* frames_out,
+                                       size_t n_frames) {
+    ACM_ENTER(ctx);
+    ACM_REQUIRE(ctx, plan, "remap_host: null plan");
+    ACM_REQUIRE(ctx, plan->ctx == ctx, "remap_host: the plan belongs to another context");
+    ACM_REQUIRE(ctx, n_frames == 0 || (frames_in && frames_out), "remap_host: null frame buffer");
+    if (n_frames == 0) return ACM_OK;
+    const size_t in_bytes = (size_t)plan->Wi * plan->Hi * 3 * n_frames, out_bytes = (size_t)plan->Wo * plan->Ho * 3 * n_frames;
+    uint8_t *d_in = nullptr, *d_out = nullptr;
+    int32_t rc = acm_device_malloc(ctx, reinterpret_cast<void**>(&d_in), in_bytes);
+    if (!rc) rc = acm_device_malloc(ctx, reinterpret_cast<void**>(&d_out), out_bytes);
+    if (!rc) {
+        const cudaError_t e = cudaMemcpyAsync(d_in, frames_in, in_bytes, cudaMemcpyHostToDevice, ctx->stream);
+        if (e != cudaSuccess) rc = acm_fail(ctx, ACM_ERR_CUDA, "H2D failed: %s", cudaGetErrorString(e));
+    }
+    if (!rc) rc = acm_remap_rgb8(ctx, plan, d_in, d_out, n_frames);
+    if (!rc) {
+        cudaError_t e = cudaMemcpyAsync(frames_out, d_out, out_bytes, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+        if (e != cudaSuccess) rc = acm_fail(ctx, ACM_ERR_CUDA, "D2H failed: %s", cudaGetErrorString(e));
+    }
+    cudaStreamSynchronize(ctx->stream);
+    if (d_in) cudaFree(d_in);
+    if (d_out) cudaFree(d_out);
+    return rc;
 }
 
 // ---------------------------------------------------------------------------------------

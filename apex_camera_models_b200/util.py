@@ -1,5 +1,6 @@
 """util hot loops of the reference: undistort_image (src/util/undistort.rs:14-105), sample_points
-(src/util/point_sampling.rs:46-120), compute_reprojection_error (src/util/error_metrics.rs:62-121)."""
+(src/util/point_sampling.rs:46-120), compute_reprojection_error (src/util/error_metrics.rs:62-121); and remap plans
+(camera-to-camera image remap, composed of the reference's unproject, project and interpolate_pixel)."""
 from __future__ import annotations
 
 import ctypes as C
@@ -76,6 +77,108 @@ def undistort_map(camera_model: CameraModel, target_intrinsics: Intrinsics | Non
     ctx.d2h(out, d)
     ctx.sync()
     ctx.device_free(d)
+    return out
+
+
+def _check_frames(frames: np.ndarray, camera_model: CameraModel) -> np.ndarray:
+    """(F, H, W, 3) uint8 frames at the camera's resolution, as undistort.rs:23-28 requires."""
+    frames = np.ascontiguousarray(frames, dtype=np.uint8)
+    if frames.ndim != 4 or frames.shape[3] != 3:
+        raise UtilError("Invalid parameters: expected (F, H, W, 3) uint8 frames")
+    res = camera_model.get_resolution()
+    _, H, W, _ = frames.shape
+    if W != res.width or H != res.height:
+        raise UtilError(f"Invalid parameters: Image {W}x{H} doesn't match model {res.width}x{res.height}")
+    return frames
+
+
+class RemapPlan:
+    """Remap of RGB8 frames from `input_model`'s camera to `output_model`'s, built once on the device and applied to
+    any number of frame batches.  Output pixel (u, v) of the output camera's grid samples the input frame at
+    input_model.project(output_model.unproject((u, v))) with `interpolation` (undistort.rs:51-105); black where either
+    step fails.  With `output_model=None` the plan is `undistort_image(., input_model, target_intrinsics, interpolation)`
+    and its output is byte-identical to `undistort_images`.  The plan keeps 32 bytes per output pixel on the device
+    until `close()`."""
+
+    def __init__(self, input_model: CameraModel, output_model: CameraModel | None = None, target_intrinsics: Intrinsics | None = None,
+                 interpolation: InterpolationMethod = InterpolationMethod.Bilinear):
+        self.ctx = input_model.ctx
+        self.input_model = input_model
+        self.output_resolution = (output_model or input_model).get_resolution()
+        cin = input_model.camera_block()
+        cout = output_model.camera_block() if output_model is not None else None
+        h = C.c_void_p()
+        self.ctx.check(_lib.acm_remap_plan_create(self.ctx.handle, C.byref(cin), C.byref(cout) if cout is not None else None,
+                                                  _target_array(target_intrinsics), int(interpolation), C.byref(h)))
+        self._h = h
+
+    @property
+    def handle(self):
+        if not self._h:
+            raise UtilError("remap plan is closed")
+        return self._h
+
+    def apply(self, frames: np.ndarray) -> np.ndarray:
+        """Host frames (F, Hi, Wi, 3) uint8 at the input camera's resolution -> (F, Ho, Wo, 3)."""
+        frames = _check_frames(frames, self.input_model)
+        r = self.output_resolution
+        out = np.empty((frames.shape[0], r.height, r.width, 3), np.uint8)
+        self.ctx.check(_lib.acm_remap_rgb8_host(self.ctx.handle, self.handle, frames.ctypes.data_as(C.c_void_p),
+                                                out.ctypes.data_as(C.c_void_p), frames.shape[0]))
+        return out
+
+    def apply_device(self, in_ptr: int, out_ptr: int, n_frames: int) -> None:
+        """Frames resident on the plan's device: n_frames * Wi * Hi * 3 bytes at in_ptr -> n_frames * Wo * Ho * 3 at
+        out_ptr, enqueued on the context's stream."""
+        self.ctx.check(_lib.acm_remap_rgb8(self.ctx.handle, self.handle, C.c_void_p(in_ptr), C.c_void_p(out_ptr), n_frames))
+
+    def close(self) -> None:
+        if self._h:
+            h, self._h = self._h, None
+            if self.ctx.handle:
+                self.ctx.check(_lib.acm_remap_plan_destroy(self.ctx.handle, h))
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def remap_images(frames: np.ndarray, input_model: CameraModel, output_model: CameraModel,
+                 interpolation: InterpolationMethod = InterpolationMethod.Bilinear) -> np.ndarray:
+    """Frames (F, Hi, Wi, 3) uint8 of `input_model`'s camera -> (F, Ho, Wo, 3) as `output_model`'s camera sees them."""
+    frames = _check_frames(frames, input_model)
+    with RemapPlan(input_model, output_model, None, interpolation) as plan:
+        return plan.apply(frames)
+
+
+def remap_image(input_image: np.ndarray, input_model: CameraModel, output_model: CameraModel,
+                interpolation: InterpolationMethod = InterpolationMethod.Bilinear) -> np.ndarray:
+    """One (Hi, Wi, 3) uint8 image -> (Ho, Wo, 3)."""
+    img = np.ascontiguousarray(input_image, dtype=np.uint8)
+    return remap_images(img[None], input_model, output_model, interpolation)[0]
+
+
+def remap_map(input_model: CameraModel, output_model: CameraModel) -> np.ndarray:
+    """(Ho, Wo, 2) source coordinates on the input frame of every output pixel (NaN where a step fails)."""
+    ctx = input_model.ctx
+    cin, cout = input_model.camera_block(), output_model.camera_block()
+    res = output_model.get_resolution()
+    d = ctx.device_alloc(max(res.width * res.height, 1) * 16)
+    try:
+        ctx.check(_lib.acm_remap_map(ctx.handle, C.byref(cin), C.byref(cout), C.c_void_p(d)))
+        out = np.empty((res.height, res.width, 2))
+        ctx.d2h(out, d)
+        ctx.sync()
+    finally:
+        ctx.device_free(d)
     return out
 
 

@@ -228,6 +228,26 @@ int32_t acm_undistort_rgb8_host(acm_ctx* ctx, const acm_camera* cam, const doubl
  * where the projection fails */
 int32_t acm_undistort_map(acm_ctx* ctx, const acm_camera* cam, const double* target_intrinsics, double* d_src_xy);
 
+/* ---- remap plans: RGB8 frames from one camera model to another (beyond the reference) -----
+ * Output pixel (u, v) on the output camera's grid: ray = output.unproject((u, v)), then
+ * src = input.project(ray), then undistort.rs's interpolate_pixel on the input frame; black where a
+ * step fails.  Input frames have the input camera's resolution, output frames the output camera's.
+ * A plan computes the source coordinates once and keeps 32 bytes per output pixel on the device
+ * (537 MB for a 4096 x 4096 output); every acm_remap_rgb8 call then only reads them.
+ * output_cam != NULL: camera-to-camera remap (target_intrinsics must be NULL).
+ * output_cam == NULL: undistort_image semantics of input_cam with target_intrinsics (NULL = own), so the
+ * plan's output is byte-identical to acm_undistort_rgb8.  interpolation is fixed per plan.  A plan
+ * belongs to the context that created it. */
+typedef struct acm_remap_plan acm_remap_plan;
+int32_t acm_remap_plan_create(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam,
+                              const double* target_intrinsics, int32_t interpolation, acm_remap_plan** out);
+int32_t acm_remap_plan_destroy(acm_ctx* ctx, acm_remap_plan* plan);
+/* n_frames frames, Wi*Hi*3 bytes each in, Wo*Ho*3 bytes each out; n_frames == 0 is a no-op */
+int32_t acm_remap_rgb8(acm_ctx* ctx, const acm_remap_plan* plan, const uint8_t* d_frames_in, uint8_t* d_frames_out, size_t n_frames);
+int32_t acm_remap_rgb8_host(acm_ctx* ctx, const acm_remap_plan* plan, const uint8_t* frames_in, uint8_t* frames_out, size_t n_frames);
+/* the remap map itself: d_src_xy[2*(v*Wo+u)+{0,1}] over the output camera's grid, NaN where a step fails */
+int32_t acm_remap_map(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam, double* d_src_xy);
+
 /* util::compute_reprojection_error (reference src/util/error_metrics.rs:62-121) */
 typedef struct acm_projection_error {
     double rmse, min, max, mean, stddev, median;

@@ -341,6 +341,53 @@ inline std::vector<uint8_t> undistort_image(const std::vector<uint8_t>& image, u
     return out;
 }
 
+// RGB8 frames of `input`'s camera rendered as `output`'s camera sees them (beyond the reference: output.unproject,
+// input.project, interpolate_pixel of undistort.rs:51-105).  output == nullptr: undistort_image of `input` with `target`.
+// The source coordinates are computed once on the device (32 bytes per output pixel) and reused by every apply().
+class RemapPlan {
+public:
+    RemapPlan(const CameraModel& input, const CameraModel* output, const Intrinsics* target = nullptr, int interpolation = ACM_INTERP_BILINEAR)
+        : ctx_(&input.ctx()), in_(input.resolution), out_(output ? output->resolution : input.resolution) {
+        acm_camera ci = input.block(), co{};
+        if (output) co = output->block();
+        double t[4]; if (target) { t[0] = target->fx; t[1] = target->fy; t[2] = target->cx; t[3] = target->cy; }
+        ctx_->check(acm_remap_plan_create(ctx_->handle(), &ci, output ? &co : nullptr, target ? t : nullptr, interpolation, &h_));
+    }
+    ~RemapPlan() { if (h_) acm_remap_plan_destroy(ctx_->handle(), h_); }
+    RemapPlan(const RemapPlan&) = delete;
+    RemapPlan& operator=(const RemapPlan&) = delete;
+    // whole input frames (w*h*3 bytes each) on the host -> output frames
+    std::vector<uint8_t> apply(const std::vector<uint8_t>& frames) const {
+        const size_t fin = (size_t)in_.width * in_.height * 3;
+        if (frames.size() % fin != 0)
+            throw CameraModelError(ErrorKind::InvalidParams, "Invalid parameters: frames of " + std::to_string(frames.size()) +
+                                                                 " bytes don't match model " + std::to_string(in_.width) + "x" + std::to_string(in_.height));
+        const size_t n = frames.size() / fin;
+        std::vector<uint8_t> out(n * out_.width * out_.height * 3);
+        ctx_->check(acm_remap_rgb8_host(ctx_->handle(), h_, frames.data(), out.data(), n));
+        return out;
+    }
+    // frames resident on the device, enqueued on the context's stream
+    void apply_device(const uint8_t* d_in, uint8_t* d_out, size_t n_frames) const {
+        ctx_->check(acm_remap_rgb8(ctx_->handle(), h_, d_in, d_out, n_frames));
+    }
+    Resolution output_resolution() const { return out_; }
+    acm_remap_plan* handle() const { return h_; }
+private:
+    const Context* ctx_;
+    Resolution in_, out_;
+    acm_remap_plan* h_ = nullptr;
+};
+
+// one RGB8 image of `input`'s camera (w*h*3 bytes) as `output`'s camera sees it
+inline std::vector<uint8_t> remap_image(const std::vector<uint8_t>& image, uint32_t width, uint32_t height, const CameraModel& input,
+                                        const CameraModel& output, int interpolation = ACM_INTERP_BILINEAR) {
+    if (width != input.resolution.width || height != input.resolution.height || image.size() != (size_t)width * height * 3)
+        throw CameraModelError(ErrorKind::InvalidParams, "Invalid parameters: Image " + std::to_string(width) + "x" + std::to_string(height) + " doesn't match model " +
+                                                             std::to_string(input.resolution.width) + "x" + std::to_string(input.resolution.height));
+    return RemapPlan(input, &output, nullptr, interpolation).apply(image);
+}
+
 // ---- util::image_quality (image_quality.rs) on RGB8 interleaved images (w*h*3 bytes) --------------
 struct ImageQualityMetrics { double psnr, ssim; };   // image_quality.rs:20-26
 

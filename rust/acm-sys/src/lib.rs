@@ -29,6 +29,8 @@ pub const ACM_INTERP_BILINEAR: i32 = 1;
 pub struct acm_ctx { _private: [u8; 0] }
 #[repr(C)]
 pub struct acm_points { _private: [u8; 0] }
+#[repr(C)]
+pub struct acm_remap_plan { _private: [u8; 0] }
 
 #[repr(C)]
 #[derive(Clone, Copy, Debug)]
@@ -150,6 +152,12 @@ extern "C" {
     pub fn acm_undistort_rgb8(ctx: *mut acm_ctx, cam: *const acm_camera, target_intrinsics: *const f64, d_frames_in: *const u8, d_frames_out: *mut u8, n_frames: size_t, interpolation: i32) -> i32;
     pub fn acm_undistort_rgb8_host(ctx: *mut acm_ctx, cam: *const acm_camera, target_intrinsics: *const f64, frames_in: *const u8, frames_out: *mut u8, n_frames: size_t, interpolation: i32) -> i32;
     pub fn acm_undistort_map(ctx: *mut acm_ctx, cam: *const acm_camera, target_intrinsics: *const f64, d_src_xy: *mut f64) -> i32;
+
+    pub fn acm_remap_plan_create(ctx: *mut acm_ctx, input_cam: *const acm_camera, output_cam: *const acm_camera, target_intrinsics: *const f64, interpolation: i32, out: *mut *mut acm_remap_plan) -> i32;
+    pub fn acm_remap_plan_destroy(ctx: *mut acm_ctx, plan: *mut acm_remap_plan) -> i32;
+    pub fn acm_remap_rgb8(ctx: *mut acm_ctx, plan: *const acm_remap_plan, d_frames_in: *const u8, d_frames_out: *mut u8, n_frames: size_t) -> i32;
+    pub fn acm_remap_rgb8_host(ctx: *mut acm_ctx, plan: *const acm_remap_plan, frames_in: *const u8, frames_out: *mut u8, n_frames: size_t) -> i32;
+    pub fn acm_remap_map(ctx: *mut acm_ctx, input_cam: *const acm_camera, output_cam: *const acm_camera, d_src_xy: *mut f64) -> i32;
 
     pub fn acm_reprojection_error(ctx: *mut acm_ctx, cam: *const acm_camera, xyz: *const acm_points, uv: *const acm_points, out: *mut acm_projection_error) -> i32;
     pub fn acm_sample_points(ctx: *mut acm_ctx, cam: *const acm_camera, n_requested: size_t, uv_out: *mut *mut acm_points, xyz_out: *mut *mut acm_points, n_kept: *mut size_t) -> i32;

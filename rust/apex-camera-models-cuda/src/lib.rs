@@ -303,6 +303,24 @@ impl<M: CameraModel> GpuCamera<M> {
         if rc != sys::ACM_OK { Err(self.ctx.err(rc)) } else { Ok(out) }
     }
 
+    /// Remap plan from this camera to `output` (`None`: `undistort_image` with `target`); see [`RemapPlan`].
+    pub fn remap_plan<O: CameraModel>(&self, output: Option<&GpuCamera<O>>, target: Option<Intrinsics>, interpolation: i32)
+        -> Result<RemapPlan, CameraModelError> {
+        let cam = self.block();
+        let out_cam = output.map(|o| o.block());
+        let (wo, ho) = match output { Some(o) => { let r = o.inner.get_resolution(); (r.width, r.height) } None => { let r = self.inner.get_resolution(); (r.width, r.height) } };
+        let r = self.inner.get_resolution();
+        let t = target.map(|t| [t.fx, t.fy, t.cx, t.cy]);
+        let mut h: *mut sys::acm_remap_plan = ptr::null_mut();
+        let _g = self.ctx.lock();
+        let rc = unsafe {
+            sys::acm_remap_plan_create(self.ctx.0, &cam, out_cam.as_ref().map_or(ptr::null(), |c| c as *const sys::acm_camera),
+                                       t.as_ref().map_or(ptr::null(), |a| a.as_ptr()), interpolation, &mut h)
+        };
+        if rc != sys::ACM_OK { return Err(self.ctx.err(rc)); }
+        Ok(RemapPlan { h, ctx: self.ctx.clone(), wi: r.width, hi: r.height, wo, ho })
+    }
+
     /// README-era `project(&p, compute_jacobian = true)`: uv plus the 2xP Jacobian w.r.t. `[fx, fy, cx, cy, dist..]`
     /// (per-model docs, double_sphere.rs:326-332) and the 2x3 Jacobian w.r.t. the 3-D point (trait doc, mod.rs:246-252).
     pub fn project_with_jacobians(&self, p: &Vector3<f64>)
@@ -561,6 +579,41 @@ impl DeviceGroup {
 }
 impl Drop for DeviceGroup {
     fn drop(&mut self) { unsafe { sys::acm_comm_destroy_all(self.raw.as_mut_ptr(), self.raw.len() as i32); } }
+}
+
+/// RGB8 frames of one camera rendered as another camera sees them (beyond the reference: the output camera's
+/// `unproject`, the input camera's `project`, then `interpolate_pixel`, undistort.rs:51-105).  The source coordinates
+/// are computed once on the device (32 bytes per output pixel) and reused by every `apply`; dropped with the plan.
+pub struct RemapPlan { h: *mut sys::acm_remap_plan, ctx: Arc<Context>, wi: u32, hi: u32, wo: u32, ho: u32 }
+unsafe impl Send for RemapPlan {}
+
+impl RemapPlan {
+    /// `frames`: whole Wi x Hi RGB8 frames of the input camera; returns the Wo x Ho frames of the output camera.
+    pub fn apply(&self, frames: &[u8]) -> Result<Vec<u8>, CameraModelError> {
+        let fin = self.wi as usize * self.hi as usize * 3;
+        if frames.len() % fin != 0 {   // undistort.rs:23-28
+            return Err(CameraModelError::InvalidParams(format!("frames of {} bytes don't match model {}x{}", frames.len(), self.wi, self.hi)));
+        }
+        let n = frames.len() / fin;
+        let mut out = vec![0u8; n * self.wo as usize * self.ho as usize * 3];
+        let _g = self.ctx.lock();
+        let rc = unsafe { sys::acm_remap_rgb8_host(self.ctx.0, self.h, frames.as_ptr(), out.as_mut_ptr(), n) };
+        if rc != sys::ACM_OK { Err(self.ctx.err(rc)) } else { Ok(out) }
+    }
+    /// Frames resident on the plan's device, enqueued on the context's stream.
+    ///
+    /// # Safety
+    /// `d_in` / `d_out` must be device buffers of `n_frames` input / output frames.
+    pub unsafe fn apply_device(&self, d_in: *const u8, d_out: *mut u8, n_frames: usize) -> Result<(), CameraModelError> {
+        let _g = self.ctx.lock();
+        let rc = sys::acm_remap_rgb8(self.ctx.0, self.h, d_in, d_out, n_frames);
+        if rc != sys::ACM_OK { Err(self.ctx.err(rc)) } else { Ok(()) }
+    }
+    /// Output resolution (width, height).
+    pub fn output_size(&self) -> (u32, u32) { (self.wo, self.ho) }
+}
+impl Drop for RemapPlan {
+    fn drop(&mut self) { let _g = self.ctx.lock(); unsafe { sys::acm_remap_plan_destroy(self.ctx.0, self.h); } }
 }
 
 /// `util::ImageQualityMetrics` (image_quality.rs:20-26).

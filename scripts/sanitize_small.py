@@ -24,6 +24,10 @@ for interp in (acm.InterpolationMethod.Bilinear, acm.InterpolationMethod.Nearest
     out = acm.undistort_images(frames, kb, None, interp)
     out2 = acm.undistort_images(frames, kb, acm.Intrinsics(100.0, 100.0, 256.0, 256.0), interp)  # zoom-out: list kernel
     print("undistort", int(interp), out.mean(), out2.mean())
+ds = acm.DoubleSphereModel(acm.Intrinsics(150.0, 150.0, 192.3, 143.8), acm.Resolution(384, 288), [0.56, -0.24], ctx=ctx)
+for interp in (acm.InterpolationMethod.Bilinear, acm.InterpolationMethod.Nearest):  # remap plans: TMA + leftover gather, byte kernel
+    with acm.RemapPlan(kb, ds, None, interp) as plan, acm.RemapPlan(ds, kb, None, interp) as back:
+        print("remap", int(interp), plan.apply(frames).mean(), back.apply(frames[:, :288, :384]).mean(), acm.remap_map(kb, ds).shape)
 ctx.sync()
 print("ok")
 # round 2: scalar host path (mapped staging + completion flag), small batches, Jacobian kernels (vector and scalar forms)
