@@ -111,6 +111,9 @@ SIGNATURES = {
     "acm_remap_rgb8": (C.c_int32, [_vp, _vp, _vp, _vp, C.c_size_t]),
     "acm_remap_rgb8_host": (C.c_int32, [_vp, _vp, _vp, _vp, C.c_size_t]),
     "acm_remap_map": (C.c_int32, [_vp, _cam, _cam, _vp]),
+    "acm_remap_plan_create_rotated": (C.c_int32, [_vp, _cam, _cam, _dp, C.c_int32, C.POINTER(_vp)]),
+    "acm_remap_map_rotated": (C.c_int32, [_vp, _cam, _cam, _dp, _vp]),
+    "acm_stereo_rectify": (C.c_int32, [_dp, _dp, _dp, _dp, _dp, C.POINTER(C.c_int32)]),
     "acm_reprojection_error": (C.c_int32, [_vp, _cam, _vp, _vp, C.POINTER(ProjectionError)]),
     "acm_sample_points": (C.c_int32, [_vp, _cam, C.c_size_t, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(C.c_size_t)]),
     "acm_sample_points_shard": (C.c_int32, [_vp, _cam, C.c_size_t, C.c_int32, C.c_int32, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(C.c_size_t)]),

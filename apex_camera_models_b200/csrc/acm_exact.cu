@@ -8,6 +8,8 @@
 // per thread (2 f64 or 4 f32 points), grid-stride loop over a grid of sm_count * k blocks.
 #include <stdlib.h>
 
+#include <cmath>
+#include <cstring>
 #include <new>
 
 #include <cuda.h>
@@ -1082,24 +1084,40 @@ extern "C" int32_t acm_undistort_map(acm_ctx* ctx, const acm_camera* cam, const 
 // interpolate_pixel of undistort.rs:51-105 on the input frame; black where a step fails.  Both steps keep their IEEE
 // forms (unproject<true> as acm_unproject_ieee, the non-FAST project<true> as undistort), so the map of the five
 // arithmetic-only models is bit-identical to the oracle's.
+// A rotated map (stereo rectification; OpenCV's R1 / R2) puts ray_in = R^T ray_out between the two steps, with R taking
+// input-camera coordinates to output-camera ones (x_out = R x_in).  The rotation is a uniform kernel argument, not a
+// template axis, so the 49 instantiations stay 49; unrotated launches skip it and run the operations they always ran.
 // ---------------------------------------------------------------------------------------
+struct Rot3 {
+    double r[9];  // row-major
+};
+
 template <int MI, int MO>
 __global__ void __launch_bounds__(256) remap_map_kernel(const __grid_constant__ CamParams ci, const __grid_constant__ CamParams co,
-                                                        double* __restrict__ src_xy, int W, int H) {
+                                                        const __grid_constant__ Rot3 R, int rotated, double* __restrict__ src_xy,
+                                                        int W, int H) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (size_t)W * H) return;
     const int uo = (int)(i % W), vo = (int)(i / W);
     double x, y, z, sx, sy;
     int st = CamModel<MO>::template unproject<true>(co, (double)uo, (double)vo, x, y, z);
+    if (rotated && st == ACM_POINT_OK) {  // ray_in[k] = (R[0][k] x + R[1][k] y) + R[2][k] z, each operation rounded (-fmad=false)
+        const double* r = R.r;
+        const double xi = (r[0] * x + r[3] * y) + r[6] * z;
+        const double yi = (r[1] * x + r[4] * y) + r[7] * z;
+        const double zi = (r[2] * x + r[5] * y) + r[8] * z;
+        x = xi; y = yi; z = zi;
+    }
     if (st == ACM_POINT_OK) st = CamModel<MI>::template project<true>(ci, x, y, z, sx, sy);
     if (st != ACM_POINT_OK) sx = sy = acm_nan();
     reinterpret_cast<double2*>(src_xy)[i] = make_double2(sx, sy);
 }
 
 template <int MO>
-static int32_t launch_remap_map(acm_ctx* ctx, const CamParams& ci, const CamParams& co, double* d_src_xy, int W, int H) {
+static int32_t launch_remap_map(acm_ctx* ctx, const CamParams& ci, const CamParams& co, const Rot3& R, int rotated, double* d_src_xy,
+                                int W, int H) {
     const int grid = (int)(((size_t)W * H + 255) / 256);
-    ACM_DISPATCH_MODEL(ci.model, (remap_map_kernel<M, MO><<<grid, 256, 0, ctx->stream>>>(ci, co, d_src_xy, W, H)))
+    ACM_DISPATCH_MODEL(ci.model, (remap_map_kernel<M, MO><<<grid, 256, 0, ctx->stream>>>(ci, co, R, rotated, d_src_xy, W, H)))
     ACM_CHECK_LAUNCH(ctx);
     return ACM_OK;
 }
@@ -1113,24 +1131,56 @@ static int32_t check_frame_camera(acm_ctx* ctx, const acm_camera* cam, const cha
     return ACM_OK;
 }
 
-// source coordinates of every pixel of output_cam's grid: the remap map of input_cam -> output_cam
-static int32_t remap_map(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam, double* d_src_xy) {
+// R must be a proper rotation: finite entries, max |R R^T - I| <= 1e-9, det R > 0.  ctx may be null (acm_stereo_rectify).
+static int32_t check_rotation(acm_ctx* ctx, const double* R, const char* who) {
+    if (!R) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: null rotation", who);
+    for (int k = 0; k < 9; ++k)
+        if (!std::isfinite(R[k])) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: rotation has a non-finite entry", who);
+    double dev = 0.0;
+    for (int i = 0; i < 3; ++i)
+        for (int j = 0; j < 3; ++j) {
+            const double d = R[3 * i] * R[3 * j] + R[3 * i + 1] * R[3 * j + 1] + R[3 * i + 2] * R[3 * j + 2] - (i == j ? 1.0 : 0.0);
+            dev = std::fmax(dev, std::fabs(d));
+        }
+    if (!(dev <= 1e-9)) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: rotation is not orthonormal (max |R R^T - I| = %.3g > 1e-9)", who, dev);
+    const double det = R[0] * (R[4] * R[8] - R[5] * R[7]) - R[1] * (R[3] * R[8] - R[5] * R[6]) + R[2] * (R[3] * R[7] - R[4] * R[6]);
+    if (det < 0.0) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: rotation is a reflection (det R < 0)", who);
+    return ACM_OK;
+}
+
+// source coordinates of every pixel of output_cam's grid: the remap map of input_cam -> output_cam, rotated by R unless it is
+// null (R checked by the caller)
+static int32_t remap_map(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam, const double* R, double* d_src_xy) {
     CamParams ci, co;
     int32_t rc = acm_make_cam_params(ctx, input_cam, &ci);
     if (!rc) rc = acm_make_cam_params(ctx, output_cam, &co);
     if (rc) return rc;
+    Rot3 rot{};
+    if (R) std::memcpy(rot.r, R, sizeof(rot.r));
     const int W = (int)output_cam->width, H = (int)output_cam->height;
-    ACM_DISPATCH_MODEL(co.model, return launch_remap_map<M>(ctx, ci, co, d_src_xy, W, H))
+    ACM_DISPATCH_MODEL(co.model, return launch_remap_map<M>(ctx, ci, co, rot, R != nullptr, d_src_xy, W, H))
     return ACM_OK;
 }
 
-extern "C" int32_t acm_remap_map(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam, double* d_src_xy) {
-    ACM_ENTER(ctx);
+static int32_t remap_map_entry(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam, const double* R, double* d_src_xy) {
     int32_t rc = check_frame_camera(ctx, input_cam, "input");
     if (!rc) rc = check_frame_camera(ctx, output_cam, "output");
     if (rc) return rc;
     ACM_REQUIRE(ctx, d_src_xy, "remap_map: null output");
-    return remap_map(ctx, input_cam, output_cam, d_src_xy);
+    return remap_map(ctx, input_cam, output_cam, R, d_src_xy);
+}
+
+extern "C" int32_t acm_remap_map(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam, double* d_src_xy) {
+    ACM_ENTER(ctx);
+    return remap_map_entry(ctx, input_cam, output_cam, nullptr, d_src_xy);
+}
+
+extern "C" int32_t acm_remap_map_rotated(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam, const double R[9],
+                                         double* d_src_xy) {
+    ACM_ENTER(ctx);
+    const int32_t rc = check_rotation(ctx, R, "remap_map");
+    if (rc) return rc;
+    return remap_map_entry(ctx, input_cam, output_cam, R, d_src_xy);
 }
 
 // A plan: the f64 map (16 B per output pixel, read by the byte kernel and the exact re-blend) and the packed records
@@ -1158,11 +1208,9 @@ static void free_plan(acm_remap_plan* p) {
     delete p;
 }
 
-extern "C" int32_t acm_remap_plan_create(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam,
-                                         const double* target_intrinsics, int32_t interpolation, acm_remap_plan** out) {
-    ACM_ENTER(ctx);
-    ACM_REQUIRE(ctx, out, "remap_plan: null output");
-    *out = nullptr;
+// R: null, or a checked rotation with output_cam != null
+static int32_t create_plan(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam, const double* target_intrinsics,
+                           const double* R, int32_t interpolation, acm_remap_plan** out) {
     ACM_REQUIRE(ctx, !(output_cam && target_intrinsics), "remap_plan: give either an output camera or target intrinsics, not both");
     int32_t rc = check_frame_camera(ctx, input_cam, "input");
     if (!rc && output_cam) rc = check_frame_camera(ctx, output_cam, "output");
@@ -1180,7 +1228,7 @@ extern "C" int32_t acm_remap_plan_create(acm_ctx* ctx, const acm_camera* input_c
     rc = acm_device_malloc(ctx, reinterpret_cast<void**>(&p->d_map), n * sizeof(double2));
     if (!rc) rc = acm_device_malloc(ctx, reinterpret_cast<void**>(&p->d_rec), n * sizeof(uint4));
     if (!rc && output_cam) {
-        rc = remap_map(ctx, input_cam, output_cam, reinterpret_cast<double*>(p->d_map));
+        rc = remap_map(ctx, input_cam, output_cam, R, reinterpret_cast<double*>(p->d_map));
     } else if (!rc) {  // undistort_image semantics: the map of acm_undistort_map
         double t[4];
         for (int i = 0; i < 4; ++i) t[i] = target_intrinsics ? target_intrinsics[i] : input_cam->params[i];
@@ -1194,6 +1242,25 @@ extern "C" int32_t acm_remap_plan_create(acm_ctx* ctx, const acm_camera* input_c
     }
     *out = p;
     return ACM_OK;
+}
+
+extern "C" int32_t acm_remap_plan_create(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam,
+                                         const double* target_intrinsics, int32_t interpolation, acm_remap_plan** out) {
+    ACM_ENTER(ctx);
+    ACM_REQUIRE(ctx, out, "remap_plan: null output");
+    *out = nullptr;
+    return create_plan(ctx, input_cam, output_cam, target_intrinsics, nullptr, interpolation, out);
+}
+
+extern "C" int32_t acm_remap_plan_create_rotated(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam,
+                                                 const double R[9], int32_t interpolation, acm_remap_plan** out) {
+    ACM_ENTER(ctx);
+    ACM_REQUIRE(ctx, out, "remap_plan: null output");
+    *out = nullptr;
+    ACM_REQUIRE(ctx, output_cam, "remap_plan: a rotated plan needs an output camera (a Pinhole camera gives undistort_image's view)");
+    const int32_t rc = check_rotation(ctx, R, "remap_plan");
+    if (rc) return rc;
+    return create_plan(ctx, input_cam, output_cam, nullptr, R, interpolation, out);
 }
 
 extern "C" int32_t acm_remap_plan_destroy(acm_ctx* ctx, acm_remap_plan* plan) {
@@ -1254,6 +1321,102 @@ extern "C" int32_t acm_remap_rgb8_host(acm_ctx* ctx, const acm_remap_plan* plan,
     if (d_in) cudaFree(d_in);
     if (d_out) cudaFree(d_out);
     return rc;
+}
+
+// ---------------------------------------------------------------------------------------
+// Stereo rectification (host only): the rotation part of OpenCV's cvStereoRectify (Bouguet).  Its R1 / R2 feed
+// acm_remap_plan_create_rotated with one pinhole camera shared by both views.
+// ---------------------------------------------------------------------------------------
+// Rodrigues vector -> matrix: R = cos t I + (1 - cos t)/t^2 w w^T + (sin t / t) [w]x with t = |w|.  1 - cos t is taken as
+// 2 sin^2(t/2) and the ratios are formed before squaring, so tiny angles keep every digit; w = 0 gives I exactly.
+static void rodrigues_matrix(const double w[3], double R[9]) {
+    const double t = std::sqrt(w[0] * w[0] + w[1] * w[1] + w[2] * w[2]);
+    double a = 1.0, b = 0.5, c = 1.0;  // sin t / t, (1 - cos t) / t^2, cos t
+    if (t > 0.0) {
+        const double h = std::sin(0.5 * t) / t;
+        a = std::sin(t) / t;
+        b = 2.0 * h * h;
+        c = std::cos(t);
+    }
+    R[0] = c + b * w[0] * w[0];         R[1] = b * w[0] * w[1] - a * w[2];  R[2] = b * w[0] * w[2] + a * w[1];
+    R[3] = b * w[1] * w[0] + a * w[2];  R[4] = c + b * w[1] * w[1];         R[5] = b * w[1] * w[2] - a * w[0];
+    R[6] = b * w[2] * w[0] - a * w[1];  R[7] = b * w[2] * w[1] + a * w[0];  R[8] = c + b * w[2] * w[2];
+}
+
+// Rodrigues matrix -> vector of a rotation.  s = vee(R - R^T)/2 = sin t k, c = (trace R - 1)/2, t = atan2(|s|, c).  For c >= 0
+// the axis is s / |s| and w = s t/|s|, which tends to s as t -> 0: unlike OpenCV's Rodrigues, which returns 0 below
+// sin t = 1e-5, a 1e-9 rad rotation keeps its 1e-9.  For c < 0 (t > 90 degrees, |s| -> 0 towards 180) the axis comes from
+// the symmetric part, (R + R^T)/2 - c I = (1 - c) k k^T, through its largest diagonal entry (k_i^2 >= 1/3), signed to
+// agree with s.
+static void rodrigues_vector(const double R[9], double w[3]) {
+    const double s[3] = {0.5 * (R[7] - R[5]), 0.5 * (R[2] - R[6]), 0.5 * (R[3] - R[1])};
+    const double sn = std::sqrt(s[0] * s[0] + s[1] * s[1] + s[2] * s[2]);
+    const double c = 0.5 * (R[0] + R[4] + R[8] - 1.0);
+    const double t = std::atan2(sn, c);
+    if (c >= 0.0) {
+        const double f = sn > 0.0 ? t / sn : 1.0;
+        for (int j = 0; j < 3; ++j) w[j] = s[j] * f;
+        return;
+    }
+    int i = R[4] > R[0] ? 1 : 0;
+    if (R[8] > R[4 * i]) i = 2;
+    const double d = 1.0 - c;
+    double k[3];
+    k[i] = std::sqrt(std::fmax((R[4 * i] - c) / d, 0.0));
+    for (int j = 0; j < 3; ++j)
+        if (j != i) k[j] = 0.5 * (R[3 * i + j] + R[3 * j + i]) / (d * k[i]);
+    const double sign = k[0] * s[0] + k[1] * s[1] + k[2] * s[2] < 0.0 ? -1.0 : 1.0;
+    for (int j = 0; j < 3; ++j) w[j] = sign * t * k[j];
+}
+
+// C = A B (transpose_b: A B^T), 3 x 3 row-major
+static void mat3_mul(const double* A, const double* B, bool transpose_b, double* C) {
+    for (int i = 0; i < 3; ++i)
+        for (int j = 0; j < 3; ++j) {
+            double acc = 0.0;
+            for (int k = 0; k < 3; ++k) acc += A[3 * i + k] * (transpose_b ? B[3 * j + k] : B[3 * k + j]);
+            C[3 * i + j] = acc;
+        }
+}
+
+static void mat3_vec(const double* A, const double* x, double* y) {
+    for (int i = 0; i < 3; ++i) y[i] = A[3 * i] * x[0] + A[3 * i + 1] * x[1] + A[3 * i + 2] * x[2];
+}
+
+extern "C" int32_t acm_stereo_rectify(const double R[9], const double t[3], double R1[9], double R2[9], double* baseline,
+                                      int32_t* vertical) {
+    if (!t || !R1 || !R2 || !baseline || !vertical) return acm_fail(nullptr, ACM_ERR_INVALID_ARG, "stereo_rectify: null argument");
+    const int32_t rc = check_rotation(nullptr, R, "stereo_rectify");
+    if (rc) return rc;
+    if (!std::isfinite(t[0]) || !std::isfinite(t[1]) || !std::isfinite(t[2]))
+        return acm_fail(nullptr, ACM_ERR_INVALID_ARG, "stereo_rectify: translation has a non-finite entry");
+    if (t[0] == 0.0 && t[1] == 0.0 && t[2] == 0.0)
+        return acm_fail(nullptr, ACM_ERR_INVALID_ARG, "stereo_rectify: translation is zero (no baseline)");
+    // half the relative rotation each way brings both cameras to the same orientation
+    double om[3], r_r[9], tp[3];
+    rodrigues_vector(R, om);
+    for (int j = 0; j < 3; ++j) om[j] *= -0.5;
+    rodrigues_matrix(om, r_r);
+    mat3_vec(r_r, t, tp);
+    // then one common rotation takes the baseline t' onto the x axis (or the y axis when the pair is stacked vertically)
+    const int idx = std::fabs(tp[0]) > std::fabs(tp[1]) ? 0 : 1;
+    const double c = tp[idx], nt = std::sqrt(tp[0] * tp[0] + tp[1] * tp[1] + tp[2] * tp[2]);
+    double uu[3] = {0.0, 0.0, 0.0};
+    uu[idx] = c > 0.0 ? 1.0 : -1.0;
+    double ww[3] = {tp[1] * uu[2] - tp[2] * uu[1], tp[2] * uu[0] - tp[0] * uu[2], tp[0] * uu[1] - tp[1] * uu[0]};
+    const double nw = std::sqrt(ww[0] * ww[0] + ww[1] * ww[1] + ww[2] * ww[2]);
+    if (nw > 0.0) {
+        const double f = std::acos(std::fmin(std::fabs(c) / nt, 1.0)) / nw;
+        for (int j = 0; j < 3; ++j) ww[j] *= f;
+    }
+    double wR[9], t2[3];
+    rodrigues_matrix(ww, wR);
+    mat3_mul(wR, r_r, true, R1);
+    mat3_mul(wR, r_r, false, R2);
+    mat3_vec(R2, t, t2);
+    *baseline = t2[idx];
+    *vertical = idx;
+    return ACM_OK;
 }
 
 // ---------------------------------------------------------------------------------------

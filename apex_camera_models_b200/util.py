@@ -1,6 +1,7 @@
 """util hot loops of the reference: undistort_image (src/util/undistort.rs:14-105), sample_points
 (src/util/point_sampling.rs:46-120), compute_reprojection_error (src/util/error_metrics.rs:62-121); and remap plans
-(camera-to-camera image remap, composed of the reference's unproject, project and interpolate_pixel)."""
+(camera-to-camera image remap, composed of the reference's unproject, project and interpolate_pixel), rotated plans and
+stereo rectification."""
 from __future__ import annotations
 
 import ctypes as C
@@ -10,8 +11,8 @@ from dataclasses import dataclass
 import numpy as np
 
 from . import _native as N
-from .camera import CameraModel, Intrinsics
-from .errors import UtilError
+from .camera import CameraModel, Intrinsics, PinholeModel
+from .errors import UtilError, raise_call_status
 from .runtime import Points
 
 _lib = N.lib
@@ -37,6 +38,18 @@ def _target_array(target: Intrinsics | None):
     if target is None:
         return None
     return (C.c_double * 4)(target.fx, target.fy, target.cx, target.cy)
+
+
+def _matrix3(a, what: str) -> np.ndarray:
+    m = np.array(a, dtype=np.float64)
+    if m.shape != (3, 3):
+        raise UtilError(f"Invalid parameters: {what} must be a 3x3 matrix, got shape {m.shape}")
+    return m
+
+
+def _rotation_array(rotation):
+    """Row-major double[9] of a 3x3 rotation (libacm checks that it is one)."""
+    return (C.c_double * 9)(*_matrix3(rotation, "rotation").ravel())
 
 
 def undistort_images(frames: np.ndarray, camera_model: CameraModel, target_intrinsics: Intrinsics | None = None,
@@ -101,15 +114,23 @@ class RemapPlan:
     until `close()`."""
 
     def __init__(self, input_model: CameraModel, output_model: CameraModel | None = None, target_intrinsics: Intrinsics | None = None,
-                 interpolation: InterpolationMethod = InterpolationMethod.Bilinear):
+                 interpolation: InterpolationMethod = InterpolationMethod.Bilinear, *, rotation=None):
+        """`rotation`: a 3x3 rotation R with x_out = R x_in (OpenCV's R1 / R2), applied between the output camera's
+        unproject and the input camera's project as ray_in = R^T ray_out.  It needs an output camera."""
         self.ctx = input_model.ctx
         self.input_model = input_model
         self.output_resolution = (output_model or input_model).get_resolution()
         cin = input_model.camera_block()
         cout = output_model.camera_block() if output_model is not None else None
         h = C.c_void_p()
-        self.ctx.check(_lib.acm_remap_plan_create(self.ctx.handle, C.byref(cin), C.byref(cout) if cout is not None else None,
-                                                  _target_array(target_intrinsics), int(interpolation), C.byref(h)))
+        if rotation is not None:
+            if output_model is None or target_intrinsics is not None:
+                raise UtilError("Invalid parameters: a rotated remap plan needs an output camera and no target intrinsics")
+            self.ctx.check(_lib.acm_remap_plan_create_rotated(self.ctx.handle, C.byref(cin), C.byref(cout), _rotation_array(rotation),
+                                                              int(interpolation), C.byref(h)))
+        else:
+            self.ctx.check(_lib.acm_remap_plan_create(self.ctx.handle, C.byref(cin), C.byref(cout) if cout is not None else None,
+                                                      _target_array(target_intrinsics), int(interpolation), C.byref(h)))
         self._h = h
 
     @property
@@ -166,20 +187,80 @@ def remap_image(input_image: np.ndarray, input_model: CameraModel, output_model:
     return remap_images(img[None], input_model, output_model, interpolation)[0]
 
 
-def remap_map(input_model: CameraModel, output_model: CameraModel) -> np.ndarray:
-    """(Ho, Wo, 2) source coordinates on the input frame of every output pixel (NaN where a step fails)."""
+def remap_map(input_model: CameraModel, output_model: CameraModel, rotation=None) -> np.ndarray:
+    """(Ho, Wo, 2) source coordinates on the input frame of every output pixel (NaN where a step fails); `rotation` as in
+    `RemapPlan`."""
     ctx = input_model.ctx
     cin, cout = input_model.camera_block(), output_model.camera_block()
     res = output_model.get_resolution()
     d = ctx.device_alloc(max(res.width * res.height, 1) * 16)
     try:
-        ctx.check(_lib.acm_remap_map(ctx.handle, C.byref(cin), C.byref(cout), C.c_void_p(d)))
+        if rotation is not None:
+            ctx.check(_lib.acm_remap_map_rotated(ctx.handle, C.byref(cin), C.byref(cout), _rotation_array(rotation), C.c_void_p(d)))
+        else:
+            ctx.check(_lib.acm_remap_map(ctx.handle, C.byref(cin), C.byref(cout), C.c_void_p(d)))
         out = np.empty((res.height, res.width, 2))
         ctx.d2h(out, d)
         ctx.sync()
     finally:
         ctx.device_free(d)
     return out
+
+
+def stereo_rectify(R, t):
+    """Bouguet rectification of a calibrated pair (the rotation part of OpenCV's `stereoRectify`), x_cam2 = R x_cam1 + t.
+    Returns (R1, R2, baseline, vertical): x_rect1 = R1 x_cam1, x_rect2 = R2 x_cam2; `baseline` is the signed component
+    of R2 t along the rectified baseline axis, which is x, or y when `vertical` (the pair is stacked vertically).  Host
+    only; no device needed."""
+    Rm = _rotation_array(R)
+    tv = np.array(t, dtype=np.float64).ravel()
+    if tv.shape != (3,):
+        raise UtilError(f"Invalid parameters: translation must have 3 entries, got {tv.size}")
+    R1, R2 = (C.c_double * 9)(), (C.c_double * 9)()
+    baseline, vertical = C.c_double(), C.c_int32()
+    rc = _lib.acm_stereo_rectify(Rm, (C.c_double * 3)(*tv), R1, R2, C.byref(baseline), C.byref(vertical))
+    if rc != N.OK:
+        raise_call_status(rc, _lib.acm_last_error(None).decode())
+    return np.array(R1[:]).reshape(3, 3), np.array(R2[:]).reshape(3, 3), baseline.value, bool(vertical.value)
+
+
+class StereoRectifier:
+    """Rectifies frames of a calibrated pair (x_cam2 = R x_cam1 + t) onto one caller-chosen Pinhole camera shared by both
+    views: two rotated remap plans, `left` through R1 and `right` through R2 of `stereo_rectify(R, t)`.  Rectified rows
+    correspond (columns when `vertical`); P1 = K [I | 0] and P2 = K [I | baseline e] with e the x (or y) axis.  Any
+    camera models work on either side.  The plans stay on the device until `close()`."""
+
+    def __init__(self, left: CameraModel, right: CameraModel, R, t, rectified_pinhole: CameraModel,
+                 interpolation: InterpolationMethod = InterpolationMethod.Bilinear):
+        if not isinstance(rectified_pinhole, PinholeModel):
+            raise UtilError("Invalid parameters: the rectified camera must be a PinholeModel")
+        self.R1, self.R2, self.baseline, self.vertical = stereo_rectify(R, t)
+        i = rectified_pinhole.get_intrinsics()
+        K = np.array([[i.fx, 0.0, i.cx], [0.0, i.fy, i.cy], [0.0, 0.0, 1.0]])
+        e = np.zeros((3, 1))
+        e[1 if self.vertical else 0, 0] = self.baseline
+        self.P1 = K @ np.hstack([np.eye(3), np.zeros((3, 1))])
+        self.P2 = K @ np.hstack([np.eye(3), e])
+        self.left_plan = RemapPlan(left, rectified_pinhole, None, interpolation, rotation=self.R1)
+        try:
+            self.right_plan = RemapPlan(right, rectified_pinhole, None, interpolation, rotation=self.R2)
+        except Exception:
+            self.left_plan.close()
+            raise
+
+    def apply(self, left_frames: np.ndarray, right_frames: np.ndarray) -> tuple[np.ndarray, np.ndarray]:
+        """(F, H, W, 3) uint8 frames of each camera -> both rectified batches (F, Ho, Wo, 3)."""
+        return self.left_plan.apply(left_frames), self.right_plan.apply(right_frames)
+
+    def close(self) -> None:
+        self.left_plan.close()
+        self.right_plan.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
 
 
 def sample_points(camera_model: CameraModel, n: int, device: bool = False, shard: tuple[int, int] | None = None):

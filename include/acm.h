@@ -248,6 +248,31 @@ int32_t acm_remap_rgb8_host(acm_ctx* ctx, const acm_remap_plan* plan, const uint
 /* the remap map itself: d_src_xy[2*(v*Wo+u)+{0,1}] over the output camera's grid, NaN where a step fails */
 int32_t acm_remap_map(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam, double* d_src_xy);
 
+/* ---- rotated remap plans and stereo rectification (beyond the reference) -----
+ * R: row-major 3x3 rotation taking input-camera coordinates to output-camera ones, x_out = R * x_in
+ * (OpenCV's R1 / R2, the R of initUndistortRectifyMap).  Output pixel (u, v): ray_o = output.unproject((u, v)),
+ * ray_i = R^T * ray_o (ray_i[k] = (R[0][k]*x + R[1][k]*y) + R[2][k]*z, each operation rounded), then
+ * src = input.project(ray_i); black / NaN where a step fails.  output_cam is required (a Pinhole output camera gives
+ * the rectified undistort view).  R must be finite, orthonormal to 1e-9 (max |R R^T - I|) and have det R > 0;
+ * otherwise ACM_ERR_INVALID_ARG.  Frames go through acm_remap_rgb8 / acm_remap_rgb8_host and the plan is freed by
+ * acm_remap_plan_destroy, as for any plan. */
+int32_t acm_remap_plan_create_rotated(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam,
+                                      const double R[9], int32_t interpolation, acm_remap_plan** out);
+/* the rotated remap map: d_src_xy[2*(v*Wo+u)+{0,1}] over the output camera's grid, NaN where a step fails */
+int32_t acm_remap_map_rotated(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam,
+                              const double R[9], double* d_src_xy);
+
+/* Bouguet rectification of a calibrated pair, the rotation part of OpenCV's stereoRectify, on the host (no context,
+ * no device): x_cam2 = R * x_cam1 + t.  Outputs R1, R2 (row-major; x_rect1 = R1 x_cam1, x_rect2 = R2 x_cam2) and
+ * *baseline = the signed component of R2 * t along the rectified baseline axis; *vertical = 1 when |t'_y| >= |t'_x|
+ * (t' = t rotated by half the relative rotation; the pair is stacked vertically and rows become columns, as in
+ * OpenCV), else 0.  With one Pinhole camera K shared by both views, P1 = K [I | 0] and P2 = K [I | baseline * e]
+ * with e = x (or y when vertical).  Unlike OpenCV, the Rodrigues conversions have no small-angle cut-off.
+ * ACM_ERR_INVALID_ARG (message in acm_last_error(NULL)) for a null argument, non-finite input, t = 0, or an R that
+ * is not a rotation (the check of acm_remap_plan_create_rotated). */
+int32_t acm_stereo_rectify(const double R[9], const double t[3], double R1[9], double R2[9],
+                           double* baseline, int32_t* vertical);
+
 /* util::compute_reprojection_error (reference src/util/error_metrics.rs:62-121) */
 typedef struct acm_projection_error {
     double rmse, min, max, mean, stddev, median;

@@ -353,6 +353,12 @@ public:
         double t[4]; if (target) { t[0] = target->fx; t[1] = target->fy; t[2] = target->cx; t[3] = target->cy; }
         ctx_->check(acm_remap_plan_create(ctx_->handle(), &ci, output ? &co : nullptr, target ? t : nullptr, interpolation, &h_));
     }
+    // rotated plan (stereo rectification): R row-major with x_out = R x_in (OpenCV's R1 / R2); ray_in = R^T ray_out
+    RemapPlan(const CameraModel& input, const CameraModel& output, const std::array<double, 9>& R, int interpolation = ACM_INTERP_BILINEAR)
+        : ctx_(&input.ctx()), in_(input.resolution), out_(output.resolution) {
+        const acm_camera ci = input.block(), co = output.block();
+        ctx_->check(acm_remap_plan_create_rotated(ctx_->handle(), &ci, &co, R.data(), interpolation, &h_));
+    }
     ~RemapPlan() { if (h_) acm_remap_plan_destroy(ctx_->handle(), h_); }
     RemapPlan(const RemapPlan&) = delete;
     RemapPlan& operator=(const RemapPlan&) = delete;
@@ -386,6 +392,24 @@ inline std::vector<uint8_t> remap_image(const std::vector<uint8_t>& image, uint3
         throw CameraModelError(ErrorKind::InvalidParams, "Invalid parameters: Image " + std::to_string(width) + "x" + std::to_string(height) + " doesn't match model " +
                                                              std::to_string(input.resolution.width) + "x" + std::to_string(input.resolution.height));
     return RemapPlan(input, &output, nullptr, interpolation).apply(image);
+}
+
+// Bouguet rectification of a calibrated pair, x_cam2 = R x_cam1 + t (the rotation part of OpenCV's stereoRectify; host
+// only).  x_rect1 = R1 x_cam1, x_rect2 = R2 x_cam2; baseline = the component of R2 t along x (along y when vertical).
+// With one Pinhole camera K for both views, P1 = K [I | 0] and P2 = K [I | baseline e].
+struct StereoRectification {
+    std::array<double, 9> R1, R2;
+    double baseline;
+    bool vertical;
+};
+
+inline StereoRectification stereo_rectify(const std::array<double, 9>& R, const std::array<double, 3>& t) {
+    StereoRectification s{};
+    int32_t vertical = 0;
+    const int32_t rc = acm_stereo_rectify(R.data(), t.data(), s.R1.data(), s.R2.data(), &s.baseline, &vertical);
+    if (rc != ACM_OK) throw_call_status(rc, acm_last_error(nullptr));
+    s.vertical = vertical != 0;
+    return s;
 }
 
 // ---- util::image_quality (image_quality.rs) on RGB8 interleaved images (w*h*3 bytes) --------------

@@ -158,6 +158,9 @@ extern "C" {
     pub fn acm_remap_rgb8(ctx: *mut acm_ctx, plan: *const acm_remap_plan, d_frames_in: *const u8, d_frames_out: *mut u8, n_frames: size_t) -> i32;
     pub fn acm_remap_rgb8_host(ctx: *mut acm_ctx, plan: *const acm_remap_plan, frames_in: *const u8, frames_out: *mut u8, n_frames: size_t) -> i32;
     pub fn acm_remap_map(ctx: *mut acm_ctx, input_cam: *const acm_camera, output_cam: *const acm_camera, d_src_xy: *mut f64) -> i32;
+    pub fn acm_remap_plan_create_rotated(ctx: *mut acm_ctx, input_cam: *const acm_camera, output_cam: *const acm_camera, r: *const f64, interpolation: i32, out: *mut *mut acm_remap_plan) -> i32;
+    pub fn acm_remap_map_rotated(ctx: *mut acm_ctx, input_cam: *const acm_camera, output_cam: *const acm_camera, r: *const f64, d_src_xy: *mut f64) -> i32;
+    pub fn acm_stereo_rectify(r: *const f64, t: *const f64, r1: *mut f64, r2: *mut f64, baseline: *mut f64, vertical: *mut i32) -> i32;
 
     pub fn acm_reprojection_error(ctx: *mut acm_ctx, cam: *const acm_camera, xyz: *const acm_points, uv: *const acm_points, out: *mut acm_projection_error) -> i32;
     pub fn acm_sample_points(ctx: *mut acm_ctx, cam: *const acm_camera, n_requested: size_t, uv_out: *mut *mut acm_points, xyz_out: *mut *mut acm_points, n_kept: *mut size_t) -> i32;

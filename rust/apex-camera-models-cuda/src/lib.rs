@@ -321,6 +321,19 @@ impl<M: CameraModel> GpuCamera<M> {
         Ok(RemapPlan { h, ctx: self.ctx.clone(), wi: r.width, hi: r.height, wo, ho })
     }
 
+    /// Rotated remap plan from this camera to `output` (stereo rectification): `r` row-major with x_out = R x_in
+    /// (OpenCV's R1 / R2, see [`stereo_rectify`]); the ray between the two models is R^T ray_out.
+    pub fn remap_plan_rotated<O: CameraModel>(&self, output: &GpuCamera<O>, r: &[f64; 9], interpolation: i32)
+        -> Result<RemapPlan, CameraModelError> {
+        let (cam, out_cam) = (self.block(), output.block());
+        let (ri, ro) = (self.inner.get_resolution(), output.inner.get_resolution());
+        let mut h: *mut sys::acm_remap_plan = ptr::null_mut();
+        let _g = self.ctx.lock();
+        let rc = unsafe { sys::acm_remap_plan_create_rotated(self.ctx.0, &cam, &out_cam, r.as_ptr(), interpolation, &mut h) };
+        if rc != sys::ACM_OK { return Err(self.ctx.err(rc)); }
+        Ok(RemapPlan { h, ctx: self.ctx.clone(), wi: ri.width, hi: ri.height, wo: ro.width, ho: ro.height })
+    }
+
     /// README-era `project(&p, compute_jacobian = true)`: uv plus the 2xP Jacobian w.r.t. `[fx, fy, cx, cy, dist..]`
     /// (per-model docs, double_sphere.rs:326-332) and the 2x3 Jacobian w.r.t. the 3-D point (trait doc, mod.rs:246-252).
     pub fn project_with_jacobians(&self, p: &Vector3<f64>)
@@ -614,6 +627,25 @@ impl RemapPlan {
 }
 impl Drop for RemapPlan {
     fn drop(&mut self) { let _g = self.ctx.lock(); unsafe { sys::acm_remap_plan_destroy(self.ctx.0, self.h); } }
+}
+
+/// Bouguet rectification of a calibrated pair, x_cam2 = R x_cam1 + t (the rotation part of OpenCV's `stereoRectify`;
+/// host only).  x_rect1 = R1 x_cam1, x_rect2 = R2 x_cam2; `baseline` is the component of R2 t along x (along y when
+/// `vertical`).  With one pinhole camera K for both views, P1 = K [I | 0] and P2 = K [I | baseline e].
+#[derive(Debug, Clone)]
+pub struct StereoRectification { pub r1: [f64; 9], pub r2: [f64; 9], pub baseline: f64, pub vertical: bool }
+
+/// `r` row-major, `t` as in x_cam2 = R x_cam1 + t; see [`StereoRectification`].
+pub fn stereo_rectify(r: &[f64; 9], t: &[f64; 3]) -> Result<StereoRectification, CameraModelError> {
+    let mut s = StereoRectification { r1: [0.0; 9], r2: [0.0; 9], baseline: 0.0, vertical: false };
+    let mut vertical = 0i32;
+    let rc = unsafe { sys::acm_stereo_rectify(r.as_ptr(), t.as_ptr(), s.r1.as_mut_ptr(), s.r2.as_mut_ptr(), &mut s.baseline, &mut vertical) };
+    if rc != sys::ACM_OK {
+        let msg = unsafe { CStr::from_ptr(sys::acm_last_error(ptr::null())) }.to_string_lossy().into_owned();
+        return Err(CameraModelError::InvalidParams(msg));
+    }
+    s.vertical = vertical != 0;
+    Ok(s)
 }
 
 /// `util::ImageQualityMetrics` (image_quality.rs:20-26).

@@ -28,6 +28,10 @@ ds = acm.DoubleSphereModel(acm.Intrinsics(150.0, 150.0, 192.3, 143.8), acm.Resol
 for interp in (acm.InterpolationMethod.Bilinear, acm.InterpolationMethod.Nearest):  # remap plans: TMA + leftover gather, byte kernel
     with acm.RemapPlan(kb, ds, None, interp) as plan, acm.RemapPlan(ds, kb, None, interp) as back:
         print("remap", int(interp), plan.apply(frames).mean(), back.apply(frames[:, :288, :384]).mean(), acm.remap_map(kb, ds).shape)
+c, s = np.cos(0.3), np.sin(0.3)
+R1, R2, _, _ = acm.stereo_rectify([[c, 0.0, s], [0.0, 1.0, 0.0], [-s, 0.0, c]], [-0.1, 0.01, 0.0])
+with acm.RemapPlan(kb, ds, rotation=R1) as plan:  # rotated plan: map kernel with the rotation, leftover gather for the skewed boxes
+    print("rotated remap", plan.apply(frames).mean(), acm.remap_map(kb, ds, rotation=R2).shape)
 ctx.sync()
 print("ok")
 # round 2: scalar host path (mapped staging + completion flag), small batches, Jacobian kernels (vector and scalar forms)
