@@ -765,29 +765,6 @@ extern "C" int32_t acm_unproject_host(acm_ctx* ctx, const acm_camera* cam, const
     return host_map(ctx, cam, uv_aos, n, xyz_aos, status, false);
 }
 
-extern "C" int32_t acm_undistort_rgb8_host(acm_ctx* ctx, const acm_camera* cam, const double* target_intrinsics, const uint8_t* frames_in,
-                                           uint8_t* frames_out, size_t n_frames, int32_t interpolation) {
-    ACM_ENTER(ctx);
-    ACM_REQUIRE(ctx, cam && (n_frames == 0 || (frames_in && frames_out)), "undistort_host: null argument");
-    if (n_frames == 0) return ACM_OK;
-    size_t fb = (size_t)cam->width * cam->height * 3;
-    uint8_t *d_in = nullptr, *d_out = nullptr;
-    ACM_CUDA(ctx, cudaMalloc(&d_in, fb * n_frames));
-    if (cudaMalloc(&d_out, fb * n_frames) != cudaSuccess) { cudaFree(d_in); return acm_fail(ctx, ACM_ERR_CUDA, "cudaMalloc failed"); }
-    int32_t rc = ACM_OK;
-    cudaError_t e = cudaMemcpyAsync(d_in, frames_in, fb * n_frames, cudaMemcpyHostToDevice, ctx->stream);
-    if (e != cudaSuccess) rc = acm_fail(ctx, ACM_ERR_CUDA, "H2D failed: %s", cudaGetErrorString(e));
-    if (!rc) rc = acm_undistort_rgb8(ctx, cam, target_intrinsics, d_in, d_out, n_frames, interpolation);
-    if (!rc) {
-        e = cudaMemcpyAsync(frames_out, d_out, fb * n_frames, cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-        if (e != cudaSuccess) rc = acm_fail(ctx, ACM_ERR_CUDA, "D2H failed: %s", cudaGetErrorString(e));
-    }
-    cudaStreamSynchronize(ctx->stream);
-    cudaFree(d_in); cudaFree(d_out);
-    return rc;
-}
-
 // ---------------------------------------------------------------------------------------
 // NCCL (loaded at run time so that single-GPU use has no NCCL dependency)
 // ---------------------------------------------------------------------------------------

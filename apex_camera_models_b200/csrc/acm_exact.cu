@@ -11,6 +11,7 @@
 #include <cmath>
 #include <cstring>
 #include <new>
+#include <type_traits>
 
 #include <cuda.h>
 
@@ -486,7 +487,8 @@ __device__ __forceinline__ FixedTap tap_from_coord(double sx, double sy, int st,
 
 // Where the frame kernels get their taps.  W x H is the output grid.
 //  * ModelSrc<M>: undistort_image computes each pixel's source coordinate per launch (the ray through the target pinhole,
-//    then CamModel<M>::project, undistort.rs:33-46); input and output grids are the camera's.
+//    then CamModel<M>::project, undistort.rs:33-46); input and output grids are the camera's.  undistort_map_kernel
+//    writes the same coordinates out.
 //  * PlanSrc: an acm_remap_plan's record (remap_pack_kernel) per pixel on any Wi x Hi input.  The plan's f64 map is read
 //    only where the f64 weights are needed: by the byte kernel and by the rare exact re-blend.
 // coord(): source coordinate and status; tap(): FixedTap; in_w / in_h: the input grid.
@@ -558,6 +560,19 @@ __global__ void __launch_bounds__(256) remap_pack_kernel(const double2* __restri
     rec[i] = make_uint4((uint32_t)(p.t.off00 / 3) | ((uint32_t)p.slow << 30) | ((uint32_t)p.t.ok << 31), p.wlo, p.w01, p.w23);
 }
 
+// nearest: the sample is the pixel itself (undistort.rs:79-90), byte by byte from global memory; returns [R G B 0]
+__device__ __forceinline__ uint32_t nearest_px(const uint8_t* p) { return __ldg(p) | (__ldg(p + 1) << 8) | ((uint32_t)__ldg(p + 2) << 16); }
+
+// the reference's f64 expression for one pixel, p = its p00 in global memory; returns [R G B 0]
+__device__ __forceinline__ uint32_t blend_exact_px(const uint8_t* p, int row_stride, double wx, double wy) {
+    const uint8_t* q = p + row_stride;
+    const double wxi = 1.0 - wx, wyi = 1.0 - wy;
+    const uint32_t r = blend(__ldg(p), __ldg(p + 3), __ldg(q), __ldg(q + 3), wx, wy, wxi, wyi);
+    const uint32_t g = blend(__ldg(p + 1), __ldg(p + 4), __ldg(q + 1), __ldg(q + 4), wx, wy, wxi, wyi);
+    const uint32_t b = blend(__ldg(p + 2), __ldg(p + 5), __ldg(q + 2), __ldg(q + 5), wx, wy, wxi, wyi);
+    return r | (g << 8) | (b << 16);
+}
+
 // Generic byte kernel (any width and alignment): one thread owns 4 horizontally adjacent output pixels: it finds their
 // source coordinates once, then loops over the frames of the batch, gathers the taps through the read-only path, blends
 // with the reference's f64 expression and stages the 12 output bytes in shared memory so that the block writes the row
@@ -585,27 +600,19 @@ __global__ void __launch_bounds__(256) undistort_kernel(const __grid_constant__ 
     const bool vec_ok = ((seg_off & 15) == 0) && ((frame_bytes & 15) == 0) && ((reinterpret_cast<uintptr_t>(out) & 15) == 0);
     for (size_t f = 0; f < n_frames; ++f) {
         const uint8_t* src = in + f * in_frame_bytes;
-        uint8_t o[12];
+        uint32_t px[4];  // [R G B 0] per pixel
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
-            uint8_t r = 0, g = 0, b = 0;
-            if (taps[k].ok) {
-                const uint8_t* p = src + taps[k].off00;
-                if (interp == ACM_INTERP_NEAREST) { r = __ldg(p); g = __ldg(p + 1); b = __ldg(p + 2); }
-                else {
-                    const uint8_t* q = p + row_stride;
-                    double wx = taps[k].wx, wy = taps[k].wy, wxi = 1.0 - wx, wyi = 1.0 - wy;
-                    r = blend(__ldg(p), __ldg(p + 3), __ldg(q), __ldg(q + 3), wx, wy, wxi, wyi);
-                    g = blend(__ldg(p + 1), __ldg(p + 4), __ldg(q + 1), __ldg(q + 4), wx, wy, wxi, wyi);
-                    b = blend(__ldg(p + 2), __ldg(p + 5), __ldg(q + 2), __ldg(q + 5), wx, wy, wxi, wyi);
-                }
-            }
-            o[3 * k] = r; o[3 * k + 1] = g; o[3 * k + 2] = b;
+            const uint8_t* p = src + taps[k].off00;
+            px[k] = !taps[k].ok                     ? 0u
+                    : interp == ACM_INTERP_NEAREST ? nearest_px(p)
+                                                    : blend_exact_px(p, row_stride, taps[k].wx, taps[k].wy);
         }
+        // the 12 bytes of the four pixels as three words
         uint32_t* smw = reinterpret_cast<uint32_t*>(sm) + threadIdx.x * 3;
-        smw[0] = o[0] | (o[1] << 8) | (o[2] << 16) | ((uint32_t)o[3] << 24);
-        smw[1] = o[4] | (o[5] << 8) | (o[6] << 16) | ((uint32_t)o[7] << 24);
-        smw[2] = o[8] | (o[9] << 8) | (o[10] << 16) | ((uint32_t)o[11] << 24);
+        smw[0] = px[0] | (px[1] << 24);
+        smw[1] = (px[1] >> 8) | (px[2] << 16);
+        smw[2] = (px[2] >> 16) | (px[3] << 8);
         __syncthreads();
         uint8_t* dst = out + f * frame_bytes + seg_off;
         if (vec_ok) {
@@ -649,16 +656,6 @@ __device__ __forceinline__ uint32_t tie_bits(const uint32_t tz[4]) {
 
 // nearest: the sample is the pixel itself (undistort.rs:79-90), 3 bytes out of two aligned words
 __device__ __forceinline__ uint32_t pick_nearest(uint32_t a0, uint32_t a1, uint32_t sel) { return __byte_perm(a0, a1, sel) & 0xFFFFFFu; }
-
-// the reference's f64 expression for one pixel, p = its p00 in global memory; returns [R G B 0]
-__device__ __forceinline__ uint32_t blend_exact_px(const uint8_t* p, int row_stride, double wx, double wy) {
-    const uint8_t* q = p + row_stride;
-    const double wxi = 1.0 - wx, wyi = 1.0 - wy;
-    const uint32_t r = blend(__ldg(p), __ldg(p + 3), __ldg(q), __ldg(q + 3), wx, wy, wxi, wyi);
-    const uint32_t g = blend(__ldg(p + 1), __ldg(p + 4), __ldg(q + 1), __ldg(q + 4), wx, wy, wxi, wyi);
-    const uint32_t b = blend(__ldg(p + 2), __ldg(p + 5), __ldg(q + 2), __ldg(q + 5), wx, wy, wxi, wyi);
-    return r | (g << 8) | (b << 16);
-}
 
 // Stores a finished patch: px[k] = [R G B .] of this lane's pixel in row k.  The 96 output bytes of a patch row are
 // exchanged with two shuffles so that lane j < 24 stores word j (bytes of pixels 4j/3 and 4j/3 + 1) at dst + 4j.
@@ -744,8 +741,7 @@ __global__ void __launch_bounds__(256, 3) undistort_gather_kernel(const __grid_c
                         const uint8_t* p = src + tap[k].t.off00;
                         double wx = tap[k].t.wx, wy = tap[k].t.wy;
                         if constexpr (Src::PLAN) { if (!NEAREST) source.exact_w(x0 + lane, y0 + k, W, wx, wy); }
-                        px[k] = NEAREST ? (__ldg(p) | (__ldg(p + 1) << 8) | ((uint32_t)__ldg(p + 2) << 16))
-                                        : blend_exact_px(p, in_stride, wx, wy);
+                        px[k] = NEAREST ? nearest_px(p) : blend_exact_px(p, in_stride, wx, wy);
                     }
                 }
             }
@@ -943,14 +939,13 @@ __global__ void __launch_bounds__(256, 3) undistort_tma_kernel(const __grid_cons
 }
 
 template <int M>
-__global__ void __launch_bounds__(256) undistort_map_kernel(const __grid_constant__ CamParams c, double tfx, double tfy, double tcx,
-                                                            double tcy, double* __restrict__ src_xy, int W, int H) {
-    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+__global__ void __launch_bounds__(256) undistort_map_kernel(const __grid_constant__ ModelSrc<M> source, double* __restrict__ src_xy, int W,
+                                                            int H) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (size_t)W * H) return;
-    int uo = (int)(i % W), vo = (int)(i / W);
-    double xn = ((double)uo - tcx) / tfx, yn = ((double)vo - tcy) / tfy;
+    const int uo = (int)(i % W), vo = (int)(i / W);
     double sx, sy;
-    int st = CamModel<M>::template project<true>(c, xn, yn, 1.0, sx, sy);
+    const int st = source.coord(uo, vo, W, H, sx, sy);
     if (st != ACM_POINT_OK) sx = sy = acm_nan();
     reinterpret_cast<double2*>(src_xy)[i] = make_double2(sx, sy);
 }
@@ -982,59 +977,96 @@ static bool make_frame_tensor_map(CUtensorMap* map, const uint8_t* d_in, int W, 
                   CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-static int32_t check_undistort_args(acm_ctx* ctx, const acm_camera* cam, const double* target, double t[4]) {
-    ACM_REQUIRE(ctx, cam, "undistort: null camera");
-    ACM_REQUIRE(ctx, cam->width > 0 && cam->height > 0, "undistort: camera resolution must be set (image must match model resolution)");
-    ACM_REQUIRE(ctx, (uint64_t)cam->width * cam->height * 3 < 0x7fffffffULL, "undistort: frame larger than 2 GiB is not supported");
-    for (int i = 0; i < 4; ++i) t[i] = target ? target[i] : cam->params[i];
+// A camera whose frames the frame kernels read or write: resolution set, one frame under 2 GiB (the kernels address a frame
+// with int offsets).  `who` names the entry point in the messages, `side` the camera ("input " / "output " / "").  With t
+// given, it receives the target pinhole of undistort_image: `target`, or the camera's own intrinsics.
+static int32_t check_frame_camera(acm_ctx* ctx, const acm_camera* cam, const char* who, const char* side, const double* target = nullptr,
+                                  double* t = nullptr) {
+    if (!cam) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: null %scamera", who, side);
+    if (cam->width == 0 || cam->height == 0)
+        return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: %scamera resolution must be set (frames have the camera's resolution)", who, side);
+    if ((uint64_t)cam->width * cam->height * 3 >= 0x7fffffffULL)
+        return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: %sframe larger than 2 GiB is not supported", who, side);
+    if (t)
+        for (int i = 0; i < 4; ++i) t[i] = target ? target[i] : cam->params[i];
     return ACM_OK;
 }
 
-// maps != nullptr: the TMA kernel, then the gather over the patches it lists (list = d_count + 64);
-// gather: the gather over the whole image; otherwise the generic byte kernel.  W x H: the output grid.
-template <class Src, bool NEAREST>
-static int32_t launch_undistort(acm_ctx* ctx, const Src& source, const UndMaps* maps, bool gather, const uint8_t* d_in, uint8_t* d_out,
-                                int W, int H, size_t n_frames, uint32_t* d_count) {
-    const dim3 patch_grid((W + 63) / 64, (H + 15) / 16);  // block = 64 x 16 output pixels
-    if (maps) {
-        constexpr int smem = 8 * UND_STAGES * UND_FPS * UND_BOX_W * UND_BOX_ROWS + 8 * UND_STAGES * 8 + 2 * 4 * 256 * 8;
-        uint32_t* const d_list = d_count + 64;
-        cudaFuncSetAttribute(undistort_tma_kernel<Src, NEAREST>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-        undistort_tma_kernel<Src, NEAREST><<<patch_grid, 256, smem, ctx->stream>>>(source, *maps, d_in, d_out, W, H, (int)n_frames, d_list,
-                                                                                 d_count);
+// n_frames Wi x Hi input frames -> W x H output frames through the frame kernel the path rule picks (DESIGN 4.3): the TMA
+// kernel, then the gather over the patches whose source box does not fit its tile, when Wi % 16 == 0, W % 4 == 0, the input
+// is 16-byte and the output 4-byte aligned, n_frames < 2^31 and the driver encodes the tensor maps; the gather over the whole
+// image when Wi % 4 == 0, W % 4 == 0 and both buffers are 4-byte aligned; the byte kernel otherwise.
+template <class Src>
+static int32_t launch_frames(acm_ctx* ctx, const Src& source, int Wi, int Hi, int W, int H, const uint8_t* d_in, uint8_t* d_out,
+                             size_t n_frames, int32_t interpolation) {
+    const uintptr_t in_addr = reinterpret_cast<uintptr_t>(d_in), out_addr = reinterpret_cast<uintptr_t>(d_out);
+    if (Wi % 4 != 0 || W % 4 != 0 || (in_addr & 3) != 0 || (out_addr & 3) != 0) {
+        undistort_kernel<Src><<<dim3((W + 1023) / 1024, H), 256, 0, ctx->stream>>>(source, d_in, d_out, W, H, n_frames, interpolation);
         ACM_CHECK_LAUNCH(ctx);
-        undistort_gather_kernel<Src, NEAREST><<<ctx->sm_count * 3, 256, 0, ctx->stream>>>(source, d_in, d_out, W, H, n_frames, d_list, d_count);
-    } else if (gather) {
-        undistort_gather_kernel<Src, NEAREST><<<patch_grid, 256, 0, ctx->stream>>>(source, d_in, d_out, W, H, n_frames, nullptr, nullptr);
-    } else {
-        undistort_kernel<Src><<<dim3((W + 1023) / 1024, H), 256, 0, ctx->stream>>>(source, d_in, d_out, W, H, n_frames,
-                                                                                  NEAREST ? ACM_INTERP_NEAREST : ACM_INTERP_BILINEAR);
+        return ACM_OK;
     }
-    ACM_CHECK_LAUNCH(ctx);
-    return ACM_OK;
+    UndMaps maps;
+    bool tma = Wi % 16 == 0 && (in_addr & 15) == 0 && n_frames < 0x7fffffffULL;
+    for (int r = UND_MIN_ROWS; tma && r <= UND_BOX_ROWS; ++r) tma = make_frame_tensor_map(&maps.m[r - UND_MIN_ROWS], d_in, Wi, Hi, n_frames, r);
+    // the TMA kernel's leftover list in the context's scratch: [count] at d_count, patch ids (one per 32 x 4 output patch
+    // at most) from d_count + 64
+    uint32_t* d_count = nullptr;
+    if (tma) {
+        const size_t n_patches = (size_t)((W + 31) / 32) * (size_t)((H + 3) / 4);
+        const int32_t rc = acm_ensure_scratch(ctx, 256 + n_patches * sizeof(uint32_t));
+        if (rc) return rc;
+        d_count = static_cast<uint32_t*>(ctx->d_scratch);
+        ACM_CUDA(ctx, cudaMemsetAsync(d_count, 0, sizeof(uint32_t), ctx->stream));
+    }
+    const dim3 patch_grid((W + 63) / 64, (H + 15) / 16);  // block = 64 x 16 output pixels
+    const auto launch = [&](auto nearest) -> int32_t {
+        constexpr bool NEAREST = decltype(nearest)::value;
+        if (tma) {
+            constexpr int smem = 8 * UND_STAGES * UND_FPS * UND_BOX_W * UND_BOX_ROWS + 8 * UND_STAGES * 8 + 2 * 4 * 256 * 8;
+            uint32_t* const d_list = d_count + 64;
+            cudaFuncSetAttribute(undistort_tma_kernel<Src, NEAREST>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+            undistort_tma_kernel<Src, NEAREST><<<patch_grid, 256, smem, ctx->stream>>>(source, maps, d_in, d_out, W, H, (int)n_frames, d_list,
+                                                                                     d_count);
+            ACM_CHECK_LAUNCH(ctx);
+            undistort_gather_kernel<Src, NEAREST><<<ctx->sm_count * 3, 256, 0, ctx->stream>>>(source, d_in, d_out, W, H, n_frames, d_list,
+                                                                                              d_count);
+        } else {
+            undistort_gather_kernel<Src, NEAREST><<<patch_grid, 256, 0, ctx->stream>>>(source, d_in, d_out, W, H, n_frames, nullptr, nullptr);
+        }
+        ACM_CHECK_LAUNCH(ctx);
+        return ACM_OK;
+    };
+    return interpolation == ACM_INTERP_NEAREST ? launch(std::true_type{}) : launch(std::false_type{});
 }
 
-// Tensor maps of the TMA path over a Wi x Hi input batch, and the leftover list ([count][patch ids], one id per 32 x 4
-// patch of the W x H output at most) in the context's scratch.  *tma (in: the path rule allows TMA) turns false when the
-// driver refuses a tensor map: the caller then gathers.
-static int32_t prepare_tma(acm_ctx* ctx, UndMaps* maps, const uint8_t* d_in, int Wi, int Hi, int W, int H, size_t n_frames, bool* tma,
-                           uint32_t** d_count) {
-    *d_count = nullptr;
-    for (int r = UND_MIN_ROWS; *tma && r <= UND_BOX_ROWS; ++r) *tma = make_frame_tensor_map(&maps->m[r - UND_MIN_ROWS], d_in, Wi, Hi, n_frames, r);
-    if (!*tma) return ACM_OK;
-    const size_t n_patches = (size_t)((W + 31) / 32) * (size_t)((H + 3) / 4);
-    int32_t rc = acm_ensure_scratch(ctx, 256 + n_patches * sizeof(uint32_t));
-    if (rc) return rc;
-    *d_count = static_cast<uint32_t*>(ctx->d_scratch);
-    ACM_CUDA(ctx, cudaMemsetAsync(*d_count, 0, sizeof(uint32_t), ctx->stream));
-    return ACM_OK;
+// Host frames through the device: a device copy of both batches, in_bytes up, run(d_in, d_out) on the context's stream,
+// out_bytes down, synchronise, free.
+template <class Run>
+static int32_t frames_through_device(acm_ctx* ctx, const uint8_t* frames_in, size_t in_bytes, uint8_t* frames_out, size_t out_bytes, Run run) {
+    uint8_t *d_in = nullptr, *d_out = nullptr;
+    int32_t rc = acm_device_malloc(ctx, reinterpret_cast<void**>(&d_in), in_bytes);
+    if (!rc) rc = acm_device_malloc(ctx, reinterpret_cast<void**>(&d_out), out_bytes);
+    if (!rc) {
+        const cudaError_t e = cudaMemcpyAsync(d_in, frames_in, in_bytes, cudaMemcpyHostToDevice, ctx->stream);
+        if (e != cudaSuccess) rc = acm_fail(ctx, ACM_ERR_CUDA, "H2D failed: %s", cudaGetErrorString(e));
+    }
+    if (!rc) rc = run(d_in, d_out);
+    if (!rc) {
+        cudaError_t e = cudaMemcpyAsync(frames_out, d_out, out_bytes, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+        if (e != cudaSuccess) rc = acm_fail(ctx, ACM_ERR_CUDA, "D2H failed: %s", cudaGetErrorString(e));
+    }
+    cudaStreamSynchronize(ctx->stream);
+    if (d_in) cudaFree(d_in);
+    if (d_out) cudaFree(d_out);
+    return rc;
 }
 
 extern "C" int32_t acm_undistort_rgb8(acm_ctx* ctx, const acm_camera* cam, const double* target_intrinsics, const uint8_t* d_in,
                                       uint8_t* d_out, size_t n_frames, int32_t interpolation) {
     ACM_ENTER(ctx);
     double t[4];
-    int32_t rc = check_undistort_args(ctx, cam, target_intrinsics, t);
+    int32_t rc = check_frame_camera(ctx, cam, "undistort", "", target_intrinsics, t);
     if (rc) return rc;
     ACM_REQUIRE(ctx, d_in && d_out, "undistort: null frame buffer");
     ACM_REQUIRE(ctx, interpolation == ACM_INTERP_NEAREST || interpolation == ACM_INTERP_BILINEAR, "undistort: unknown interpolation");
@@ -1043,25 +1075,26 @@ extern "C" int32_t acm_undistort_rgb8(acm_ctx* ctx, const acm_camera* cam, const
     rc = acm_make_cam_params(ctx, cam, &c);
     if (rc) return rc;
     const int W = (int)cam->width, H = (int)cam->height;
-    const uintptr_t in_addr = reinterpret_cast<uintptr_t>(d_in), out_addr = reinterpret_cast<uintptr_t>(d_out);
-    const bool gather = W % 4 == 0 && (in_addr & 3) == 0 && (out_addr & 3) == 0;
-    UndMaps maps;
-    bool tma = gather && W % 16 == 0 && (in_addr & 15) == 0 && n_frames < 0x7fffffffULL;
-    uint32_t* d_count;
-    rc = prepare_tma(ctx, &maps, d_in, W, H, W, H, n_frames, &tma, &d_count);
-    if (rc) return rc;
-    const UndMaps* const tma_maps = tma ? &maps : nullptr;
-    ACM_DISPATCH_MODEL(cam->model, {
-        const ModelSrc<M> source{c, t[0], t[1], t[2], t[3]};
-        return interpolation == ACM_INTERP_NEAREST ? launch_undistort<ModelSrc<M>, true>(ctx, source, tma_maps, gather, d_in, d_out, W, H, n_frames, d_count)
-                                                   : launch_undistort<ModelSrc<M>, false>(ctx, source, tma_maps, gather, d_in, d_out, W, H, n_frames, d_count);
-    })
+    ACM_DISPATCH_MODEL(cam->model, return launch_frames(ctx, ModelSrc<M>{c, t[0], t[1], t[2], t[3]}, W, H, W, H, d_in, d_out, n_frames, interpolation))
     return ACM_OK;
+}
+
+extern "C" int32_t acm_undistort_rgb8_host(acm_ctx* ctx, const acm_camera* cam, const double* target_intrinsics, const uint8_t* frames_in,
+                                           uint8_t* frames_out, size_t n_frames, int32_t interpolation) {
+    ACM_ENTER(ctx);
+    const int32_t rc = check_frame_camera(ctx, cam, "undistort_host", "");
+    if (rc) return rc;
+    ACM_REQUIRE(ctx, n_frames == 0 || (frames_in && frames_out), "undistort_host: null frame buffer");
+    if (n_frames == 0) return ACM_OK;
+    const size_t bytes = (size_t)cam->width * cam->height * 3 * n_frames;
+    return frames_through_device(ctx, frames_in, bytes, frames_out, bytes, [&](const uint8_t* d_in, uint8_t* d_out) {
+        return acm_undistort_rgb8(ctx, cam, target_intrinsics, d_in, d_out, n_frames, interpolation);
+    });
 }
 
 static int32_t launch_undistort_map(acm_ctx* ctx, const CamParams& c, const double* t, double* d_src_xy, int W, int H) {
     const int grid = (int)(((size_t)W * H + 255) / 256);
-    ACM_DISPATCH_MODEL(c.model, (undistort_map_kernel<M><<<grid, 256, 0, ctx->stream>>>(c, t[0], t[1], t[2], t[3], d_src_xy, W, H)))
+    ACM_DISPATCH_MODEL(c.model, (undistort_map_kernel<M><<<grid, 256, 0, ctx->stream>>>(ModelSrc<M>{c, t[0], t[1], t[2], t[3]}, d_src_xy, W, H)))
     ACM_CHECK_LAUNCH(ctx);
     return ACM_OK;
 }
@@ -1069,7 +1102,7 @@ static int32_t launch_undistort_map(acm_ctx* ctx, const CamParams& c, const doub
 extern "C" int32_t acm_undistort_map(acm_ctx* ctx, const acm_camera* cam, const double* target_intrinsics, double* d_src_xy) {
     ACM_ENTER(ctx);
     double t[4];
-    int32_t rc = check_undistort_args(ctx, cam, target_intrinsics, t);
+    int32_t rc = check_frame_camera(ctx, cam, "undistort", "", target_intrinsics, t);
     if (rc) return rc;
     ACM_REQUIRE(ctx, d_src_xy, "undistort_map: null output");
     CamParams c;
@@ -1122,15 +1155,6 @@ static int32_t launch_remap_map(acm_ctx* ctx, const CamParams& ci, const CamPara
     return ACM_OK;
 }
 
-static int32_t check_frame_camera(acm_ctx* ctx, const acm_camera* cam, const char* side) {
-    if (!cam) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "remap: null %s camera", side);
-    if (cam->width == 0 || cam->height == 0)
-        return acm_fail(ctx, ACM_ERR_INVALID_ARG, "remap: %s camera resolution must be set (frames have the camera's resolution)", side);
-    if ((uint64_t)cam->width * cam->height * 3 >= 0x7fffffffULL)
-        return acm_fail(ctx, ACM_ERR_INVALID_ARG, "remap: %s frame larger than 2 GiB is not supported", side);
-    return ACM_OK;
-}
-
 // R must be a proper rotation: finite entries, max |R R^T - I| <= 1e-9, det R > 0.  ctx may be null (acm_stereo_rectify).
 static int32_t check_rotation(acm_ctx* ctx, const double* R, const char* who) {
     if (!R) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: null rotation", who);
@@ -1163,8 +1187,8 @@ static int32_t remap_map(acm_ctx* ctx, const acm_camera* input_cam, const acm_ca
 }
 
 static int32_t remap_map_entry(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam, const double* R, double* d_src_xy) {
-    int32_t rc = check_frame_camera(ctx, input_cam, "input");
-    if (!rc) rc = check_frame_camera(ctx, output_cam, "output");
+    int32_t rc = check_frame_camera(ctx, input_cam, "remap", "input ");
+    if (!rc) rc = check_frame_camera(ctx, output_cam, "remap", "output ");
     if (rc) return rc;
     ACM_REQUIRE(ctx, d_src_xy, "remap_map: null output");
     return remap_map(ctx, input_cam, output_cam, R, d_src_xy);
@@ -1212,8 +1236,9 @@ static void free_plan(acm_remap_plan* p) {
 static int32_t create_plan(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam, const double* target_intrinsics,
                            const double* R, int32_t interpolation, acm_remap_plan** out) {
     ACM_REQUIRE(ctx, !(output_cam && target_intrinsics), "remap_plan: give either an output camera or target intrinsics, not both");
-    int32_t rc = check_frame_camera(ctx, input_cam, "input");
-    if (!rc && output_cam) rc = check_frame_camera(ctx, output_cam, "output");
+    double t[4];
+    int32_t rc = check_frame_camera(ctx, input_cam, "remap", "input ", target_intrinsics, t);
+    if (!rc && output_cam) rc = check_frame_camera(ctx, output_cam, "remap", "output ");
     if (rc) return rc;
     ACM_REQUIRE(ctx, interpolation == ACM_INTERP_NEAREST || interpolation == ACM_INTERP_BILINEAR, "remap_plan: unknown interpolation");
     CamParams ci;
@@ -1230,8 +1255,6 @@ static int32_t create_plan(acm_ctx* ctx, const acm_camera* input_cam, const acm_
     if (!rc && output_cam) {
         rc = remap_map(ctx, input_cam, output_cam, R, reinterpret_cast<double*>(p->d_map));
     } else if (!rc) {  // undistort_image semantics: the map of acm_undistort_map
-        double t[4];
-        for (int i = 0; i < 4; ++i) t[i] = target_intrinsics ? target_intrinsics[i] : input_cam->params[i];
         rc = launch_undistort_map(ctx, ci, t, reinterpret_cast<double*>(p->d_map), p->Wo, p->Ho);
     }
     if (!rc) rc = launch_remap_pack(ctx, p);
@@ -1272,28 +1295,14 @@ extern "C" int32_t acm_remap_plan_destroy(acm_ctx* ctx, acm_remap_plan* plan) {
     return ACM_OK;
 }
 
-// Path rule: TMA + leftover gather when Wi % 16 == 0, the input is 16-byte and the output 4-byte aligned, Wo % 4 == 0 and the
-// tensor maps encode; the whole-image gather when Wi % 4 == 0, Wo % 4 == 0 and both buffers are 4-byte aligned; the byte
-// kernel otherwise.
 extern "C" int32_t acm_remap_rgb8(acm_ctx* ctx, const acm_remap_plan* plan, const uint8_t* d_in, uint8_t* d_out, size_t n_frames) {
     ACM_ENTER(ctx);
     ACM_REQUIRE(ctx, plan, "remap: null plan");
     ACM_REQUIRE(ctx, plan->ctx == ctx, "remap: the plan belongs to another context");
     ACM_REQUIRE(ctx, d_in && d_out, "remap: null frame buffer");
     if (n_frames == 0) return ACM_OK;
-    const int Wi = plan->Wi, Hi = plan->Hi, W = plan->Wo, H = plan->Ho;
-    const uintptr_t in_addr = reinterpret_cast<uintptr_t>(d_in), out_addr = reinterpret_cast<uintptr_t>(d_out);
-    const bool gather = Wi % 4 == 0 && W % 4 == 0 && (in_addr & 3) == 0 && (out_addr & 3) == 0;
-    UndMaps maps;
-    bool tma = gather && Wi % 16 == 0 && (in_addr & 15) == 0 && n_frames < 0x7fffffffULL;
-    uint32_t* d_count;
-    int32_t rc = prepare_tma(ctx, &maps, d_in, Wi, Hi, W, H, n_frames, &tma, &d_count);
-    if (rc) return rc;
-    const PlanSrc source{plan->d_rec, plan->d_map, Wi, Hi};
-    const UndMaps* const tma_maps = tma ? &maps : nullptr;
-    return plan->interpolation == ACM_INTERP_NEAREST
-               ? launch_undistort<PlanSrc, true>(ctx, source, tma_maps, gather, d_in, d_out, W, H, n_frames, d_count)
-               : launch_undistort<PlanSrc, false>(ctx, source, tma_maps, gather, d_in, d_out, W, H, n_frames, d_count);
+    return launch_frames(ctx, PlanSrc{plan->d_rec, plan->d_map, plan->Wi, plan->Hi}, plan->Wi, plan->Hi, plan->Wo, plan->Ho, d_in, d_out,
+                         n_frames, plan->interpolation);
 }
 
 extern "C" int32_t acm_remap_rgb8_host(acm_ctx* ctx, const acm_remap_plan* plan, const uint8_t* frames_in, uint8_t* frames_out,
@@ -1303,24 +1312,8 @@ extern "C" int32_t acm_remap_rgb8_host(acm_ctx* ctx, const acm_remap_plan* plan,
     ACM_REQUIRE(ctx, plan->ctx == ctx, "remap_host: the plan belongs to another context");
     ACM_REQUIRE(ctx, n_frames == 0 || (frames_in && frames_out), "remap_host: null frame buffer");
     if (n_frames == 0) return ACM_OK;
-    const size_t in_bytes = (size_t)plan->Wi * plan->Hi * 3 * n_frames, out_bytes = (size_t)plan->Wo * plan->Ho * 3 * n_frames;
-    uint8_t *d_in = nullptr, *d_out = nullptr;
-    int32_t rc = acm_device_malloc(ctx, reinterpret_cast<void**>(&d_in), in_bytes);
-    if (!rc) rc = acm_device_malloc(ctx, reinterpret_cast<void**>(&d_out), out_bytes);
-    if (!rc) {
-        const cudaError_t e = cudaMemcpyAsync(d_in, frames_in, in_bytes, cudaMemcpyHostToDevice, ctx->stream);
-        if (e != cudaSuccess) rc = acm_fail(ctx, ACM_ERR_CUDA, "H2D failed: %s", cudaGetErrorString(e));
-    }
-    if (!rc) rc = acm_remap_rgb8(ctx, plan, d_in, d_out, n_frames);
-    if (!rc) {
-        cudaError_t e = cudaMemcpyAsync(frames_out, d_out, out_bytes, cudaMemcpyDeviceToHost, ctx->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-        if (e != cudaSuccess) rc = acm_fail(ctx, ACM_ERR_CUDA, "D2H failed: %s", cudaGetErrorString(e));
-    }
-    cudaStreamSynchronize(ctx->stream);
-    if (d_in) cudaFree(d_in);
-    if (d_out) cudaFree(d_out);
-    return rc;
+    return frames_through_device(ctx, frames_in, (size_t)plan->Wi * plan->Hi * 3 * n_frames, frames_out, (size_t)plan->Wo * plan->Ho * 3 * n_frames,
+                                 [&](const uint8_t* d_in, uint8_t* d_out) { return acm_remap_rgb8(ctx, plan, d_in, d_out, n_frames); });
 }
 
 // ---------------------------------------------------------------------------------------

@@ -18,17 +18,9 @@ import sys
 
 import numpy as np
 
+from ._image_cli import expand_inputs, load_model, load_rgb, save_rgb
 from .camera import Intrinsics, PinholeModel, Resolution
-from .image_remap import _load_model
-from .image_undistort import _load_rgb, _save_rgb
 from .util import InterpolationMethod, StereoRectifier
-
-
-def _expand(paths):
-    out = []
-    for p in paths:
-        out += sorted(os.path.join(p, f) for f in os.listdir(p)) if os.path.isdir(p) else [p]
-    return out
 
 
 def main(argv=None) -> int:
@@ -49,22 +41,22 @@ def main(argv=None) -> int:
     ap.add_argument("--right-output", required=True, help="output directory of the rectified right images")
     args = ap.parse_args(argv)
 
-    left, right = _load_model(args.left_model, args.left_calib), _load_model(args.right_model, args.right_calib)
+    left, right = load_model(args.left_model, args.left_calib), load_model(args.right_model, args.right_calib)
     W, H = args.size
     cx, cy = args.principal if args.principal else ((W - 1) / 2.0, (H - 1) / 2.0)
     rect = PinholeModel(Intrinsics(args.focal, args.focal, cx, cy), Resolution(W, H), ctx=left.ctx)
-    left_paths, right_paths = _expand(args.left), _expand(args.right)
+    left_paths, right_paths = expand_inputs(args.left), expand_inputs(args.right)
     if len(left_paths) != len(right_paths):
         raise SystemExit(f"need as many right images as left images ({len(right_paths)} != {len(left_paths)})")
     interp = InterpolationMethod.Nearest if args.interpolation == "nearest" else InterpolationMethod.Bilinear
     with StereoRectifier(left, right, np.reshape(args.rotation, (3, 3)), args.translation, rect, interp) as rig:
         print(f"Rectifying {len(left_paths)} pair(s) onto a {W}x{H} pinhole (f={args.focal}, c=({cx}, {cy})): "
               f"baseline {rig.baseline:.6g} along {'y' if rig.vertical else 'x'}")
-        out_l, out_r = rig.apply(np.stack([_load_rgb(p) for p in left_paths]), np.stack([_load_rgb(p) for p in right_paths]))
+        out_l, out_r = rig.apply(np.stack([load_rgb(p) for p in left_paths]), np.stack([load_rgb(p) for p in right_paths]))
     for d, paths, frames in ((args.left_output, left_paths, out_l), (args.right_output, right_paths, out_r)):
         os.makedirs(d, exist_ok=True)
         for p, a in zip(paths, frames):
-            _save_rgb(os.path.join(d, os.path.basename(p)), a)
+            save_rgb(os.path.join(d, os.path.basename(p)), a)
     print(f"Saved rectified images to: {args.left_output}, {args.right_output}")
     return 0
 

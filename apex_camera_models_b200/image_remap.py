@@ -10,21 +10,12 @@ Several inputs may be given (repeat `-i` / `-o`, or pass directories); they are 
 from __future__ import annotations
 
 import argparse
-import os
 import sys
 
 import numpy as np
 
-from .camera_converter import INPUT_ALIASES
-from .image_undistort import _load_rgb, _save_rgb
+from ._image_cli import expand_inputs, load_model, load_rgb, pair_outputs, save_rgb
 from .util import InterpolationMethod, RemapPlan
-
-
-def _load_model(kind: str, calib: str):
-    cls = INPUT_ALIASES.get(kind.lower())
-    if cls is None:
-        raise SystemExit(f"Unsupported model: {kind}")
-    return cls.load_from_yaml(calib)
 
 
 def main(argv=None) -> int:
@@ -38,27 +29,19 @@ def main(argv=None) -> int:
     ap.add_argument("--interpolation", choices=["bilinear", "nearest"], default="bilinear")
     args = ap.parse_args(argv)
 
-    src, dst = _load_model(args.model, args.calib), _load_model(args.output_model, args.output_calib)
+    src, dst = load_model(args.model, args.calib), load_model(args.output_model, args.output_calib)
     ri, ro = src.get_resolution(), dst.get_resolution()
     print(f"Remapping {args.model} {ri.width}x{ri.height} -> {args.output_model} {ro.width}x{ro.height} ({args.interpolation})")
 
-    inputs = []
-    for p in args.input:
-        inputs += sorted(os.path.join(p, f) for f in os.listdir(p)) if os.path.isdir(p) else [p]
-    if len(args.output) == 1 and (os.path.isdir(args.output[0]) or len(inputs) > 1):
-        os.makedirs(args.output[0], exist_ok=True)
-        outputs = [os.path.join(args.output[0], os.path.basename(p)) for p in inputs]
-    else:
-        outputs = args.output
-    if len(outputs) != len(inputs):
-        raise SystemExit("need one output per input (or one output directory)")
+    inputs = expand_inputs(args.input)
+    outputs = pair_outputs(inputs, args.output)
 
-    frames = np.stack([_load_rgb(p) for p in inputs])
+    frames = np.stack([load_rgb(p) for p in inputs])
     interp = InterpolationMethod.Nearest if args.interpolation == "nearest" else InterpolationMethod.Bilinear
     with RemapPlan(src, dst, None, interp) as plan:
         out = plan.apply(frames)
     for p, a in zip(outputs, out):
-        _save_rgb(p, a)
+        save_rgb(p, a)
         print(f"Saved remapped image to: {p}")
     return 0
 

@@ -8,29 +8,13 @@ pass directories): they are undistorted as ONE batch, which is what the GPU kern
 from __future__ import annotations
 
 import argparse
-import os
 import sys
 
 import numpy as np
 
+from ._image_cli import expand_inputs, load_model, load_rgb, pair_outputs, save_rgb
 from .camera import Intrinsics
-from .camera_converter import INPUT_ALIASES
 from .util import InterpolationMethod, undistort_images
-
-
-def _load_rgb(path: str) -> np.ndarray:
-    if path.endswith(".npy"):
-        return np.ascontiguousarray(np.load(path), dtype=np.uint8)
-    from PIL import Image  # image decoding is host-side glue, like the `image` crate in the reference
-    return np.asarray(Image.open(path).convert("RGB"), dtype=np.uint8)
-
-
-def _save_rgb(path: str, a: np.ndarray) -> None:
-    if path.endswith(".npy"):
-        np.save(path, a)
-        return
-    from PIL import Image
-    Image.fromarray(a, "RGB").save(path)
 
 
 def main(argv=None) -> int:
@@ -44,26 +28,15 @@ def main(argv=None) -> int:
     ap.add_argument("--nearest", action="store_true", help="nearest-neighbour instead of the reference's bilinear sampling")
     args = ap.parse_args(argv)
 
-    cls = INPUT_ALIASES.get(args.model.lower())
-    if cls is None:
-        raise SystemExit(f"Unsupported model: {args.model}")
-    model = cls.load_from_yaml(args.calib)
+    model = load_model(args.model, args.calib)
     intr, res = model.get_intrinsics(), model.get_resolution()
     print("Image Undistortion Tool (B200 path)")
     print(f"Loaded {args.model} camera model: fx={intr.fx:.2f}, fy={intr.fy:.2f}, cx={intr.cx:.2f}, cy={intr.cy:.2f}, resolution {res.width}x{res.height}")
 
-    inputs = []
-    for p in args.input:
-        inputs += sorted(os.path.join(p, f) for f in os.listdir(p)) if os.path.isdir(p) else [p]
-    if len(args.output) == 1 and (os.path.isdir(args.output[0]) or len(inputs) > 1):
-        os.makedirs(args.output[0], exist_ok=True)
-        outputs = [os.path.join(args.output[0], os.path.basename(p)) for p in inputs]
-    else:
-        outputs = args.output
-    if len(outputs) != len(inputs):
-        raise SystemExit("need one output per input (or one output directory)")
+    inputs = expand_inputs(args.input)
+    outputs = pair_outputs(inputs, args.output)
 
-    frames = np.stack([_load_rgb(p) for p in inputs])
+    frames = np.stack([load_rgb(p) for p in inputs])
     print(f"Loaded {len(inputs)} input image(s): {frames.shape[2]}x{frames.shape[1]}")
     target = None
     if args.target_fx is not None or args.target_fy is not None:  # image_undistort.rs:78-91
@@ -72,7 +45,7 @@ def main(argv=None) -> int:
         print(f"Using custom target focal lengths: fx={target.fx:.2f}, fy={target.fy:.2f}")
     out = undistort_images(frames, model, target, InterpolationMethod.Nearest if args.nearest else InterpolationMethod.Bilinear)
     for p, a in zip(outputs, out):
-        _save_rgb(p, a)
+        save_rgb(p, a)
         print(f"Saved undistorted image to: {p}")
     return 0
 

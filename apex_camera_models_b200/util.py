@@ -52,21 +52,41 @@ def _rotation_array(rotation):
     return (C.c_double * 9)(*_matrix3(rotation, "rotation").ravel())
 
 
-def undistort_images(frames: np.ndarray, camera_model: CameraModel, target_intrinsics: Intrinsics | None = None,
-                     interpolation: InterpolationMethod = InterpolationMethod.Bilinear) -> np.ndarray:
-    """Batch form: frames (F, H, W, 3) uint8 -> same shape."""
+def _check_frames(frames: np.ndarray, camera_model: CameraModel) -> np.ndarray:
+    """(F, H, W, 3) uint8 frames at the camera's resolution, as undistort.rs:23-28 requires."""
     frames = np.ascontiguousarray(frames, dtype=np.uint8)
     if frames.ndim != 4 or frames.shape[3] != 3:
         raise UtilError("Invalid parameters: expected (F, H, W, 3) uint8 frames")
     res = camera_model.get_resolution()
-    F, H, W, _ = frames.shape
-    if W != res.width or H != res.height:  # undistort.rs:23-28
+    _, H, W, _ = frames.shape
+    if W != res.width or H != res.height:
         raise UtilError(f"Invalid parameters: Image {W}x{H} doesn't match model {res.width}x{res.height}")
+    return frames
+
+
+def _download_map(ctx, res, call) -> np.ndarray:
+    """(H, W, 2) source-coordinate map at resolution `res`: `call(device_ptr)` writes it on the device and returns libacm's
+    status; the device buffer is freed whatever happens."""
+    d = ctx.device_alloc(max(res.width * res.height, 1) * 16)
+    try:
+        ctx.check(call(C.c_void_p(d)))
+        out = np.empty((res.height, res.width, 2))
+        ctx.d2h(out, d)
+        ctx.sync()
+    finally:
+        ctx.device_free(d)
+    return out
+
+
+def undistort_images(frames: np.ndarray, camera_model: CameraModel, target_intrinsics: Intrinsics | None = None,
+                     interpolation: InterpolationMethod = InterpolationMethod.Bilinear) -> np.ndarray:
+    """Batch form: frames (F, H, W, 3) uint8 -> same shape."""
+    frames = _check_frames(frames, camera_model)
     ctx = camera_model.ctx
     cam = camera_model.camera_block()
     out = np.empty_like(frames)
     ctx.check(_lib.acm_undistort_rgb8_host(ctx.handle, C.byref(cam), _target_array(target_intrinsics), frames.ctypes.data_as(C.c_void_p),
-                                           out.ctypes.data_as(C.c_void_p), F, int(interpolation)))
+                                           out.ctypes.data_as(C.c_void_p), frames.shape[0], int(interpolation)))
     return out
 
 
@@ -82,27 +102,8 @@ def undistort_map(camera_model: CameraModel, target_intrinsics: Intrinsics | Non
     """(H, W, 2) source coordinates of every output pixel (NaN where the projection fails)."""
     ctx = camera_model.ctx
     cam = camera_model.camera_block()
-    res = camera_model.get_resolution()
-    n = res.width * res.height
-    d = ctx.device_alloc(max(n, 1) * 16)
-    ctx.check(_lib.acm_undistort_map(ctx.handle, C.byref(cam), _target_array(target_intrinsics), C.c_void_p(d)))
-    out = np.empty((res.height, res.width, 2))
-    ctx.d2h(out, d)
-    ctx.sync()
-    ctx.device_free(d)
-    return out
-
-
-def _check_frames(frames: np.ndarray, camera_model: CameraModel) -> np.ndarray:
-    """(F, H, W, 3) uint8 frames at the camera's resolution, as undistort.rs:23-28 requires."""
-    frames = np.ascontiguousarray(frames, dtype=np.uint8)
-    if frames.ndim != 4 or frames.shape[3] != 3:
-        raise UtilError("Invalid parameters: expected (F, H, W, 3) uint8 frames")
-    res = camera_model.get_resolution()
-    _, H, W, _ = frames.shape
-    if W != res.width or H != res.height:
-        raise UtilError(f"Invalid parameters: Image {W}x{H} doesn't match model {res.width}x{res.height}")
-    return frames
+    target = _target_array(target_intrinsics)
+    return _download_map(ctx, camera_model.get_resolution(), lambda d: _lib.acm_undistort_map(ctx.handle, C.byref(cam), target, d))
 
 
 class RemapPlan:
@@ -192,19 +193,12 @@ def remap_map(input_model: CameraModel, output_model: CameraModel, rotation=None
     `RemapPlan`."""
     ctx = input_model.ctx
     cin, cout = input_model.camera_block(), output_model.camera_block()
-    res = output_model.get_resolution()
-    d = ctx.device_alloc(max(res.width * res.height, 1) * 16)
-    try:
-        if rotation is not None:
-            ctx.check(_lib.acm_remap_map_rotated(ctx.handle, C.byref(cin), C.byref(cout), _rotation_array(rotation), C.c_void_p(d)))
-        else:
-            ctx.check(_lib.acm_remap_map(ctx.handle, C.byref(cin), C.byref(cout), C.c_void_p(d)))
-        out = np.empty((res.height, res.width, 2))
-        ctx.d2h(out, d)
-        ctx.sync()
-    finally:
-        ctx.device_free(d)
-    return out
+    if rotation is not None:
+        R = _rotation_array(rotation)
+        call = lambda d: _lib.acm_remap_map_rotated(ctx.handle, C.byref(cin), C.byref(cout), R, d)
+    else:
+        call = lambda d: _lib.acm_remap_map(ctx.handle, C.byref(cin), C.byref(cout), d)
+    return _download_map(ctx, output_model.get_resolution(), call)
 
 
 def stereo_rectify(R, t):

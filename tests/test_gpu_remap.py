@@ -228,6 +228,12 @@ def test_remap_argument_errors(acm, ctx, O, cameras):
             d = ctx.device_alloc(16)
             fails(L.acm_remap_map(ctx.handle, *args, C.c_void_p(d)), text)
             ctx.device_free(d)
+    # the undistort host entry checks its camera as plan creation does, before it allocates
+    b = N.Camera.from_buffer_copy(bi)
+    b.width = 0
+    frame = np.zeros((48, 64, 3), np.uint8)
+    fails(L.acm_undistort_rgb8_host(ctx.handle, C.byref(b), None, frame.ctypes.data_as(C.c_void_p), frame.ctypes.data_as(C.c_void_p), 1, 1),
+          "resolution must be set")
     fails(L.acm_remap_plan_create(ctx.handle, C.byref(bi), C.byref(bo), None, 2, C.byref(h)), "unknown interpolation")
     fails(L.acm_remap_map(ctx.handle, C.byref(bi), C.byref(bo), None), "null output")
     with acm.RemapPlan(gi, go) as plan:
