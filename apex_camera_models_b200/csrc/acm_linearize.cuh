@@ -14,6 +14,7 @@
 //   HFD[2][ND]  H[f*,d_k]               HCD[2][ND]  H[c*,d_k]           HDD[ND(ND+1)/2]
 //   GF[2] GC[2] GD[ND]   COST   COUNT
 #pragma once
+#include <type_traits>
 #include "acm_internal.cuh"
 #include "acm_math.cuh"
 
@@ -538,3 +539,124 @@ template <> struct LinOps<ACM_MODEL_RADTAN, ACM_RESIDUAL_PIXEL> {
         *count = cnt;
     }
 };
+
+// ---------------------------------------------------------------------------------------
+// Double Sphere, pixel residual (the headline kernel): 68 FP64 instructions per point instead of the generic 77.
+//
+// Precision budget.  The residual needs full precision: near the minimiser ru, rv are ~0.01 px, and an error of 2^-46 in
+// 1/den or d1 moves fx*mx by ~1e-11 px, a cost error of ~1e-9 relative.  So:
+//   * everything that feeds ru, rv or the validity tests stays within a few ulp: d1 and d2 (<= 1 ulp, a Heron step with
+//     the exact fma residual), g (one fma, as before), den, 1/den (<= 1 ulp), mx and my (one product each);
+//   * quantities that only feed Jacobian columns may carry ~2^-44 relative error: h ~ 1/(2 d2) (one Goldschmidt step, the
+//     same order as the one Newton step of the generic form's 1/d2), hence dd1, cu and cv;
+//   * dd0 = d2 - g keeps its form (the oracle computes it so, and it cancels for points near the axis).
+// Where the instructions went (generic form -> this one, per point):
+//   * d1 = sqrt(x^2 + y^2 + z^2): 8 -> 5.  Seed s ~ 1/sqrt(a), h0 = s/2 by an exponent decrement (an integer add, off the
+//     FP64 pipe; s is normal, or inf / 0 / NaN for a degenerate point, whose g0 = a s is then NaN as before), one coupled
+//     Goldschmidt step on g ~ sqrt(a) only, then Heron with h0: its error is ~1.5 e0^3 (e0 the seed's) before the last
+//     rounding, far under 2^-53, so d1 is within 1 ulp.
+//   * d2 = sqrt(g^2 + x^2 + y^2): 8 -> 6, the same with h refined too; h feeds dd1 = d1 (1 + alpha (2 g h - 1)), written
+//     so that no loop-invariant 1 - alpha or 2 alpha is recomputed in the loop (the one-pass kernel reads alpha from the
+//     constant bank, and ptxas rematerialises such values rather than keep them in registers).
+//   * den = alpha d2 + (1 - alpha) g = g + alpha dd0: 2 -> 1 (dd0 is needed anyway).  Correctly rounded when g >= d2/2 (dd0
+//     is then exact, Sterbenz); otherwise an absolute error of ~1 ulp of max(d2, |g|), as in the two-product form.
+//   * 1/den: one Newton step with the cubic term, r (1 + e + e^2), e = 1 - den r: error e^3 ~ 2^-66 before the last
+//     rounding, <= 1 ulp, in 3 fma instead of 4.
+//   * accumulation: every distortion entry is cu dd_k or cv dd_k (cu = d(u)/d(den)), so the products with them factor:
+//       H[f,d_k] = sum (mx cu) dd_k   H[c,d_k] = sum cu dd_k   g[d_k] = sum (cu ru + cv rv) dd_k
+//       H[d_j,d_k] = sum (cu^2 + cv^2) dd_j dd_k
+//     30 FP64 instructions instead of 33 with the count: the valid points are counted in an int in the loop
+//     (point(acc, count, ...)) that the kernel converts once, exactly.
+// Invalid points are folded in by selects on mx, my, ru, rv, cu, cv and both dd_k: a rejected point can carry NaN in any of
+// them, and every accumulated term is a product of those.
+// ---------------------------------------------------------------------------------------
+// y * 2^e for a normal y and a normal result, by an integer add to the exponent field instead of a DMUL.
+__device__ __forceinline__ double lin_scale2(double y, int e) { return __hiloint2double(__double2hiint(y) + (e << 20), __double2loint(y)); }
+
+template <> struct LinOps<ACM_MODEL_DOUBLE_SPHERE, ACM_RESIDUAL_PIXEL> {
+    static constexpr int ND = 2, P = 6;
+    static constexpr bool INT_COUNT = true;
+    // HFD / HCD: u-row d0, u-row d1, v-row d0, v-row d1; HDD: d0 d0, d0 d1, d1 d1
+    static constexpr int HFF = 0, HFC = 2, GF = 4, GC = 6, HFD = 8, HCD = 12, GD = 16, HDD = 18, COST = 21, COUNT = 22, NACC = 23;
+    static __device__ __forceinline__ void point(double* acc, int& count, const LinParams& p, double x, double y, double z, double u, double v) {
+        const double alpha = p.d[0], xi = p.d[1];
+        const double nk0 = -p.k0;
+        const double rr = fma(y, y, x * x);
+        const double a1 = fma(z, z, rr);
+        double s, h, g, r;
+        asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(s) : "d"(a1));
+        h = lin_scale2(s, -1); g = a1 * s;
+        r = fma(-g, h, 0.5);
+        g = fma(g, r, g);
+        const double d1 = fma(fma(-g, g, a1), h, g);
+        const double gz = fma(xi, d1, z);
+        const double q = fma(gz, gz, rr);
+        asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(s) : "d"(q));
+        h = lin_scale2(s, -1); g = q * s;
+        r = fma(-g, h, 0.5);
+        g = fma(g, r, g); h = fma(h, r, h);
+        const double d2 = fma(fma(-g, g, q), h, g);
+        double dd0 = d2 - gz;
+        const double den = fma(alpha, dd0, gz);
+        double dd1 = d1 * fma(alpha, fma(gz, lin_scale2(h, 1), -1.0), 1.0);   // d1 (1 - alpha + alpha g / d2)
+        const bool ok = (den >= LIN_PRECISION) && (z > nk0 * d1);
+        double inv;
+        asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(inv) : "d"(den));
+        const double e = fma(-den, inv, 1.0);
+        inv = fma(inv, fma(e, e, e), inv);
+        double mx = x * inv, my = y * inv;
+        double ru = fma(p.fx, mx, p.cx) - u, rv = fma(p.fy, my, p.cy) - v;
+        double cu = -(p.fx * mx) * inv, cv = -(p.fy * my) * inv;   // d(u)/d(den), d(v)/d(den)
+        mx = ok ? mx : 0.0; my = ok ? my : 0.0; ru = ok ? ru : 0.0; rv = ok ? rv : 0.0;
+        cu = ok ? cu : 0.0; cv = ok ? cv : 0.0; dd0 = ok ? dd0 : 0.0; dd1 = ok ? dd1 : 0.0;
+        acc[HFF] = fma(mx, mx, acc[HFF]); acc[HFF + 1] = fma(my, my, acc[HFF + 1]);
+        acc[HFC] += mx; acc[HFC + 1] += my;
+        acc[GF] = fma(mx, ru, acc[GF]); acc[GF + 1] = fma(my, rv, acc[GF + 1]);
+        acc[GC] += ru; acc[GC + 1] += rv;
+        const double a = mx * cu, b = my * cv, c = fma(cu, ru, cv * rv), w = fma(cu, cu, cv * cv);
+        const double dd[2] = {dd0, dd1};
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+            acc[HFD + k] = fma(a, dd[k], acc[HFD + k]);
+            acc[HFD + 2 + k] = fma(b, dd[k], acc[HFD + 2 + k]);
+            acc[HCD + k] = fma(cu, dd[k], acc[HCD + k]);
+            acc[HCD + 2 + k] = fma(cv, dd[k], acc[HCD + 2 + k]);
+            acc[GD + k] = fma(c, dd[k], acc[GD + k]);
+        }
+        const double wd0 = w * dd0, wd1 = w * dd1;
+        acc[HDD + 0] = fma(wd0, dd0, acc[HDD + 0]);
+        acc[HDD + 1] = fma(wd0, dd1, acc[HDD + 1]);
+        acc[HDD + 2] = fma(wd1, dd1, acc[HDD + 2]);
+        acc[COST] = fma(ru, ru, fma(rv, rv, acc[COST]));
+        count += ok;
+    }
+    template <bool FULL = true>
+    __host__ __device__ static void unpack(const double* __restrict__ r, const double* __restrict__ x, double* __restrict__ H, double* __restrict__ g, double* __restrict__ cost, double* __restrict__ count) {
+        (void)x;
+        if (FULL) for (int i = 0; i < P * P; ++i) H[i] = 0.0;
+        const double cnt = r[COUNT];
+        H[0 * P + 0] = r[HFF]; H[1 * P + 1] = r[HFF + 1];
+        H[0 * P + 2] = r[HFC]; H[1 * P + 3] = r[HFC + 1];
+        H[2 * P + 2] = cnt; H[3 * P + 3] = cnt;
+        for (int k = 0; k < 2; ++k) {
+            H[0 * P + 4 + k] = r[HFD + k]; H[1 * P + 4 + k] = r[HFD + 2 + k];
+            H[2 * P + 4 + k] = r[HCD + k]; H[3 * P + 4 + k] = r[HCD + 2 + k];
+            g[4 + k] = r[GD + k];
+        }
+        H[4 * P + 4] = r[HDD]; H[4 * P + 5] = r[HDD + 1]; H[5 * P + 5] = r[HDD + 2];
+        g[0] = r[GF]; g[1] = r[GF + 1]; g[2] = r[GC]; g[3] = r[GC + 1];
+        if (FULL) for (int a = 0; a < P; ++a) for (int b = 0; b < a; ++b) H[a * P + b] = H[b * P + a];
+        *cost = 0.5 * r[COST];
+        *count = cnt;
+    }
+};
+
+// What the streaming kernel calls per point: ops.point(acc, ...), or ops.point(acc, count, ...) for the specialisations
+// that count valid points in an int (INT_COUNT = true); the kernel stores that count into acc[COUNT] once after its loop.
+template <class Ops, class = void> struct LinIntCount { static constexpr bool value = false; };
+template <class Ops> struct LinIntCount<Ops, std::void_t<decltype(Ops::INT_COUNT)>> { static constexpr bool value = Ops::INT_COUNT; };
+template <class Ops>
+__device__ __forceinline__ void lin_point(double* acc, int& count, const LinParams& p, double x, double y, double z, double u, double v) {
+    if constexpr (LinIntCount<Ops>::value) Ops::point(acc, count, p, x, y, z, u, v);
+    else Ops::point(acc, p, x, y, z, u, v);
+}

@@ -520,6 +520,7 @@ __device__ __forceinline__ void lin_stream_pass(const LinKernelArgs& a, const Li
     double acc[NACC];
 #pragma unroll
     for (int i = 0; i < NACC; ++i) acc[i] = 0.0;
+    int cnt = 0;   // valid points, for the specialisations that count them in an int (LinIntCount)
     size_t i = i0;
     if constexpr (DEPTH > 0 && StreamCfg<M, SOLVE>::PTS == 4) {
         // two packets (four points) per trip: the four evaluation chains are independent, the points still enter every
@@ -532,10 +533,10 @@ __device__ __forceinline__ void lin_stream_pass(const LinKernelArgs& a, const Li
             asm volatile("cp.async.wait_group %0;" ::"n"(DEPTH > 1 ? DEPTH - 2 : 0) : "memory");
             const double2 x0 = ld(stage, 0), y0 = ld(stage, 1), z0 = ld(stage, 2), u0 = ld(stage, 3), v0 = ld(stage, 4);
             const double2 x1 = ld(stage + 1, 0), y1 = ld(stage + 1, 1), z1 = ld(stage + 1, 2), u1 = ld(stage + 1, 3), v1 = ld(stage + 1, 4);
-            LM_::point(acc, p, x0.x, y0.x, z0.x, u0.x, v0.x);
-            LM_::point(acc, p, x0.y, y0.y, z0.y, u0.y, v0.y);
-            LM_::point(acc, p, x1.x, y1.x, z1.x, u1.x, v1.x);
-            LM_::point(acc, p, x1.y, y1.y, z1.y, u1.y, v1.y);
+            lin_point<LM_>(acc, cnt, p, x0.x, y0.x, z0.x, u0.x, v0.x);
+            lin_point<LM_>(acc, cnt, p, x0.y, y0.y, z0.y, u0.y, v0.y);
+            lin_point<LM_>(acc, cnt, p, x1.x, y1.x, z1.x, u1.x, v1.x);
+            lin_point<LM_>(acc, cnt, p, x1.y, y1.y, z1.y, u1.y, v1.y);
             issue(stage, i + (size_t)DEPTH * stride);
             issue(stage + 1, i + (size_t)(DEPTH + 1) * stride);
             stage = (stage + 2 == DEPTH) ? 0 : stage + 2;
@@ -544,8 +545,8 @@ __device__ __forceinline__ void lin_stream_pass(const LinKernelArgs& a, const Li
         if (i < npairs) {   // odd number of packets: the last one alone
             asm volatile("cp.async.wait_group 0;" ::: "memory");
             const double2 x0 = ld(stage, 0), y0 = ld(stage, 1), z0 = ld(stage, 2), u0 = ld(stage, 3), v0 = ld(stage, 4);
-            LM_::point(acc, p, x0.x, y0.x, z0.x, u0.x, v0.x);
-            LM_::point(acc, p, x0.y, y0.y, z0.y, u0.y, v0.y);
+            lin_point<LM_>(acc, cnt, p, x0.x, y0.x, z0.x, u0.x, v0.x);
+            lin_point<LM_>(acc, cnt, p, x0.y, y0.y, z0.y, u0.y, v0.y);
             i += stride;
         }
         asm volatile("cp.async.wait_group 0;" ::: "memory");
@@ -557,8 +558,8 @@ __device__ __forceinline__ void lin_stream_pass(const LinKernelArgs& a, const Li
             const double2 x = lin_ring[(stage * 5 + 0) * BS + tid], y = lin_ring[(stage * 5 + 1) * BS + tid],
                           z = lin_ring[(stage * 5 + 2) * BS + tid], u = lin_ring[(stage * 5 + 3) * BS + tid],
                           v = lin_ring[(stage * 5 + 4) * BS + tid];
-            LM_::point(acc, p, x.x, y.x, z.x, u.x, v.x);
-            LM_::point(acc, p, x.y, y.y, z.y, u.y, v.y);
+            lin_point<LM_>(acc, cnt, p, x.x, y.x, z.x, u.x, v.x);
+            lin_point<LM_>(acc, cnt, p, x.y, y.y, z.y, u.y, v.y);
             issue(stage, i + (size_t)DEPTH * stride);  // after the packet has been consumed
             stage = (stage + 1 == DEPTH) ? 0 : stage + 1;
             i += stride;
@@ -574,8 +575,8 @@ __device__ __forceinline__ void lin_stream_pass(const LinKernelArgs& a, const Li
             const size_t nx = i + stride;
             const size_t j = nx < npairs ? nx : i;  // clamp: the tail re-reads its own (cached) packet
             const double2 x2 = __ldcs(a.X + j), y2 = __ldcs(a.Y + j), z2 = __ldcs(a.Z + j), u2 = __ldcs(a.U + j), v2 = __ldcs(a.V + j);
-            LM_::point(acc, p, x.x, y.x, z.x, u.x, v.x);
-            LM_::point(acc, p, x.y, y.y, z.y, u.y, v.y);
+            lin_point<LM_>(acc, cnt, p, x.x, y.x, z.x, u.x, v.x);
+            lin_point<LM_>(acc, cnt, p, x.y, y.y, z.y, u.y, v.y);
             x = x2; y = y2; z = z2; u = u2; v = v2;
             i = nx;
         }
@@ -586,9 +587,10 @@ __device__ __forceinline__ void lin_stream_pass(const LinKernelArgs& a, const Li
         const double* Xs = reinterpret_cast<const double*>(a.X); const double* Ys = reinterpret_cast<const double*>(a.Y);
         const double* Zs = reinterpret_cast<const double*>(a.Z); const double* Us = reinterpret_cast<const double*>(a.U);
         const double* Vs = reinterpret_cast<const double*>(a.V);
-        LM_::point(acc, p, Xs[t], Ys[t], Zs[t], Us[t], Vs[t]);
+        lin_point<LM_>(acc, cnt, p, Xs[t], Ys[t], Zs[t], Us[t], Vs[t]);
         npts += 1;
     }
+    if constexpr (LinIntCount<LM_>::value) acc[LM_::COUNT] = (double)cnt;
     // invalid points carry the residual (pen, pen): cost += pen^2 per invalid point
     if (a.pen2x2 != 0.0) acc[LM_::COST] += a.pen2x2 * ((double)npts - acc[LM_::COUNT]);
 
