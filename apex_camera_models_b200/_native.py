@@ -16,6 +16,7 @@ ABI_VERSION = 2  # include/acm.h ACM_ABI_VERSION: acm_lm_result gained device_ms
 F64, F32 = 0, 1
 RESIDUAL_PIXEL, RESIDUAL_ALGEBRAIC = 0, 1
 INTERP_NEAREST, INTERP_BILINEAR = 0, 1
+TRI_OK, TRI_UNPROJECT_FIRST, TRI_UNPROJECT_SECOND, TRI_PARALLEL, TRI_BEHIND, TRI_PROJECT = 0, 1, 2, 3, 4, 5
 
 OK = 0
 ERR_INVALID_ARG, ERR_CUDA, ERR_NCCL, ERR_INVALID_PARAMS, ERR_NUMERICAL = -1, -2, -3, -4, -5
@@ -114,6 +115,8 @@ SIGNATURES = {
     "acm_remap_plan_create_rotated": (C.c_int32, [_vp, _cam, _cam, _dp, C.c_int32, C.POINTER(_vp)]),
     "acm_remap_map_rotated": (C.c_int32, [_vp, _cam, _cam, _dp, _vp]),
     "acm_stereo_rectify": (C.c_int32, [_dp, _dp, _dp, _dp, _dp, C.POINTER(C.c_int32)]),
+    "acm_triangulate": (C.c_int32, [_vp, _cam, _cam, _dp, _dp, _vp, _vp, C.c_int32, _vp, _vp, _vp]),
+    "acm_triangulate_host": (C.c_int32, [_vp, _cam, _cam, _dp, _dp, _vp, _vp, C.c_size_t, C.c_int32, _vp, _vp, _vp]),
     "acm_reprojection_error": (C.c_int32, [_vp, _cam, _vp, _vp, C.POINTER(ProjectionError)]),
     "acm_sample_points": (C.c_int32, [_vp, _cam, C.c_size_t, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(C.c_size_t)]),
     "acm_sample_points_shard": (C.c_int32, [_vp, _cam, C.c_size_t, C.c_int32, C.c_int32, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(C.c_size_t)]),

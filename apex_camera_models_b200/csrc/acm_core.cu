@@ -9,6 +9,7 @@
 #include <cmath>
 
 #include <new>
+#include <utility>
 
 #include "acm_internal.cuh"
 
@@ -61,7 +62,7 @@ extern "C" int32_t acm_ctx_create(int32_t device, void* cuda_stream, acm_ctx** o
     ctx->peer_local = nullptr; ctx->d_peer_ptrs = nullptr; ctx->peer_n = 0; ctx->peer_rank = 0; ctx->peer_seq = 0; ctx->peer_failed = false;
     ctx->group = nullptr; ctx->lm_tag = 0; ctx->d_lm_ll = nullptr; ctx->lm_ll_cap = 0; ctx->coop_launch = 0;
     ctx->h_small = nullptr; ctx->d_small_alias = nullptr; ctx->small_cap = 0;
-    ctx->cam_cache_valid = false;
+    ctx->cam_cache[0].valid = ctx->cam_cache[1].valid = false;
     for (int i = 0; i < ACM_MAX_PEERS; ++i) ctx->peer_mapped[i] = nullptr;
 #define CREATE_CUDA(call)                                                                                     \
     do { cudaError_t _e = (call); if (_e != cudaSuccess) { int32_t rc = acm_fail(nullptr, ACM_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(_e)); delete ctx; return rc; } } while (0)
@@ -240,17 +241,47 @@ extern "C" int32_t acm_camera_new(int32_t model, const double* params, size_t n,
 static int32_t make_cam_params_uncached(acm_ctx* ctx, const acm_camera* cam, CamParams* c);
 
 // The host-side gates of the contracted Newton iterations (Kannala-Brandt, RadTan) cost 20-100 us; a context remembers the
-// block of the last camera it prepared, so that a loop of scalar project / unproject calls on one model pays them once.
+// blocks of the two cameras it prepared last, so that a loop of scalar project / unproject calls on one model, or of
+// triangulations on one camera pair, pays them once.
+static bool same_camera(const acm_camera* a, const acm_camera* b) {
+    return a->model == b->model && a->width == b->width && a->height == b->height && a->n_params == b->n_params && a->n_params >= 0 &&
+           a->n_params <= ACM_MAX_PARAMS && memcmp(a->params, b->params, sizeof(double) * a->n_params) == 0;
+}
+
 int32_t acm_make_cam_params(acm_ctx* ctx, const acm_camera* cam, CamParams* c) {
-    if (ctx && cam && ctx->cam_cache_valid && cam->model == ctx->cam_cache_key.model && cam->width == ctx->cam_cache_key.width &&
-        cam->height == ctx->cam_cache_key.height && cam->n_params == ctx->cam_cache_key.n_params && cam->n_params >= 0 &&
-        cam->n_params <= ACM_MAX_PARAMS && memcmp(cam->params, ctx->cam_cache_key.params, sizeof(double) * cam->n_params) == 0) {
-        *c = ctx->cam_cache_val;
-        return ACM_OK;
+    if (ctx && cam) {
+        for (int k = 0; k < 2; ++k) {
+            acm_ctx::CamCacheEntry& e = ctx->cam_cache[k];
+            if (!e.valid || !same_camera(cam, &e.key)) continue;
+            *c = e.val;
+            if (k == 1) std::swap(ctx->cam_cache[0], ctx->cam_cache[1]);  // most recent first
+            return ACM_OK;
+        }
     }
     int32_t rc = make_cam_params_uncached(ctx, cam, c);
-    if (rc == ACM_OK && ctx) { ctx->cam_cache_key = *cam; ctx->cam_cache_val = *c; ctx->cam_cache_valid = true; }
+    if (rc == ACM_OK && ctx) {
+        ctx->cam_cache[1] = ctx->cam_cache[0];
+        ctx->cam_cache[0].key = *cam; ctx->cam_cache[0].val = *c; ctx->cam_cache[0].valid = true;
+    }
     return rc;
+}
+
+// R must be a proper rotation: finite entries, max |R R^T - I| <= 1e-9, det R > 0 (rotated remap plans, acm_stereo_rectify,
+// acm_triangulate).  ctx may be null (acm_stereo_rectify).
+int32_t acm_check_rotation(acm_ctx* ctx, const double* R, const char* who) {
+    if (!R) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: null rotation", who);
+    for (int k = 0; k < 9; ++k)
+        if (!std::isfinite(R[k])) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: rotation has a non-finite entry", who);
+    double dev = 0.0;
+    for (int i = 0; i < 3; ++i)
+        for (int j = 0; j < 3; ++j) {
+            const double d = R[3 * i] * R[3 * j] + R[3 * i + 1] * R[3 * j + 1] + R[3 * i + 2] * R[3 * j + 2] - (i == j ? 1.0 : 0.0);
+            dev = std::fmax(dev, std::fabs(d));
+        }
+    if (!(dev <= 1e-9)) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: rotation is not orthonormal (max |R R^T - I| = %.3g > 1e-9)", who, dev);
+    const double det = R[0] * (R[4] * R[8] - R[5] * R[7]) - R[1] * (R[3] * R[8] - R[5] * R[6]) + R[2] * (R[3] * R[7] - R[4] * R[6]);
+    if (det < 0.0) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: rotation is a reflection (det R < 0)", who);
+    return ACM_OK;
 }
 
 static int32_t make_cam_params_uncached(acm_ctx* ctx, const acm_camera* cam, CamParams* c) {

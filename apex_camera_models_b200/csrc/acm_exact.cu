@@ -1155,23 +1155,6 @@ static int32_t launch_remap_map(acm_ctx* ctx, const CamParams& ci, const CamPara
     return ACM_OK;
 }
 
-// R must be a proper rotation: finite entries, max |R R^T - I| <= 1e-9, det R > 0.  ctx may be null (acm_stereo_rectify).
-static int32_t check_rotation(acm_ctx* ctx, const double* R, const char* who) {
-    if (!R) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: null rotation", who);
-    for (int k = 0; k < 9; ++k)
-        if (!std::isfinite(R[k])) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: rotation has a non-finite entry", who);
-    double dev = 0.0;
-    for (int i = 0; i < 3; ++i)
-        for (int j = 0; j < 3; ++j) {
-            const double d = R[3 * i] * R[3 * j] + R[3 * i + 1] * R[3 * j + 1] + R[3 * i + 2] * R[3 * j + 2] - (i == j ? 1.0 : 0.0);
-            dev = std::fmax(dev, std::fabs(d));
-        }
-    if (!(dev <= 1e-9)) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: rotation is not orthonormal (max |R R^T - I| = %.3g > 1e-9)", who, dev);
-    const double det = R[0] * (R[4] * R[8] - R[5] * R[7]) - R[1] * (R[3] * R[8] - R[5] * R[6]) + R[2] * (R[3] * R[7] - R[4] * R[6]);
-    if (det < 0.0) return acm_fail(ctx, ACM_ERR_INVALID_ARG, "%s: rotation is a reflection (det R < 0)", who);
-    return ACM_OK;
-}
-
 // source coordinates of every pixel of output_cam's grid: the remap map of input_cam -> output_cam, rotated by R unless it is
 // null (R checked by the caller)
 static int32_t remap_map(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam, const double* R, double* d_src_xy) {
@@ -1202,7 +1185,7 @@ extern "C" int32_t acm_remap_map(acm_ctx* ctx, const acm_camera* input_cam, cons
 extern "C" int32_t acm_remap_map_rotated(acm_ctx* ctx, const acm_camera* input_cam, const acm_camera* output_cam, const double R[9],
                                          double* d_src_xy) {
     ACM_ENTER(ctx);
-    const int32_t rc = check_rotation(ctx, R, "remap_map");
+    const int32_t rc = acm_check_rotation(ctx, R, "remap_map");
     if (rc) return rc;
     return remap_map_entry(ctx, input_cam, output_cam, R, d_src_xy);
 }
@@ -1281,7 +1264,7 @@ extern "C" int32_t acm_remap_plan_create_rotated(acm_ctx* ctx, const acm_camera*
     ACM_REQUIRE(ctx, out, "remap_plan: null output");
     *out = nullptr;
     ACM_REQUIRE(ctx, output_cam, "remap_plan: a rotated plan needs an output camera (a Pinhole camera gives undistort_image's view)");
-    const int32_t rc = check_rotation(ctx, R, "remap_plan");
+    const int32_t rc = acm_check_rotation(ctx, R, "remap_plan");
     if (rc) return rc;
     return create_plan(ctx, input_cam, output_cam, nullptr, R, interpolation, out);
 }
@@ -1379,7 +1362,7 @@ static void mat3_vec(const double* A, const double* x, double* y) {
 extern "C" int32_t acm_stereo_rectify(const double R[9], const double t[3], double R1[9], double R2[9], double* baseline,
                                       int32_t* vertical) {
     if (!t || !R1 || !R2 || !baseline || !vertical) return acm_fail(nullptr, ACM_ERR_INVALID_ARG, "stereo_rectify: null argument");
-    const int32_t rc = check_rotation(nullptr, R, "stereo_rectify");
+    const int32_t rc = acm_check_rotation(nullptr, R, "stereo_rectify");
     if (rc) return rc;
     if (!std::isfinite(t[0]) || !std::isfinite(t[1]) || !std::isfinite(t[2]))
         return acm_fail(nullptr, ACM_ERR_INVALID_ARG, "stereo_rectify: translation has a non-finite entry");

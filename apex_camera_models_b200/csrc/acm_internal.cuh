@@ -99,8 +99,9 @@ struct acm_ctx {
     std::unordered_map<const void*, int> blocks_per_sm;
     // small-batch host path (acm_project_host / acm_unproject_host with few points): mapped pinned staging, no allocation per call
     void* h_small; void* d_small_alias; size_t small_cap; unsigned long long small_seq;
-    // last camera block prepared by acm_make_cam_params and its device form (the Newton gates are not free)
-    acm_camera cam_cache_key; CamParams cam_cache_val; bool cam_cache_valid;
+    // the two camera blocks acm_make_cam_params prepared last and their device forms, most recent first (the Newton gates are
+    // not free, and a call on a camera pair -- acm_triangulate -- prepares two blocks)
+    struct CamCacheEntry { acm_camera key; CamParams val; bool valid; } cam_cache[2];
 };
 
 // Make the context's device current on the calling thread (contexts of several GPUs may be driven by one thread).
@@ -150,6 +151,8 @@ void acm_set_global_error(const char* msg);
 
 // host helpers implemented in acm_core.cu
 int32_t acm_make_cam_params(acm_ctx* ctx, const acm_camera* cam, CamParams* out);
+// R (row-major 3x3) must be a proper rotation: finite entries, max |R R^T - I| <= 1e-9, det R > 0.  ctx may be null.
+int32_t acm_check_rotation(acm_ctx* ctx, const double* R, const char* who);
 int32_t acm_device_malloc(acm_ctx* ctx, void** out, size_t bytes);  // cudaMalloc; empties the free list and retries when out of memory
 int32_t acm_ensure_stage(acm_ctx* ctx, size_t bytes);
 int32_t acm_ensure_host_stage(acm_ctx* ctx, size_t bytes);

@@ -91,6 +91,14 @@ __host__ __device__ inline void lin_derive(int model, LinParams& p) {
     }
 }
 
+// LinParams of a camera block on the host (acm_solver.cu's passes and Jacobian kernels, acm_triangulate.cu)
+static inline void make_lin_params(const acm_camera* cam, LinParams* p) {
+    memset(p, 0, sizeof(*p));
+    p->fx = cam->params[0]; p->fy = cam->params[1]; p->cx = cam->params[2]; p->cy = cam->params[3];
+    for (int i = 4; i < cam->n_params; ++i) p->d[i - 4] = cam->params[i];
+    lin_derive(cam->model, *p);
+}
+
 // ---------------------------------------------------------------------------------------
 // Per-model residual + Jacobian rows.  eval() returns validity (the model's geometric test,
 // no image-bounds test: the factor has no resolution) and fills

@@ -910,13 +910,6 @@ static int32_t check_lin_args(acm_ctx* ctx, const acm_camera* cam, const acm_poi
     return ACM_OK;
 }
 
-static void make_lin_params(const acm_camera* cam, LinParams* p) {
-    memset(p, 0, sizeof(*p));
-    p->fx = cam->params[0]; p->fy = cam->params[1]; p->cx = cam->params[2]; p->cy = cam->params[3];
-    for (int i = 4; i < cam->n_params; ++i) p->d[i - 4] = cam->params[i];
-    lin_derive(cam->model, *p);
-}
-
 static bool peers_usable(const acm_ctx* ctx) { return ctx->peer_n > 1; }
 
 // A peer exchange that timed out leaves the ranks' exchange counters out of step: refuse to go on

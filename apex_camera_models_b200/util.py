@@ -1,7 +1,7 @@
 """util hot loops of the reference: undistort_image (src/util/undistort.rs:14-105), sample_points
 (src/util/point_sampling.rs:46-120), compute_reprojection_error (src/util/error_metrics.rs:62-121); and remap plans
-(camera-to-camera image remap, composed of the reference's unproject, project and interpolate_pixel), rotated plans and
-stereo rectification."""
+(camera-to-camera image remap, composed of the reference's unproject, project and interpolate_pixel), rotated plans,
+stereo rectification and triangulation of matched pixels of a calibrated pair."""
 from __future__ import annotations
 
 import ctypes as C
@@ -297,3 +297,84 @@ def compute_reprojection_error(camera_model: CameraModel, points3d, points2d) ->
         p.free()
     ctx.check(rc)
     return ProjectionError(out.rmse, out.min, out.max, out.mean, out.stddev, out.median, int(out.count))
+
+
+class TriangulationStatus(enum.IntEnum):
+    """Per-pair status of `triangulate_points` (include/acm.h ACM_TRI_*), in the order the steps decide it."""
+    Ok = N.TRI_OK
+    UnprojectFirst = N.TRI_UNPROJECT_FIRST      # the first camera's unproject failed (any CameraModelError)
+    UnprojectSecond = N.TRI_UNPROJECT_SECOND    # the second camera's unproject failed
+    Parallel = N.TRI_PARALLEL                   # 1 - (d1 . d2')^2 <= 1e-12: the rays are parallel
+    Behind = N.TRI_BEHIND                       # the closest approach lies behind either camera
+    Project = N.TRI_PROJECT                     # the point does not project into both cameras
+
+
+def _translation_array(t):
+    tv = np.array(t, dtype=np.float64).ravel()
+    if tv.shape != (3,):
+        raise UtilError(f"Invalid parameters: translation must have 3 entries, got {tv.size}")
+    return (C.c_double * 3)(*tv)
+
+
+def triangulate_points(first: CameraModel, second: CameraModel, R, t, points1, points2, max_iterations: int = 10):
+    """3-D points of matched pixels of a calibrated pair, x_cam2 = R x_cam1 + t (the convention of `stereo_rectify`).
+
+    points1 / points2: (N, 2) pixels of `first` / `second` (numpy arrays or device `Points`).  Per pair: both pixels are
+    unprojected (IEEE form, with each model's pixel-bounds test), the midpoint of the rays' closest approach is taken in
+    the first camera's frame, and with `max_iterations > 0` up to that many damped Gauss-Newton (Levenberg-Marquardt)
+    trials minimise the squared pixel errors of the point's projections into both cameras.  Any two camera models work,
+    including fields of view beyond 90 degrees.
+
+    Returns (points_3d (N, 3) in the first camera's frame, errors (N, 2) = |first.project(X) - uv1| and
+    |second.project(R X + t) - uv2| in pixels, status (N,) uint8 of `TriangulationStatus`); points and errors are NaN
+    where the status is not Ok.  Always numpy, whatever the input.
+
+    Rectified pixels of a `StereoRectifier` triangulate with the rectified pinhole on both sides, R = I and
+    t = baseline * e (e = x axis, or y when `vertical`); the points are then in the first RECTIFIED frame, and
+    `rig.R1.T @ X` takes them back to the first camera's."""
+    if first is None or second is None:
+        raise UtilError("Camera model does not exist")
+    if max_iterations < 0:
+        raise UtilError("Invalid parameters: max_iterations must be >= 0")
+    ctx = first.ctx
+    Rm, tv = _rotation_array(R), _translation_array(t)
+    ca, cb = first.camera_block(), second.camera_block()
+    if isinstance(points1, Points) or isinstance(points2, Points):
+        own = []
+
+        def dev(a):
+            if isinstance(a, Points):
+                return a
+            p = Points.from_numpy(ctx, np.ascontiguousarray(a, dtype=np.float64).reshape(-1, 2))
+            own.append(p)
+            return p
+        try:
+            a, b = dev(points1), dev(points2)
+            n = len(a)
+            xyz = Points(ctx, 3, n)
+            own.append(xyz)
+            d = ctx.device_alloc(max(n, 1) * 17)  # two rows of errors, then the status bytes
+            try:
+                ctx.check(_lib.acm_triangulate(ctx.handle, C.byref(ca), C.byref(cb), Rm, tv, a.handle, b.handle, int(max_iterations),
+                                               xyz.handle, C.c_void_p(d), C.c_void_p(d + 16 * n)))
+                err, st = np.empty((2, n)), np.empty(n, np.uint8)
+                if n:
+                    ctx.d2h(err, d); ctx.d2h(st, d + 16 * n)
+                ctx.sync()
+                pts = xyz.numpy()
+            finally:
+                ctx.device_free(d)
+        finally:
+            for p in own:
+                p.free()
+        return pts, np.ascontiguousarray(err.T), st
+    uv1 = np.ascontiguousarray(points1, dtype=np.float64).reshape(-1, 2)
+    uv2 = np.ascontiguousarray(points2, dtype=np.float64).reshape(-1, 2)
+    if len(uv1) != len(uv2):
+        raise UtilError(f"Invalid parameters: {len(uv1)} pixels of the first camera but {len(uv2)} of the second")
+    n = len(uv1)
+    xyz, err, st = np.empty((n, 3)), np.empty((n, 2)), np.empty(n, np.uint8)
+    ctx.check(_lib.acm_triangulate_host(ctx.handle, C.byref(ca), C.byref(cb), Rm, tv, uv1.ctypes.data_as(C.c_void_p),
+                                        uv2.ctypes.data_as(C.c_void_p), n, int(max_iterations), xyz.ctypes.data_as(C.c_void_p),
+                                        err.ctypes.data_as(C.c_void_p), st.ctypes.data_as(C.c_void_p)))
+    return xyz, err, st

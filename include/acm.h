@@ -273,6 +273,49 @@ int32_t acm_remap_map_rotated(acm_ctx* ctx, const acm_camera* input_cam, const a
 int32_t acm_stereo_rectify(const double R[9], const double t[3], double R1[9], double R2[9],
                            double* baseline, int32_t* vertical);
 
+/* ---- triangulation of matched pixels of a calibrated pair (beyond the reference) -----
+ * x_cam2 = R x_cam1 + t (R row-major; the convention of acm_stereo_rectify).  Per pair, in this order:
+ *   1. d1 = first.unproject(uv1), d2 = second.unproject(uv2) in the IEEE form of acm_unproject_ieee (with each model's
+ *      pixel-bounds test): UNPROJECT_FIRST / UNPROJECT_SECOND on any CameraModelError.
+ *   2. In the first camera's frame: d2' = R^T d2 and c2 = -R^T t, d2'[k] = (R[0][k]*x + R[1][k]*y) + R[2][k]*z with every
+ *      operation rounded (the rotated remap's order).
+ *   3. Midpoint of the closest approach of s1 d1 and c2 + s2 d2': b = d1.d2', p = d1.c2, q = d2'.c2,
+ *      PARALLEL when 1 - b^2 <= ACM_TRI_PARALLEL_EPS (rays within ~1e-6 rad of each other), s1 = (p - b q) / (1 - b^2),
+ *      s2 = (b p - q) / (1 - b^2), BEHIND when s1 <= 0 or s2 <= 0, X = ((s1 d1 + c2) + s2 d2') / 2.
+ *   4. PROJECT unless X projects into both cameras (project with geometric validity, no image-bounds test, like
+ *      acm_project_point_jacobian; the second camera sees R X + t).
+ *   5. max_iterations > 0: at most that many damped Gauss-Newton (Levenberg-Marquardt) trials on the 4 pixel residuals
+ *      first.project(X) - uv1, second.project(R X + t) - uv2, Jacobian [J1(X); J2(R X + t) R] with the analytic 2x3 point
+ *      Jacobians, step from a 3x3 Cholesky of H + lambda diag(H) (H = J^T J); a trial is accepted only when both projections
+ *      stay valid and the cost (sum of the squared residuals) decreases.  lambda starts at ACM_TRI_LAMBDA0, is divided by
+ *      ACM_TRI_LAMBDA_FACTOR on acceptance and multiplied by it on rejection (a failed factorisation is a rejection); the
+ *      loop stops after an accepted step with max|delta| <= ACM_TRI_STEP_TOL * max(1, max|X|).
+ * uv1 / uv2: dim-2 f64 buffers of n pixels of the first / second camera; xyz: dim-3 f64 buffer, the point in the FIRST
+ * camera's frame, NaN where status != OK.  d_err (optional): two rows of n doubles, |first.project(X) - uv1| and
+ * |second.project(R X + t) - uv2| (Euclidean, pixels; NaN where status != OK).  d_status (optional): ACM_TRI_* per pair.
+ * ACM_ERR_INVALID_ARG for a null camera or buffer, a dimension or length mismatch, non-f64 buffers, max_iterations < 0,
+ * an R that is not a rotation (the check of acm_remap_plan_create_rotated), a non-finite t or t = 0.  n = 0 launches
+ * nothing; otherwise one kernel. */
+enum {
+    ACM_TRI_OK = 0,
+    ACM_TRI_UNPROJECT_FIRST = 1,   /* first.unproject(uv1) failed (any CameraModelError) */
+    ACM_TRI_UNPROJECT_SECOND = 2,  /* second.unproject(uv2) failed */
+    ACM_TRI_PARALLEL = 3,          /* 1 - (d1.d2')^2 <= ACM_TRI_PARALLEL_EPS */
+    ACM_TRI_BEHIND = 4,            /* the closest-approach parameter along either ray is <= 0 */
+    ACM_TRI_PROJECT = 5            /* the returned point does not project (geometric validity) into both cameras */
+};
+#define ACM_TRI_PARALLEL_EPS 1e-12
+#define ACM_TRI_LAMBDA0 1e-3
+#define ACM_TRI_LAMBDA_FACTOR 10.0
+#define ACM_TRI_STEP_TOL 1e-12
+int32_t acm_triangulate(acm_ctx* ctx, const acm_camera* first, const acm_camera* second, const double R[9], const double t[3],
+                        const acm_points* uv1, const acm_points* uv2, int32_t max_iterations, acm_points* xyz,
+                        double* d_err, uint8_t* d_status);
+/* synchronous host form: AoS f64 in (uvuv...), xyz AoS out (xyzxyz...), err (2n, AoS: e1 e2 per pair) or NULL, status or NULL */
+int32_t acm_triangulate_host(acm_ctx* ctx, const acm_camera* first, const acm_camera* second, const double R[9], const double t[3],
+                             const double* uv1_aos, const double* uv2_aos, size_t n, int32_t max_iterations,
+                             double* xyz_aos, double* err, uint8_t* status);
+
 /* util::compute_reprojection_error (reference src/util/error_metrics.rs:62-121) */
 typedef struct acm_projection_error {
     double rmse, min, max, mean, stddev, median;

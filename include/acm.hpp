@@ -412,6 +412,26 @@ inline StereoRectification stereo_rectify(const std::array<double, 9>& R, const 
     return s;
 }
 
+// Triangulation of matched pixels of a calibrated pair, x_cam2 = R x_cam1 + t (acm_triangulate_host): points in the first
+// camera's frame (NaN where status != ACM_TRI_OK), per-pair pixel errors in both cameras and the ACM_TRI_* status.
+// max_iterations = 0: the midpoint of the rays' closest approach; > 0: at most that many Levenberg-Marquardt trials.
+struct Triangulation {
+    std::vector<double> points;  // xyz per pair (Matrix3xX memory order)
+    std::vector<double> errors;  // |first.project(X) - uv1|, |second.project(R X + t) - uv2| per pair
+    std::vector<uint8_t> status;
+};
+
+inline Triangulation triangulate(const CameraModel& first, const CameraModel& second, const std::array<double, 9>& R,
+                                 const std::array<double, 3>& t, const double* uv1_aos, const double* uv2_aos, size_t n,
+                                 int32_t max_iterations = 10) {
+    Triangulation out;
+    out.points.resize(3 * n); out.errors.resize(2 * n); out.status.resize(n);
+    const acm_camera a = first.block(), b = second.block();
+    first.ctx().check(acm_triangulate_host(first.ctx().handle(), &a, &b, R.data(), t.data(), uv1_aos, uv2_aos, n, max_iterations,
+                                           out.points.data(), out.errors.data(), out.status.data()));
+    return out;
+}
+
 // ---- util::image_quality (image_quality.rs) on RGB8 interleaved images (w*h*3 bytes) --------------
 struct ImageQualityMetrics { double psnr, ssim; };   // image_quality.rs:20-26
 

@@ -334,6 +334,30 @@ impl<M: CameraModel> GpuCamera<M> {
         Ok(RemapPlan { h, ctx: self.ctx.clone(), wi: ri.width, hi: ri.height, wo: ro.width, ho: ro.height })
     }
 
+    /// Triangulation of matched pixels of this camera (`uv1`, first) and `second` (`uv2`), x_cam2 = R x_cam1 + t with `r`
+    /// row-major (the convention of [`stereo_rectify`]).  `max_iterations` = 0: the midpoint of the rays' closest approach;
+    /// > 0: at most that many Levenberg-Marquardt trials on the four pixel residuals.  Returns the points in this camera's
+    /// frame (NaN where the status is not `ACM_TRI_OK`), the pixel errors in both cameras per pair and the `ACM_TRI_*` status.
+    pub fn triangulate<O: CameraModel>(&self, second: &GpuCamera<O>, r: &[f64; 9], t: &[f64; 3], uv1: &Matrix2xX<f64>,
+                                       uv2: &Matrix2xX<f64>, max_iterations: i32)
+        -> Result<(Matrix3xX<f64>, Matrix2xX<f64>, Vec<u8>), CameraModelError> {
+        let n = uv1.ncols();
+        if uv2.ncols() != n {
+            return Err(CameraModelError::InvalidParams(format!("{} pixels of the first camera but {} of the second", n, uv2.ncols())));
+        }
+        let (a, b) = (self.block(), second.block());
+        let mut xyz = Matrix3xX::<f64>::zeros(n);
+        let mut err = Matrix2xX::<f64>::zeros(n);
+        let mut status = vec![0u8; n];
+        let _g = self.ctx.lock();
+        let rc = unsafe {
+            sys::acm_triangulate_host(self.ctx.0, &a, &b, r.as_ptr(), t.as_ptr(), uv1.as_ptr(), uv2.as_ptr(), n, max_iterations,
+                                      xyz.as_mut_ptr(), err.as_mut_ptr(), status.as_mut_ptr())
+        };
+        if rc != sys::ACM_OK { return Err(self.ctx.err(rc)); }
+        Ok((xyz, err, status))
+    }
+
     /// README-era `project(&p, compute_jacobian = true)`: uv plus the 2xP Jacobian w.r.t. `[fx, fy, cx, cy, dist..]`
     /// (per-model docs, double_sphere.rs:326-332) and the 2x3 Jacobian w.r.t. the 3-D point (trait doc, mod.rs:246-252).
     pub fn project_with_jacobians(&self, p: &Vector3<f64>)
