@@ -17,9 +17,9 @@ from .camera import (CameraModel, DoubleSphereModel, EucmModel, FovModel, Intrin
 from .optimization import (DoubleSphereOptimizationCost, EucmOptimizationCost, FovOptimizationCost,
                            KannalaBrandtOptimizationCost, LevenbergMarquardtConfig, OptimizationCost, RadTanOptimizationCost,
                            UcmOptimizationCost, CONVERTER_BOUNDS, CANONICAL_RESIDUAL)
-from .util import (InterpolationMethod, ProjectionError, RemapPlan, StereoRectifier, TriangulationStatus, compute_reprojection_error,
-                   remap_image, remap_images, remap_map, sample_points, stereo_rectify, triangulate_points, undistort_image,
-                   undistort_images, undistort_map)
+from .util import (DepthStatus, InterpolationMethod, ProjectionError, RemapPlan, StereoRectifier, TriangulationStatus,
+                   compute_reprojection_error, depth_to_points, remap_image, remap_images, remap_map, render_depth, sample_points,
+                   stereo_rectify, triangulate_points, undistort_image, undistort_images, undistort_map)
 from .image_quality import (ImageQualityMetrics, calculate_psnr, calculate_ssim, compute_image_quality_metrics,
                             create_combined_projection_image, create_combined_projection_image_on_reference,
                             create_projection_image, model_projection_visualization)

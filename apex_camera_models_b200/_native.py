@@ -17,6 +17,7 @@ F64, F32 = 0, 1
 RESIDUAL_PIXEL, RESIDUAL_ALGEBRAIC = 0, 1
 INTERP_NEAREST, INTERP_BILINEAR = 0, 1
 TRI_OK, TRI_UNPROJECT_FIRST, TRI_UNPROJECT_SECOND, TRI_PARALLEL, TRI_BEHIND, TRI_PROJECT = 0, 1, 2, 3, 4, 5
+DEPTH_OK, DEPTH_EMPTY, DEPTH_UNPROJECT = 0, 1, 2
 
 OK = 0
 ERR_INVALID_ARG, ERR_CUDA, ERR_NCCL, ERR_INVALID_PARAMS, ERR_NUMERICAL = -1, -2, -3, -4, -5
@@ -117,6 +118,9 @@ SIGNATURES = {
     "acm_stereo_rectify": (C.c_int32, [_dp, _dp, _dp, _dp, _dp, C.POINTER(C.c_int32)]),
     "acm_triangulate": (C.c_int32, [_vp, _cam, _cam, _dp, _dp, _vp, _vp, C.c_int32, _vp, _vp, _vp]),
     "acm_triangulate_host": (C.c_int32, [_vp, _cam, _cam, _dp, _dp, _vp, _vp, C.c_size_t, C.c_int32, _vp, _vp, _vp]),
+    "acm_render_depth": (C.c_int32, [_vp, _cam, _dp, _dp, _vp, _vp, _vp]),
+    "acm_render_depth_host": (C.c_int32, [_vp, _cam, _dp, _dp, _vp, C.c_size_t, _vp, _vp]),
+    "acm_depth_to_points": (C.c_int32, [_vp, _cam, _dp, _dp, _vp, _vp, _vp]),
     "acm_reprojection_error": (C.c_int32, [_vp, _cam, _vp, _vp, C.POINTER(ProjectionError)]),
     "acm_sample_points": (C.c_int32, [_vp, _cam, C.c_size_t, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(C.c_size_t)]),
     "acm_sample_points_shard": (C.c_int32, [_vp, _cam, C.c_size_t, C.c_int32, C.c_int32, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(C.c_size_t)]),

@@ -415,9 +415,8 @@ __device__ __forceinline__ Tap make_tap(double sx, double sy, int status, int W,
     if (status != ACM_POINT_OK) return t;
     if (isnan(sx) || isnan(sy)) return t;
     if (interp == ACM_INTERP_NEAREST) {
-        double rx = round(sx), ry = round(sy);
-        // `as i32` saturates; anything outside [0,W) fails the guard either way
-        if (rx >= 0.0 && rx < (double)W && ry >= 0.0 && ry < (double)H) { t.ok = 1; t.off00 = 3 * ((int)ry * W + (int)rx); }
+        double rx, ry;
+        if (acm_nearest_pixel(sx, sy, W, H, rx, ry)) { t.ok = 1; t.off00 = 3 * ((int)ry * W + (int)rx); }
         return t;
     }
     double x0 = floor(sx), y0 = floor(sy);
@@ -1134,12 +1133,11 @@ __global__ void __launch_bounds__(256) remap_map_kernel(const __grid_constant__ 
     const int uo = (int)(i % W), vo = (int)(i / W);
     double x, y, z, sx, sy;
     int st = CamModel<MO>::template unproject<true>(co, (double)uo, (double)vo, x, y, z);
-    if (rotated && st == ACM_POINT_OK) {  // ray_in[k] = (R[0][k] x + R[1][k] y) + R[2][k] z, each operation rounded (-fmad=false)
-        const double* r = R.r;
-        const double xi = (r[0] * x + r[3] * y) + r[6] * z;
-        const double yi = (r[1] * x + r[4] * y) + r[7] * z;
-        const double zi = (r[2] * x + r[5] * y) + r[8] * z;
-        x = xi; y = yi; z = zi;
+    if (rotated && st == ACM_POINT_OK) {  // ray_in = R^T ray_out (acm_rot_t)
+        const double ro[3] = {x, y, z};
+        double ri[3];
+        acm_rot_t(R.r, ro, ri);
+        x = ri[0]; y = ri[1]; z = ri[2];
     }
     if (st == ACM_POINT_OK) st = CamModel<MI>::template project<true>(ci, x, y, z, sx, sy);
     if (st != ACM_POINT_OK) sx = sy = acm_nan();

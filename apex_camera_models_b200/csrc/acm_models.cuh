@@ -18,6 +18,25 @@ __device__ __forceinline__ bool acm_outside(const CamParams& c, double u, double
     return u < 0.0 || u >= c.W || v < 0.0 || v >= c.H;
 }
 
+// Rigid transforms with R row-major, every operation separately rounded in the including unit (-fmad=false there):
+//   acm_rigid_apply:  Y = R X + t,   Y[i] = ((R[i][0] X0 + R[i][1] X1) + R[i][2] X2) + t[i]
+//   acm_rot_t:        Y = R^T X,     Y[k] = (R[0][k] X0 + R[1][k] X1) + R[2][k] X2
+__device__ __forceinline__ void acm_rigid_apply(const double* R, const double* t, const double* X, double* Y) {
+#pragma unroll
+    for (int i = 0; i < 3; ++i) Y[i] = ((R[3 * i] * X[0] + R[3 * i + 1] * X[1]) + R[3 * i + 2] * X[2]) + t[i];
+}
+__device__ __forceinline__ void acm_rot_t(const double* R, const double* X, double* Y) {
+#pragma unroll
+    for (int k = 0; k < 3; ++k) Y[k] = (R[k] * X[0] + R[3 + k] * X[1]) + R[6 + k] * X[2];
+}
+
+// The nearest-pixel rule of undistort.rs:79-90: rx = round(sx), ry = round(sy) (half away from zero); true when the pixel lies
+// inside [0,W) x [0,H) (NaN fails).  `as i32` saturates in the reference; anything outside [0,W) fails the guard either way.
+__device__ __forceinline__ bool acm_nearest_pixel(double sx, double sy, int W, int H, double& rx, double& ry) {
+    rx = round(sx); ry = round(sy);
+    return rx >= 0.0 && rx < (double)W && ry >= 0.0 && ry < (double)H;
+}
+
 // nalgebra normalize(): n = sqrt((x*x + y*y) + z*z), each component divided by n
 __device__ __forceinline__ void acm_normalize_ieee(double x, double y, double z, double& ox, double& oy, double& oz) {
     double n = sqrt(x * x + y * y + z * z);

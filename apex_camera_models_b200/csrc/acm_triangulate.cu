@@ -38,11 +38,7 @@ template <int M1, int M2> struct TriPair {
     const TriRig& g;
     double u1, v1, u2, v2;
 
-    // Y = R X + t, Y[i] = ((R[i][0] X0 + R[i][1] X1) + R[i][2] X2) + t[i]
-    __device__ __forceinline__ void to_second(const double* X, double* Y) const {
-#pragma unroll
-        for (int i = 0; i < 3; ++i) Y[i] = ((g.R[3 * i] * X[0] + g.R[3 * i + 1] * X[1]) + g.R[3 * i + 2] * X[2]) + g.t[i];
-    }
+    __device__ __forceinline__ void to_second(const double* X, double* Y) const { acm_rigid_apply(g.R, g.t, X, Y); }
     // the four pixel residuals at X; false when X does not project (geometric validity) into both cameras
     __device__ __forceinline__ bool residuals(const double* X, double* r, double& cost) const {
         double pu, pv, qu, qv, Y[3];
@@ -86,8 +82,7 @@ __device__ __forceinline__ int tri_one(const TriPair<M1, M2>& P, const LinParams
     if (CamModel<M1>::template unproject<true>(P.ca, P.u1, P.v1, d1[0], d1[1], d1[2]) != ACM_POINT_OK) return ACM_TRI_UNPROJECT_FIRST;
     if (CamModel<M2>::template unproject<true>(P.cb, P.u2, P.v2, d2[0], d2[1], d2[2]) != ACM_POINT_OK) return ACM_TRI_UNPROJECT_SECOND;
     double e[3];  // d2' = R^T d2
-#pragma unroll
-    for (int k = 0; k < 3; ++k) e[k] = (g.R[k] * d2[0] + g.R[3 + k] * d2[1]) + g.R[6 + k] * d2[2];
+    acm_rot_t(g.R, d2, e);
     const double b = (d1[0] * e[0] + d1[1] * e[1]) + d1[2] * e[2];
     const double p = (d1[0] * c2[0] + d1[1] * c2[1]) + d1[2] * c2[2];
     const double q = (e[0] * c2[0] + e[1] * c2[1]) + e[2] * c2[2];
@@ -154,8 +149,9 @@ __global__ void __launch_bounds__(256) triangulate_kernel(const __grid_constant_
                                                           const __grid_constant__ TriRig g, const __grid_constant__ TriIO io, int max_iterations,
                                                           size_t n) {
     double c2[3];  // c2 = -R^T t, the second camera's centre in the first camera's frame (same order as d2')
+    acm_rot_t(g.R, g.t, c2);
 #pragma unroll
-    for (int k = 0; k < 3; ++k) c2[k] = -((g.R[k] * g.t[0] + g.R[3 + k] * g.t[1]) + g.R[6 + k] * g.t[2]);
+    for (int k = 0; k < 3; ++k) c2[k] = -c2[k];
     const size_t stride = (size_t)gridDim.x * blockDim.x;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
         const size_t j = i * io.in_stride;

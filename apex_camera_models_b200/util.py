@@ -1,7 +1,8 @@
 """util hot loops of the reference: undistort_image (src/util/undistort.rs:14-105), sample_points
 (src/util/point_sampling.rs:46-120), compute_reprojection_error (src/util/error_metrics.rs:62-121); and remap plans
 (camera-to-camera image remap, composed of the reference's unproject, project and interpolate_pixel), rotated plans,
-stereo rectification and triangulation of matched pixels of a calibrated pair."""
+stereo rectification, triangulation of matched pixels of a calibrated pair, and depth images (a point cloud rendered into a
+camera's range image, and a range image back-projected into points)."""
 from __future__ import annotations
 
 import ctypes as C
@@ -378,3 +379,80 @@ def triangulate_points(first: CameraModel, second: CameraModel, R, t, points1, p
                                         uv2.ctypes.data_as(C.c_void_p), n, int(max_iterations), xyz.ctypes.data_as(C.c_void_p),
                                         err.ctypes.data_as(C.c_void_p), st.ctypes.data_as(C.c_void_p)))
     return xyz, err, st
+
+
+class DepthStatus(enum.IntEnum):
+    """Per-pixel status of `depth_to_points` (include/acm.h ACM_DEPTH_*)."""
+    Ok = N.DEPTH_OK
+    Empty = N.DEPTH_EMPTY            # the range is not finite or <= 0 (an empty pixel of `render_depth`)
+    Unproject = N.DEPTH_UNPROJECT    # the model's unproject of the pixel centre failed
+
+
+def _pose_arrays(R, t):
+    """R = None: identity; t = None: zero."""
+    return _rotation_array(np.eye(3) if R is None else R), _translation_array(np.zeros(3) if t is None else t)
+
+
+def render_depth(model: CameraModel, points, R=None, t=None):
+    """Z-buffered range image of world points seen by `model`'s camera, x_cam = R x + t (R = None: identity, t = None: zero).
+
+    points: (N, 3) world points (a numpy array or device `Points`), N < 2^32 - 1.  A point is drawn into pixel
+    (round(u), round(v)) (half away from zero, the nearest rule of `undistort_image`) when the model projects x_cam (geometric
+    validity, any field of view, including rays beyond 90 degrees), the pixel lies inside the image and its range
+    |x_cam| is finite and > 0.  Per pixel the nearest point in float32 range wins and ties go to the lower index, so the
+    result does not depend on scheduling.  Depth is the RANGE along the ray, not z: z = range * ray_z.
+
+    Returns (range (H, W) float32, NaN where empty; index (H, W) uint32 of the winning point, 0xFFFFFFFF where empty),
+    H x W = the model's resolution.  Always numpy."""
+    if model is None:
+        raise UtilError("Camera model does not exist")
+    ctx = model.ctx
+    Rm, tv = _pose_arrays(R, t)
+    cam = model.camera_block()
+    res = model.get_resolution()
+    rng, idx = np.empty((res.height, res.width), np.float32), np.empty((res.height, res.width), np.uint32)
+    if isinstance(points, Points):
+        npix = res.width * res.height
+        d = ctx.device_alloc(max(npix, 1) * 8)  # range row, then index row
+        try:
+            ctx.check(_lib.acm_render_depth(ctx.handle, C.byref(cam), Rm, tv, points.handle, C.c_void_p(d), C.c_void_p(d + 4 * npix)))
+            ctx.d2h(rng, d); ctx.d2h(idx, d + 4 * npix)
+            ctx.sync()
+        finally:
+            ctx.device_free(d)
+        return rng, idx
+    xyz = np.ascontiguousarray(points, dtype=np.float64).reshape(-1, 3)
+    ctx.check(_lib.acm_render_depth_host(ctx.handle, C.byref(cam), Rm, tv, xyz.ctypes.data_as(C.c_void_p), len(xyz),
+                                         rng.ctypes.data_as(C.c_void_p), idx.ctypes.data_as(C.c_void_p)))
+    return rng, idx
+
+
+def depth_to_points(model: CameraModel, range_image, R=None, t=None):
+    """Back-projection of a (H, W) range image of `model`'s camera (H x W = its resolution) into world points, x_cam = R x + t
+    as in `render_depth`: pixel (c, r) with a finite range d > 0 gives x = R^T (unproject((c, r)) * d - t), the ray of the
+    integer pixel centre (IEEE unproject, with the model's pixel-bounds test).
+
+    Returns (points (H, W, 3) float64, NaN where the status is not Ok; status (H, W) uint8 of `DepthStatus`)."""
+    if model is None:
+        raise UtilError("Camera model does not exist")
+    ctx = model.ctx
+    Rm, tv = _pose_arrays(R, t)
+    cam = model.camera_block()
+    res = model.get_resolution()
+    r = np.ascontiguousarray(range_image, dtype=np.float32)
+    if r.shape != (res.height, res.width):
+        raise UtilError(f"Invalid parameters: range image {r.shape} doesn't match model {res.height}x{res.width} (H, W)")
+    npix = res.width * res.height
+    xyz = Points(ctx, 3, npix)
+    d = ctx.device_alloc(max(npix, 1) * 5)  # range, then the status bytes
+    try:
+        ctx.h2d(d, r)
+        ctx.check(_lib.acm_depth_to_points(ctx.handle, C.byref(cam), Rm, tv, C.c_void_p(d), xyz.handle, C.c_void_p(d + 4 * npix)))
+        st = np.empty((res.height, res.width), np.uint8)
+        ctx.d2h(st, d + 4 * npix)
+        ctx.sync()
+        pts = xyz.numpy().reshape(res.height, res.width, 3)
+    finally:
+        ctx.device_free(d)
+        xyz.free()
+    return pts, st

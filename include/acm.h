@@ -316,6 +316,43 @@ int32_t acm_triangulate_host(acm_ctx* ctx, const acm_camera* first, const acm_ca
                              const double* uv1_aos, const double* uv2_aos, size_t n, int32_t max_iterations,
                              double* xyz_aos, double* err, uint8_t* status);
 
+/* ---- depth images: render a point cloud, back-project a depth image (beyond the reference) -----
+ * The camera's resolution W x H is the image (width and height in [1, 2^31 - 1]); images are row-major, pixel (c, r) at r*W + c.
+ * Render: x_cam = R x + t (R row-major, x_cam[i] = ((R[i][0] x + R[i][1] y) + R[i][2] z) + t[i], each operation rounded, as
+ * acm_triangulate's second camera).  Point i is drawn when, in this order:
+ *   1. cam.project(x_cam) is Ok with geometric validity only (no image-bounds test, like acm_project_point_jacobian);
+ *   2. rx = round(u), ry = round(v) (half away from zero: the nearest rule of undistort_image) satisfy 0 <= rx < W and
+ *      0 <= ry < H (NaN fails);
+ *   3. range = sqrt((xc*xc + yc*yc) + zc*zc) is finite and > 0.
+ * Depth is the RANGE along the ray, not z: the fisheye models see rays beyond 90 degrees, where z <= 0; z = range * ray_z.
+ * Per pixel the key (uint64)bits((float)range) << 32 | i ((float): round to nearest; ranges above FLT_MAX become +inf and
+ * are still drawn) is reduced by atomicMin: the nearest point in f32 range wins, ties go to the lowest index, and the image
+ * does not depend on scheduling.  d_range (W*H floats) receives the winner's f32 range, d_index (W*H uint32) its index; an
+ * empty pixel holds the all-ones key split the same way: range bits 0xFFFFFFFF (a NaN) and index UINT32_MAX.
+ * xyz: dim-3 f64 buffer of n < 2^32 - 1 world points.  R must be a rotation (the check of acm_remap_plan_create_rotated) and
+ * t finite (zero allowed).  The key image (8 bytes per pixel) lives in the context's scratch arena.  One memset and one
+ * resolve kernel per call, plus one render kernel when n > 0.  ACM_ERR_INVALID_ARG for a null camera / buffer, a camera
+ * without a resolution, a dimension / dtype mismatch, a bad R or t, or n >= 2^32 - 1 (checked before anything is allocated). */
+int32_t acm_render_depth(acm_ctx* ctx, const acm_camera* cam, const double R[9], const double t[3], const acm_points* xyz,
+                         float* d_range, uint32_t* d_index);
+/* synchronous host form: n AoS points (xyzxyz...) staged in the scratch arena; range / index: W*H host elements; the same
+ * kernels, so the same bytes as acm_render_depth */
+int32_t acm_render_depth_host(acm_ctx* ctx, const acm_camera* cam, const double R[9], const double t[3], const double* xyz_aos,
+                              size_t n, float* range, uint32_t* index);
+/* Back-project: pixel (c, r) with range d = d_range[r*W + c]: EMPTY unless d is finite and > 0; ray = cam.unproject((c, r))
+ * at the integer pixel centre in the IEEE form of acm_unproject_ieee (with its pixel-bounds test), UNPROJECT when it fails;
+ * x_cam = ray * (double)d, then x = R^T (x_cam - t) with x[k] = (R[0][k] q0 + R[1][k] q1) + R[2][k] q2, q = x_cam - t (the
+ * rotated remap's order), so that a render followed by a back-projection with the same R, t stays in the world frame.
+ * xyz: dim-3 f64 buffer of W*H points in pixel order, NaN where the status is not OK; d_status (optional): ACM_DEPTH_* per
+ * pixel.  One kernel. */
+enum {
+    ACM_DEPTH_OK = 0,
+    ACM_DEPTH_EMPTY = 1,      /* range not finite or <= 0 (an empty pixel of acm_render_depth) */
+    ACM_DEPTH_UNPROJECT = 2   /* cam.unproject((c, r)) failed (outside the UCM / EUCM / DS domain, KB not converged, ...) */
+};
+int32_t acm_depth_to_points(acm_ctx* ctx, const acm_camera* cam, const double R[9], const double t[3], const float* d_range,
+                            acm_points* xyz, uint8_t* d_status);
+
 /* util::compute_reprojection_error (reference src/util/error_metrics.rs:62-121) */
 typedef struct acm_projection_error {
     double rmse, min, max, mean, stddev, median;

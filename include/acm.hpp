@@ -432,6 +432,55 @@ inline Triangulation triangulate(const CameraModel& first, const CameraModel& se
     return out;
 }
 
+// Depth images of `cam`'s camera (W x H = its resolution, row-major), x_cam = R x + t (acm_render_depth_host): per pixel the
+// f32 range |x_cam| of the nearest drawn point and its index; empty pixels hold range bits 0xFFFFFFFF (a NaN) and index
+// UINT32_MAX.  Depth is the range along the ray, not z.
+struct DepthImage {
+    std::vector<float> range;
+    std::vector<uint32_t> index;
+};
+
+inline DepthImage render_depth(const CameraModel& cam, const std::array<double, 9>& R, const std::array<double, 3>& t,
+                               const double* xyz_aos, size_t n) {
+    DepthImage out;
+    const size_t npix = (size_t)cam.resolution.width * cam.resolution.height;
+    out.range.resize(npix); out.index.resize(npix);
+    const acm_camera c = cam.block();
+    cam.ctx().check(acm_render_depth_host(cam.ctx().handle(), &c, R.data(), t.data(), xyz_aos, n, out.range.data(), out.index.data()));
+    return out;
+}
+
+// Back-projection of a W x H range image (acm_depth_to_points): x = R^T (unproject(pixel) * range - t) per pixel (Matrix3xX
+// memory order, NaN where status != ACM_DEPTH_OK) and the ACM_DEPTH_* status.
+struct DepthPoints {
+    std::vector<double> points;
+    std::vector<uint8_t> status;
+};
+
+inline DepthPoints depth_to_points(const CameraModel& cam, const std::array<double, 9>& R, const std::array<double, 3>& t, const float* range) {
+    const Context& ctx = cam.ctx();
+    const size_t npix = (size_t)cam.resolution.width * cam.resolution.height;
+    void* d = nullptr;  // range, then the status bytes
+    ctx.check(acm_device_alloc(ctx.handle(), npix ? 5 * npix : 5, &d));
+    DepthPoints out;
+    try {
+        Points X(ctx, 3, npix);
+        ctx.check(acm_memcpy_h2d(ctx.handle(), d, range, 4 * npix));
+        const acm_camera c = cam.block();
+        uint8_t* d_status = static_cast<uint8_t*>(d) + 4 * npix;
+        ctx.check(acm_depth_to_points(ctx.handle(), &c, R.data(), t.data(), static_cast<const float*>(d), X.handle(), d_status));
+        out.status.resize(npix);
+        ctx.check(acm_memcpy_d2h(ctx.handle(), out.status.data(), d_status, npix));
+        out.points = X.download();
+        ctx.sync();
+    } catch (...) {
+        acm_device_free(ctx.handle(), d);
+        throw;
+    }
+    acm_device_free(ctx.handle(), d);
+    return out;
+}
+
 // ---- util::image_quality (image_quality.rs) on RGB8 interleaved images (w*h*3 bytes) --------------
 struct ImageQualityMetrics { double psnr, ssim; };   // image_quality.rs:20-26
 

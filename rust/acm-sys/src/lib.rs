@@ -34,6 +34,9 @@ pub const ACM_TRI_PARALLEL_EPS: f64 = 1e-12;
 pub const ACM_TRI_LAMBDA0: f64 = 1e-3;
 pub const ACM_TRI_LAMBDA_FACTOR: f64 = 10.0;
 pub const ACM_TRI_STEP_TOL: f64 = 1e-12;
+pub const ACM_DEPTH_OK: u8 = 0;
+pub const ACM_DEPTH_EMPTY: u8 = 1;
+pub const ACM_DEPTH_UNPROJECT: u8 = 2;
 
 #[repr(C)]
 pub struct acm_ctx { _private: [u8; 0] }
@@ -173,6 +176,9 @@ extern "C" {
     pub fn acm_stereo_rectify(r: *const f64, t: *const f64, r1: *mut f64, r2: *mut f64, baseline: *mut f64, vertical: *mut i32) -> i32;
     pub fn acm_triangulate(ctx: *mut acm_ctx, first: *const acm_camera, second: *const acm_camera, r: *const f64, t: *const f64, uv1: *const acm_points, uv2: *const acm_points, max_iterations: i32, xyz: *mut acm_points, d_err: *mut f64, d_status: *mut u8) -> i32;
     pub fn acm_triangulate_host(ctx: *mut acm_ctx, first: *const acm_camera, second: *const acm_camera, r: *const f64, t: *const f64, uv1_aos: *const f64, uv2_aos: *const f64, n: size_t, max_iterations: i32, xyz_aos: *mut f64, err: *mut f64, status: *mut u8) -> i32;
+    pub fn acm_render_depth(ctx: *mut acm_ctx, cam: *const acm_camera, r: *const f64, t: *const f64, xyz: *const acm_points, d_range: *mut f32, d_index: *mut u32) -> i32;
+    pub fn acm_render_depth_host(ctx: *mut acm_ctx, cam: *const acm_camera, r: *const f64, t: *const f64, xyz_aos: *const f64, n: size_t, range: *mut f32, index: *mut u32) -> i32;
+    pub fn acm_depth_to_points(ctx: *mut acm_ctx, cam: *const acm_camera, r: *const f64, t: *const f64, d_range: *const f32, xyz: *mut acm_points, d_status: *mut u8) -> i32;
 
     pub fn acm_reprojection_error(ctx: *mut acm_ctx, cam: *const acm_camera, xyz: *const acm_points, uv: *const acm_points, out: *mut acm_projection_error) -> i32;
     pub fn acm_sample_points(ctx: *mut acm_ctx, cam: *const acm_camera, n_requested: size_t, uv_out: *mut *mut acm_points, xyz_out: *mut *mut acm_points, n_kept: *mut size_t) -> i32;

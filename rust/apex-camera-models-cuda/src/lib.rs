@@ -358,6 +358,55 @@ impl<M: CameraModel> GpuCamera<M> {
         Ok((xyz, err, status))
     }
 
+    /// Z-buffered range image of world points `xyz` seen by this camera, x_cam = R x + t with `r` row-major: per pixel
+    /// (row-major, W x H = the camera's resolution) the f32 range |x_cam| of the nearest point drawn there and its index
+    /// (ties: the lower index); empty pixels hold range bits 0xFFFFFFFF (a NaN) and index u32::MAX.  Depth is the range
+    /// along the ray, not z.
+    pub fn render_depth(&self, r: &[f64; 9], t: &[f64; 3], xyz: &Matrix3xX<f64>) -> Result<(Vec<f32>, Vec<u32>), CameraModelError> {
+        let res = self.inner.get_resolution();
+        let npix = res.width as usize * res.height as usize;
+        let cam = self.block();
+        let (mut range, mut index) = (vec![0f32; npix], vec![0u32; npix]);
+        let _g = self.ctx.lock();
+        let rc = unsafe {
+            sys::acm_render_depth_host(self.ctx.0, &cam, r.as_ptr(), t.as_ptr(), xyz.as_ptr(), xyz.ncols(), range.as_mut_ptr(), index.as_mut_ptr())
+        };
+        if rc != sys::ACM_OK { return Err(self.ctx.err(rc)); }
+        Ok((range, index))
+    }
+
+    /// Back-projection of a W x H range image of this camera (row-major): x = R^T (unproject(pixel) * range - t) per pixel,
+    /// NaN where the status is not `ACM_DEPTH_OK`, and the `ACM_DEPTH_*` status per pixel.
+    pub fn depth_to_points(&self, r: &[f64; 9], t: &[f64; 3], range: &[f32]) -> Result<(Matrix3xX<f64>, Vec<u8>), CameraModelError> {
+        let res = self.inner.get_resolution();
+        let npix = res.width as usize * res.height as usize;
+        if range.len() != npix {
+            return Err(CameraModelError::InvalidParams(format!("range image has {} pixels, the camera {}", range.len(), npix)));
+        }
+        let cam = self.block();
+        let mut xyz = Matrix3xX::<f64>::zeros(npix);
+        let mut status = vec![0u8; npix];
+        let _g = self.ctx.lock();
+        let mut h = ptr::null_mut();
+        let mut rc = unsafe { sys::acm_points_create(self.ctx.0, 3, npix, sys::ACM_F64, &mut h) };
+        if rc != sys::ACM_OK { return Err(self.ctx.err(rc)); }
+        let pts = DevicePoints::adopt(&self.ctx, h);
+        let mut d: *mut std::ffi::c_void = ptr::null_mut();  // range, then the status bytes
+        rc = unsafe { sys::acm_device_alloc(self.ctx.0, 5 * npix.max(1), &mut d) };
+        if rc != sys::ACM_OK { return Err(self.ctx.err(rc)); }
+        unsafe {
+            let ds = (d as *mut u8).add(4 * npix);
+            rc = sys::acm_memcpy_h2d(self.ctx.0, d, range.as_ptr() as *const _, 4 * npix);
+            if rc == sys::ACM_OK { rc = sys::acm_depth_to_points(self.ctx.0, &cam, r.as_ptr(), t.as_ptr(), d as *const f32, pts.h, ds); }
+            if rc == sys::ACM_OK { rc = sys::acm_memcpy_d2h(self.ctx.0, status.as_mut_ptr() as *mut _, ds as *const _, npix); }
+            if rc == sys::ACM_OK { rc = sys::acm_points_download_aos_f64(self.ctx.0, pts.h, xyz.as_mut_ptr(), npix); }
+            if rc == sys::ACM_OK { rc = sys::acm_ctx_sync(self.ctx.0); }
+            sys::acm_device_free(self.ctx.0, d);
+        }
+        if rc != sys::ACM_OK { return Err(self.ctx.err(rc)); }
+        Ok((xyz, status))
+    }
+
     /// README-era `project(&p, compute_jacobian = true)`: uv plus the 2xP Jacobian w.r.t. `[fx, fy, cx, cy, dist..]`
     /// (per-model docs, double_sphere.rs:326-332) and the 2x3 Jacobian w.r.t. the 3-D point (trait doc, mod.rs:246-252).
     pub fn project_with_jacobians(&self, p: &Vector3<f64>)
