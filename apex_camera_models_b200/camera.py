@@ -197,11 +197,8 @@ class CameraModel:
         ctx = self.ctx
         cam = self.camera_block()
         if isinstance(points_3d, Points):
-            n = len(points_3d)
-            uv = Points(ctx, 2, n, points_3d.dtype)
-            st = ctx.device_alloc(max(n, 1))
-            ctx.check(_lib.acm_project(ctx.handle, C.byref(cam), points_3d.handle, uv.handle, C.c_void_p(st)))
-            return uv, st
+            with ctx.staging() as s:
+                return s.keep(*self._map_points(s, points_3d, len(points_3d), 2, _lib.acm_project))
         a = np.ascontiguousarray(points_3d, dtype=np.float64).reshape(-1, 3)
         n = a.shape[0]
         if dtype == N.F64:
@@ -215,11 +212,8 @@ class CameraModel:
         ctx = self.ctx
         cam = self.camera_block()
         if isinstance(points_2d, Points):
-            n = len(points_2d)
-            xyz = Points(ctx, 3, n, points_2d.dtype)
-            st = ctx.device_alloc(max(n, 1))
-            ctx.check(_lib.acm_unproject(ctx.handle, C.byref(cam), points_2d.handle, xyz.handle, C.c_void_p(st)))
-            return xyz, st
+            with ctx.staging() as s:
+                return s.keep(*self._map_points(s, points_2d, len(points_2d), 3, _lib.acm_unproject))
         a = np.ascontiguousarray(points_2d, dtype=np.float64).reshape(-1, 2)
         n = a.shape[0]
         if dtype == N.F64:
@@ -235,20 +229,24 @@ class CameraModel:
         a = np.ascontiguousarray(points_2d, dtype=np.float64).reshape(-1, 2)
         return self._host_map_via_points(a, 2, 3, _lib.acm_unproject_ieee, N.F64)
 
+    def _map_points(self, s, src, n, dout, fn):
+        """`fn` (acm_project / acm_unproject / acm_unproject_ieee) of the n device points `src`: (dst `Points`, status
+        pointer), both owned by `s`."""
+        ctx = self.ctx
+        dst, st = s.own(Points(ctx, dout, n, src.dtype)), s.alloc(n)
+        ctx.check(fn(ctx.handle, C.byref(self.camera_block()), src.handle, dst.handle, C.c_void_p(st)))
+        return dst, st
+
     def _host_map_via_points(self, a, din, dout, fn, dtype):
         ctx = self.ctx
-        cam = self.camera_block()
         n = a.shape[0]
-        src = Points.from_numpy(ctx, a, dtype)
-        dst = Points(ctx, dout, n, dtype)
-        st_d = ctx.device_alloc(max(n, 1))
-        ctx.check(fn(ctx.handle, C.byref(cam), src.handle, dst.handle, C.c_void_p(st_d)))
-        out = dst.numpy()
-        st = np.empty(n, dtype=np.uint8)
-        if n:
-            ctx.d2h(st, st_d)
-        ctx.sync()
-        ctx.device_free(st_d); src.free(); dst.free()
+        with ctx.staging() as s:
+            dst, st_d = self._map_points(s, s.points(a, din, dtype), n, dout, fn)
+            out = dst.numpy()
+            st = np.empty(n, dtype=np.uint8)
+            if n:
+                ctx.d2h(st, st_d)
+            ctx.sync()
         return out, st
 
     def round_trip_batch(self, points_3d, dtype: int = N.F64):
@@ -256,60 +254,46 @@ class CameraModel:
         Host (N,3) array in -> numpy out; device `Points` in -> (Points, Points, status ptr, status ptr)."""
         ctx = self.ctx
         cam = self.camera_block()
-        on_device = isinstance(points_3d, Points)
-        src = points_3d if on_device else Points.from_numpy(ctx, np.ascontiguousarray(points_3d, dtype=np.float64).reshape(-1, 3), dtype)
-        n = len(src)
-        uv, ray = Points(ctx, 2, n, src.dtype), Points(ctx, 3, n, src.dtype)
-        sp, su = ctx.device_alloc(max(n, 1)), ctx.device_alloc(max(n, 1))
-        ctx.check(_lib.acm_project_unproject(ctx.handle, C.byref(cam), src.handle, uv.handle, ray.handle, C.c_void_p(sp), C.c_void_p(su)))
-        if on_device:
-            return uv, ray, sp, su
-        a, b = uv.numpy(), ray.numpy()
-        s1, s2 = np.empty(n, dtype=np.uint8), np.empty(n, dtype=np.uint8)
-        if n:
-            ctx.d2h(s1, sp); ctx.d2h(s2, su)
-        ctx.sync()
-        ctx.device_free(sp); ctx.device_free(su); src.free(); uv.free(); ray.free()
+        with ctx.staging() as s:
+            src = s.points(points_3d, 3, dtype)
+            n = len(src)
+            uv, ray = s.own(Points(ctx, 2, n, src.dtype)), s.own(Points(ctx, 3, n, src.dtype))
+            sp, su = s.alloc(n), s.alloc(n)
+            ctx.check(_lib.acm_project_unproject(ctx.handle, C.byref(cam), src.handle, uv.handle, ray.handle, C.c_void_p(sp), C.c_void_p(su)))
+            if isinstance(points_3d, Points):
+                return s.keep(uv, ray, sp, su)
+            a, b = uv.numpy(), ray.numpy()
+            s1, s2 = np.empty(n, dtype=np.uint8), np.empty(n, dtype=np.uint8)
+            if n:
+                ctx.d2h(s1, sp); ctx.d2h(s2, su)
+            ctx.sync()
         return a, b, s1, s2
 
-    def project_jacobian_batch(self, points_3d):
-        """uv (N,2), J (N,2,P) w.r.t. [fx,fy,cx,cy,dist..], status (N,); geometric validity only."""
-        ctx = self.ctx
-        cam = self.camera_block()
-        a = np.ascontiguousarray(points_3d, dtype=np.float64).reshape(-1, 3)
-        n, P = a.shape[0], cam.n_params
-        src = Points.from_numpy(ctx, a)
-        uv = Points(ctx, 2, n)
-        d_j = ctx.device_alloc(max(n, 1) * 2 * P * 8)
-        d_s = ctx.device_alloc(max(n, 1))
-        ctx.check(_lib.acm_project_jacobian(ctx.handle, C.byref(cam), src.handle, uv.handle, C.c_void_p(d_j), C.c_void_p(d_s)))
-        J = np.empty((2 * P, n)); st = np.empty(n, dtype=np.uint8)
-        if n:
-            ctx.d2h(J, d_j); ctx.d2h(st, d_s)
-        ctx.sync()
-        out = uv.numpy()
-        ctx.device_free(d_j); ctx.device_free(d_s); src.free(); uv.free()
-        return out, np.ascontiguousarray(J.reshape(2, P, n).transpose(2, 0, 1)), st
-
-    def project_point_jacobian_batch(self, points_3d):
-        """uv (N,2), J (N,2,3) = d(u,v)/d(x,y,z) -- the trait doc's "Jacobian matrix (2x3)" (mod.rs:246-252) --,
-        status (N,); geometric validity only, J = 0 where the projection fails."""
+    def _jacobian_batch(self, points_3d, fn, rows: int):
+        """uv (N,2), J (N,2,rows/2) written by `fn` as `rows` rows of N, status (N,)."""
         ctx = self.ctx
         cam = self.camera_block()
         a = np.ascontiguousarray(points_3d, dtype=np.float64).reshape(-1, 3)
         n = a.shape[0]
-        src = Points.from_numpy(ctx, a)
-        uv = Points(ctx, 2, n)
-        d_j = ctx.device_alloc(max(n, 1) * 6 * 8)
-        d_s = ctx.device_alloc(max(n, 1))
-        ctx.check(_lib.acm_project_point_jacobian(ctx.handle, C.byref(cam), src.handle, uv.handle, C.c_void_p(d_j), C.c_void_p(d_s)))
-        J = np.empty((6, n)); st = np.empty(n, dtype=np.uint8)
-        if n:
-            ctx.d2h(J, d_j); ctx.d2h(st, d_s)
-        ctx.sync()
-        out = uv.numpy()
-        ctx.device_free(d_j); ctx.device_free(d_s); src.free(); uv.free()
-        return out, np.ascontiguousarray(J.reshape(2, 3, n).transpose(2, 0, 1)), st
+        with ctx.staging() as s:
+            src, uv = s.points(a, 3), s.own(Points(ctx, 2, n))
+            d_j, d_s = s.alloc(n * rows * 8), s.alloc(n)
+            ctx.check(fn(ctx.handle, C.byref(cam), src.handle, uv.handle, C.c_void_p(d_j), C.c_void_p(d_s)))
+            J = np.empty((rows, n)); st = np.empty(n, dtype=np.uint8)
+            if n:
+                ctx.d2h(J, d_j); ctx.d2h(st, d_s)
+            ctx.sync()
+            out = uv.numpy()
+        return out, np.ascontiguousarray(J.reshape(2, rows // 2, n).transpose(2, 0, 1)), st
+
+    def project_jacobian_batch(self, points_3d):
+        """uv (N,2), J (N,2,P) w.r.t. [fx,fy,cx,cy,dist..], status (N,); geometric validity only."""
+        return self._jacobian_batch(points_3d, _lib.acm_project_jacobian, 2 * len(self.params()))
+
+    def project_point_jacobian_batch(self, points_3d):
+        """uv (N,2), J (N,2,3) = d(u,v)/d(x,y,z) -- the trait doc's "Jacobian matrix (2x3)" (mod.rs:246-252) --,
+        status (N,); geometric validity only, J = 0 where the projection fails."""
+        return self._jacobian_batch(points_3d, _lib.acm_project_point_jacobian, 6)
 
     # ---- trait: scalar project / unproject ---------------------------------------------------
     def project(self, point_3d, compute_jacobian=False):
@@ -337,19 +321,10 @@ class CameraModel:
     def linear_estimation(self, points_3d, points_2d):
         """`linear_estimation(&mut self, &Matrix3xX, &Matrix2xX)`; updates the distortion part."""
         ctx = self.ctx
-        own = []
-        def dev(a, dim):
-            if isinstance(a, Points):
-                return a
-            p = Points.from_numpy(ctx, np.ascontiguousarray(a, dtype=np.float64).reshape(-1, dim))
-            own.append(p)
-            return p
-        X, UV = dev(points_3d, 3), dev(points_2d, 2)
         cam = self.camera_block()
-        rc = _lib.acm_linear_estimation(ctx.handle, C.byref(cam), X.handle, UV.handle)
-        for p in own:
-            p.free()
-        ctx.check(rc)
+        with ctx.staging() as s:
+            X, UV = s.points(points_3d, 3), s.points(points_2d, 2)
+            ctx.check(_lib.acm_linear_estimation(ctx.handle, C.byref(cam), X.handle, UV.handle))
         self.set_params(cam.params[: cam.n_params])
 
 

@@ -12,7 +12,7 @@ import numpy as np
 from . import _native as N
 from .camera import CameraModel
 from .errors import UtilError
-from .runtime import Context, Points, default_context
+from .runtime import Context, Staging, default_context
 
 _lib = N.lib
 
@@ -26,10 +26,10 @@ class ImageQualityMetrics:  # image_quality.rs:20-26
 
 
 class _DeviceImage:
-    """RGB8 image in HBM for the duration of a call."""
+    """RGB8 image in HBM, owned by the call's `Staging`."""
 
-    def __init__(self, ctx: Context, host: np.ndarray | None = None, shape=None):
-        self.ctx = ctx
+    def __init__(self, s: Staging, host: np.ndarray | None = None, shape=None):
+        self.ctx = ctx = s.ctx
         if host is not None:
             host = np.ascontiguousarray(host, dtype=np.uint8)
             if host.ndim != 3 or host.shape[2] != 3:
@@ -37,7 +37,7 @@ class _DeviceImage:
             shape = host.shape
         self.shape = tuple(shape)
         self.nbytes = int(np.prod(self.shape))
-        self.ptr = ctx.device_alloc(max(self.nbytes, 4))
+        self.ptr = s.alloc(max(self.nbytes, 4))
         if host is not None and self.nbytes:
             ctx.h2d(self.ptr, host)
         elif self.nbytes:
@@ -50,78 +50,52 @@ class _DeviceImage:
             self.ctx.sync()
         return out
 
-    def free(self):
-        if self.ptr:
-            self.ctx.device_free(self.ptr)
-            self.ptr = 0
 
-
-def _pair(img1, img2, ctx):
+def _compare(fn, img1, img2, ctx: Context | None) -> float:
+    """`fn` (acm_image_psnr / acm_image_ssim) of two same-shaped images staged on the device."""
     a, b = np.asarray(img1), np.asarray(img2)
     if a.shape != b.shape:  # image_quality.rs:46-50, :109-113
         raise UtilError("Invalid parameters: Images must have the same dimensions")
     ctx = ctx or default_context()
-    return ctx, _DeviceImage(ctx, a), _DeviceImage(ctx, b)
+    out = C.c_double()
+    with ctx.staging() as s:
+        d1, d2 = _DeviceImage(s, a), _DeviceImage(s, b)
+        ctx.check(fn(ctx.handle, C.c_void_p(d1.ptr), C.c_void_p(d2.ptr), d1.shape[1], d1.shape[0], C.byref(out)))
+    return float(out.value)
 
 
 def calculate_psnr(img1: np.ndarray, img2: np.ndarray, ctx: Context | None = None) -> float:
     """PSNR in dB over the pixels that are not black in both images; inf for a perfect match."""
-    ctx, d1, d2 = _pair(img1, img2, ctx)
-    try:
-        out = C.c_double()
-        ctx.check(_lib.acm_image_psnr(ctx.handle, C.c_void_p(d1.ptr), C.c_void_p(d2.ptr), d1.shape[1], d1.shape[0], C.byref(out)))
-        return float(out.value)
-    finally:
-        d1.free(); d2.free()
+    return _compare(_lib.acm_image_psnr, img1, img2, ctx)
 
 
 def calculate_ssim(img1: np.ndarray, img2: np.ndarray, ctx: Context | None = None) -> float:
     """Mean 3x3-window SSIM of the truncated-luma grey images (interior windows only)."""
-    ctx, d1, d2 = _pair(img1, img2, ctx)
-    try:
-        out = C.c_double()
-        ctx.check(_lib.acm_image_ssim(ctx.handle, C.c_void_p(d1.ptr), C.c_void_p(d2.ptr), d1.shape[1], d1.shape[0], C.byref(out)))
-        return float(out.value)
-    finally:
-        d1.free(); d2.free()
+    return _compare(_lib.acm_image_ssim, img1, img2, ctx)
 
 
-def _draw(ctx: Context, dimg: _DeviceImage, projections, color):
-    own = None
-    if isinstance(projections, Points):
-        pts = projections
-    else:
-        pts = own = Points.from_numpy(ctx, np.ascontiguousarray(projections, dtype=np.float64).reshape(-1, 2))
-    try:
-        ctx.check(_lib.acm_draw_points_rgb8(ctx.handle, pts.handle, None, color[0], color[1], color[2], C.c_void_p(dimg.ptr),
-                                            dimg.shape[1], dimg.shape[0]))
-    finally:
-        if own is not None:
-            own.free()
+def _draw(ctx: Context | None, layers, host: np.ndarray | None = None, shape=None) -> np.ndarray:
+    """Draws each (projections, color) of `layers` in turn on a device copy of `host` (or on black at `shape`) and returns
+    the image."""
+    ctx = ctx or default_context()
+    with ctx.staging() as s:
+        d = _DeviceImage(s, host, shape)
+        for projections, color in layers:
+            pts = s.points(projections, 2)
+            ctx.check(_lib.acm_draw_points_rgb8(ctx.handle, pts.handle, None, color[0], color[1], color[2], C.c_void_p(d.ptr),
+                                                d.shape[1], d.shape[0]))
+        return d.numpy()
 
 
 def create_projection_image(projections, color, width: int, height: int, ctx: Context | None = None) -> np.ndarray:
     """image_quality.rs:338-373 with one colour for every point: radius-2 discs on black."""
-    ctx = ctx or default_context()
-    d = _DeviceImage(ctx, shape=(height, width, 3))
-    try:
-        _draw(ctx, d, projections, color)
-        return d.numpy()
-    finally:
-        d.free()
+    return _draw(ctx, [(projections, color)], shape=(height, width, 3))
 
 
 def create_combined_projection_image_on_reference(input_projections, output_projections, reference_image: np.ndarray,
                                                   ctx: Context | None = None) -> np.ndarray:
     """image_quality.rs:389-437: green input discs, then magenta output discs, on a copy of the reference."""
-    ctx = ctx or default_context()
-    d = _DeviceImage(ctx, reference_image)
-    try:
-        _draw(ctx, d, input_projections, GREEN)
-        _draw(ctx, d, output_projections, MAGENTA)
-        return d.numpy()
-    finally:
-        d.free()
+    return _draw(ctx, [(input_projections, GREEN), (output_projections, MAGENTA)], reference_image)
 
 
 def create_combined_projection_image(input_projections, output_projections, width: int, height: int,
@@ -136,13 +110,7 @@ def model_projection_visualization(points_2d, reference_image: np.ndarray | None
     """image_quality.rs:553-616 without the file: green discs on the reference image, or on black at
     `camera_resolution = (width, height)`.  Returns the image the reference would save."""
     if reference_image is not None:
-        ctx = ctx or default_context()
-        d = _DeviceImage(ctx, reference_image)
-        try:
-            _draw(ctx, d, points_2d, GREEN)
-            return d.numpy()
-        finally:
-            d.free()
+        return _draw(ctx, [(points_2d, GREEN)], reference_image)
     return create_projection_image(points_2d, GREEN, camera_resolution[0], camera_resolution[1], ctx)
 
 
@@ -159,14 +127,10 @@ def compute_image_quality_metrics(input_model: CameraModel, output_model: Camera
     else:
         res = input_model.get_resolution()
         ref, width, height = None, res.width, res.height
-    own = None
-    if isinstance(optimization_points_3d, Points):
-        X = optimization_points_3d
-    else:
-        X = own = Points.from_numpy(ctx, np.ascontiguousarray(optimization_points_3d, dtype=np.float64).reshape(-1, 3))
-    dref = _DeviceImage(ctx, ref) if ref is not None else None
-    dcomb = _DeviceImage(ctx, shape=(height, width, 3)) if return_image else None
-    try:
+    with ctx.staging() as s:
+        X = s.points(optimization_points_3d, 3)
+        dref = _DeviceImage(s, ref) if ref is not None else None
+        dcomb = _DeviceImage(s, shape=(height, width, 3)) if return_image else None
         cin, cout = input_model.camera_block(), output_model.camera_block()
         out = N.ImageQuality()
         ctx.check(_lib.acm_image_quality_metrics(ctx.handle, C.byref(cin), C.byref(cout), X.handle, width, height,
@@ -174,10 +138,3 @@ def compute_image_quality_metrics(input_model: CameraModel, output_model: Camera
                                                  C.byref(out)))
         m = ImageQualityMetrics(float(out.psnr), float(out.ssim))
         return (m, dcomb.numpy()) if return_image else m
-    finally:
-        if own is not None:
-            own.free()
-        if dref:
-            dref.free()
-        if dcomb:
-            dcomb.free()

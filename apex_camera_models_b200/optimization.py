@@ -13,7 +13,6 @@ import numpy as np
 from . import _native as N
 from .camera import (CameraModel, DoubleSphereModel, EucmModel, FovModel, KannalaBrandtModel, RadTanModel, UcmModel)
 from .errors import InvalidParams
-from .runtime import Points
 
 _lib = N.lib
 
@@ -79,16 +78,10 @@ class OptimizationCost:
         if not isinstance(model, self.MODEL):
             raise InvalidParams(f"{type(self).__name__} needs a {self.MODEL.__name__}")
         self.model = model
-        ctx = model.ctx
-        self._own = []
-        def dev(a, dim):
-            if isinstance(a, Points):
-                return a
-            p = Points.from_numpy(ctx, np.ascontiguousarray(a, dtype=np.float64).reshape(-1, dim))
-            self._own.append(p)
-            return p
-        self.points_3d, self.points_2d = dev(points_3d, 3), dev(points_2d, 2)
+        self._staging = s = model.ctx.staging()  # the correspondences staged from host arrays, until free()
+        self.points_3d, self.points_2d = s.points(points_3d, 3), s.points(points_2d, 2)
         if len(self.points_3d) != len(self.points_2d):
+            s.close()
             raise InvalidParams("Number of 2D and 3D points must match")  # assert_eq! in the factor's new()
         self.residual_kind = CANONICAL_RESIDUAL[model.MODEL_ID] if residual_kind is None else residual_kind
         self.bounds = CONVERTER_BOUNDS.get(model.MODEL_ID)
@@ -132,9 +125,7 @@ class OptimizationCost:
         return self.model.get_distortion()
 
     def free(self):
-        for p in self._own:
-            p.free()
-        self._own = []
+        self._staging.close()
 
 
 class DoubleSphereOptimizationCost(OptimizationCost):

@@ -74,6 +74,10 @@ class Context:
     def device_free(self, ptr: int):
         self.check(_lib.acm_device_free(self._h, C.c_void_p(ptr)))
 
+    def staging(self) -> "Staging":
+        """Owner of one call's device temporaries, freed when its `with` block ends."""
+        return Staging(self)
+
     def pinned_empty(self, shape, dtype) -> np.ndarray:
         """numpy array backed by page-locked host memory owned by this context."""
         dtype = np.dtype(dtype)
@@ -193,3 +197,60 @@ class Points:
                 self.free()
         except Exception:
             pass
+
+
+class Staging:
+    """The device temporaries of one call: raw buffers and `Points`.  Everything it owns is freed when its `with` block
+    ends, whether the block returns or raises; `keep` hands objects to the caller instead."""
+
+    def __init__(self, ctx: Context):
+        self.ctx = ctx
+        self._owned = []
+
+    def alloc(self, nbytes: int) -> int:
+        """A device buffer of max(nbytes, 1) bytes."""
+        return self.own(self.ctx.device_alloc(max(nbytes, 1)))
+
+    def points(self, a, dim: int, dtype: int = N.F64) -> Points:
+        """`a` itself if it is `Points` (not owned), else `a` as (-1, dim) float64 uploaded to new owned `Points`."""
+        if isinstance(a, Points):
+            return a
+        a = np.ascontiguousarray(a, dtype=np.float64).reshape(-1, dim)
+        p = self.own(Points(self.ctx, dim, a.shape[0], dtype))
+        p.upload(a)
+        return p
+
+    def own(self, obj):
+        self._owned.append(obj)
+        return obj
+
+    def keep(self, *objs):
+        """Releases `objs` to the caller and returns them."""
+        for o in objs:
+            self._owned.remove(o)
+        return objs
+
+    def close(self):
+        """Frees everything owned, going on past a failed free; raises the first failure at the end."""
+        owned, self._owned = self._owned, []
+        err = None
+        for o in owned:
+            try:
+                if isinstance(o, Points):
+                    o.free()
+                else:
+                    self.ctx.device_free(o)
+            except Exception as e:
+                err = err or e
+        if err is not None:
+            raise err
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, exc_type, exc, tb):
+        try:
+            self.close()
+        except Exception:
+            if exc_type is None:
+                raise

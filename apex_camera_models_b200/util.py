@@ -67,15 +67,13 @@ def _check_frames(frames: np.ndarray, camera_model: CameraModel) -> np.ndarray:
 
 def _download_map(ctx, res, call) -> np.ndarray:
     """(H, W, 2) source-coordinate map at resolution `res`: `call(device_ptr)` writes it on the device and returns libacm's
-    status; the device buffer is freed whatever happens."""
-    d = ctx.device_alloc(max(res.width * res.height, 1) * 16)
-    try:
+    status."""
+    with ctx.staging() as s:
+        d = s.alloc(res.width * res.height * 16)
         ctx.check(call(C.c_void_p(d)))
         out = np.empty((res.height, res.width, 2))
         ctx.d2h(out, d)
         ctx.sync()
-    finally:
-        ctx.device_free(d)
     return out
 
 
@@ -270,33 +268,20 @@ def sample_points(camera_model: CameraModel, n: int, device: bool = False, shard
     uv_h, xyz_h, kept = C.c_void_p(), C.c_void_p(), C.c_size_t()
     rank, world = shard if shard is not None else (0, 1)
     ctx.check(_lib.acm_sample_points_shard(ctx.handle, C.byref(cam), n, rank, world, C.byref(uv_h), C.byref(xyz_h), C.byref(kept)))
-    uv = Points(ctx, 2, kept.value, _handle=uv_h)
-    xyz = Points(ctx, 3, kept.value, _handle=xyz_h)
-    if device:
-        return uv, xyz
-    a, b = uv.numpy(), xyz.numpy()
-    uv.free(); xyz.free()
-    return a, b
+    with ctx.staging() as s:
+        uv, xyz = s.own(Points(ctx, 2, kept.value, _handle=uv_h)), s.own(Points(ctx, 3, kept.value, _handle=xyz_h))
+        return s.keep(uv, xyz) if device else (uv.numpy(), xyz.numpy())
 
 
 def compute_reprojection_error(camera_model: CameraModel, points3d, points2d) -> ProjectionError:
     if camera_model is None:
         raise UtilError("Camera model does not exist")
     ctx = camera_model.ctx
-    own = []
-    def dev(a, dim):
-        if isinstance(a, Points):
-            return a
-        p = Points.from_numpy(ctx, np.ascontiguousarray(a, dtype=np.float64).reshape(-1, dim))
-        own.append(p)
-        return p
-    X, UV = dev(points3d, 3), dev(points2d, 2)
     cam = camera_model.camera_block()
     out = N.ProjectionError()
-    rc = _lib.acm_reprojection_error(ctx.handle, C.byref(cam), X.handle, UV.handle, C.byref(out))
-    for p in own:
-        p.free()
-    ctx.check(rc)
+    with ctx.staging() as s:
+        X, UV = s.points(points3d, 3), s.points(points2d, 2)
+        ctx.check(_lib.acm_reprojection_error(ctx.handle, C.byref(cam), X.handle, UV.handle, C.byref(out)))
     return ProjectionError(out.rmse, out.min, out.max, out.mean, out.stddev, out.median, int(out.count))
 
 
@@ -341,33 +326,18 @@ def triangulate_points(first: CameraModel, second: CameraModel, R, t, points1, p
     Rm, tv = _rotation_array(R), _translation_array(t)
     ca, cb = first.camera_block(), second.camera_block()
     if isinstance(points1, Points) or isinstance(points2, Points):
-        own = []
-
-        def dev(a):
-            if isinstance(a, Points):
-                return a
-            p = Points.from_numpy(ctx, np.ascontiguousarray(a, dtype=np.float64).reshape(-1, 2))
-            own.append(p)
-            return p
-        try:
-            a, b = dev(points1), dev(points2)
+        with ctx.staging() as s:
+            a, b = s.points(points1, 2), s.points(points2, 2)
             n = len(a)
-            xyz = Points(ctx, 3, n)
-            own.append(xyz)
-            d = ctx.device_alloc(max(n, 1) * 17)  # two rows of errors, then the status bytes
-            try:
-                ctx.check(_lib.acm_triangulate(ctx.handle, C.byref(ca), C.byref(cb), Rm, tv, a.handle, b.handle, int(max_iterations),
-                                               xyz.handle, C.c_void_p(d), C.c_void_p(d + 16 * n)))
-                err, st = np.empty((2, n)), np.empty(n, np.uint8)
-                if n:
-                    ctx.d2h(err, d); ctx.d2h(st, d + 16 * n)
-                ctx.sync()
-                pts = xyz.numpy()
-            finally:
-                ctx.device_free(d)
-        finally:
-            for p in own:
-                p.free()
+            xyz = s.own(Points(ctx, 3, n))
+            d = s.alloc(n * 17)  # two rows of errors, then the status bytes
+            ctx.check(_lib.acm_triangulate(ctx.handle, C.byref(ca), C.byref(cb), Rm, tv, a.handle, b.handle, int(max_iterations),
+                                           xyz.handle, C.c_void_p(d), C.c_void_p(d + 16 * n)))
+            err, st = np.empty((2, n)), np.empty(n, np.uint8)
+            if n:
+                ctx.d2h(err, d); ctx.d2h(st, d + 16 * n)
+            ctx.sync()
+            pts = xyz.numpy()
         return pts, np.ascontiguousarray(err.T), st
     uv1 = np.ascontiguousarray(points1, dtype=np.float64).reshape(-1, 2)
     uv2 = np.ascontiguousarray(points2, dtype=np.float64).reshape(-1, 2)
@@ -413,13 +383,11 @@ def render_depth(model: CameraModel, points, R=None, t=None):
     rng, idx = np.empty((res.height, res.width), np.float32), np.empty((res.height, res.width), np.uint32)
     if isinstance(points, Points):
         npix = res.width * res.height
-        d = ctx.device_alloc(max(npix, 1) * 8)  # range row, then index row
-        try:
+        with ctx.staging() as s:
+            d = s.alloc(npix * 8)  # range row, then index row
             ctx.check(_lib.acm_render_depth(ctx.handle, C.byref(cam), Rm, tv, points.handle, C.c_void_p(d), C.c_void_p(d + 4 * npix)))
             ctx.d2h(rng, d); ctx.d2h(idx, d + 4 * npix)
             ctx.sync()
-        finally:
-            ctx.device_free(d)
         return rng, idx
     xyz = np.ascontiguousarray(points, dtype=np.float64).reshape(-1, 3)
     ctx.check(_lib.acm_render_depth_host(ctx.handle, C.byref(cam), Rm, tv, xyz.ctypes.data_as(C.c_void_p), len(xyz),
@@ -443,16 +411,13 @@ def depth_to_points(model: CameraModel, range_image, R=None, t=None):
     if r.shape != (res.height, res.width):
         raise UtilError(f"Invalid parameters: range image {r.shape} doesn't match model {res.height}x{res.width} (H, W)")
     npix = res.width * res.height
-    xyz = Points(ctx, 3, npix)
-    d = ctx.device_alloc(max(npix, 1) * 5)  # range, then the status bytes
-    try:
+    with ctx.staging() as s:
+        xyz = s.own(Points(ctx, 3, npix))
+        d = s.alloc(npix * 5)  # range, then the status bytes
         ctx.h2d(d, r)
         ctx.check(_lib.acm_depth_to_points(ctx.handle, C.byref(cam), Rm, tv, C.c_void_p(d), xyz.handle, C.c_void_p(d + 4 * npix)))
         st = np.empty((res.height, res.width), np.uint8)
         ctx.d2h(st, d + 4 * npix)
         ctx.sync()
         pts = xyz.numpy().reshape(res.height, res.width, 3)
-    finally:
-        ctx.device_free(d)
-        xyz.free()
     return pts, st

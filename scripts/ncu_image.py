@@ -7,7 +7,8 @@ from apex_camera_models_b200.image_quality import _DeviceImage, _lib
 ctx = acm.Context(0)
 rng = np.random.default_rng(1)
 a = rng.integers(0, 256, (4096, 4096, 3), dtype=np.uint8); b = rng.integers(0, 256, (4096, 4096, 3), dtype=np.uint8)
-da, db = _DeviceImage(ctx, a), _DeviceImage(ctx, b)
+s = ctx.staging()
+da, db = _DeviceImage(s, a), _DeviceImage(s, b)
 out = C.c_double()
 for _ in range(2):
     ctx.check(_lib.acm_image_psnr(ctx.handle, C.c_void_p(da.ptr), C.c_void_p(db.ptr), 4096, 4096, C.byref(out)))

@@ -37,7 +37,8 @@ rng = np.random.default_rng(1)
 a = rng.integers(0, 256, (4096, 4096, 3), dtype=np.uint8); b = rng.integers(0, 256, (4096, 4096, 3), dtype=np.uint8)
 from apex_camera_models_b200.image_quality import _DeviceImage, _lib
 import ctypes as C
-da, db = _DeviceImage(ctx, a), _DeviceImage(ctx, b)
+s = ctx.staging()
+da, db = _DeviceImage(s, a), _DeviceImage(s, b)
 out = C.c_double()
 ms_p, _ = timed(lambda: ctx.check(_lib.acm_image_psnr(ctx.handle, C.c_void_p(da.ptr), C.c_void_p(db.ptr), 4096, 4096, C.byref(out))), reps=10)
 ms_s, _ = timed(lambda: ctx.check(_lib.acm_image_ssim(ctx.handle, C.c_void_p(da.ptr), C.c_void_p(db.ptr), 4096, 4096, C.byref(out))), reps=10)

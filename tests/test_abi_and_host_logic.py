@@ -306,3 +306,39 @@ def test_export_point_correspondences_format(tmp_path):
     assert rust.endswith("    Vector2::new(300.000000000000000, 400.125000000000000)\n]);\n")
     with pytest.raises(UtilError):
         export_point_correspondences(p3, p2[:1], "bad", str(tmp_path))
+
+
+def test_staging_frees_everything_and_keeps_the_body_error():
+    """Staging.close() tries every free even when one fails; an error of the `with` body wins over a failed free, a failed
+    free is raised when the body succeeded, and `keep` takes objects out of the staging.  A stand-in context, no device."""
+    from apex_camera_models_b200.runtime import Staging
+
+    class Ctx:
+        def __init__(self):
+            self.sizes, self.freed, self.bad = [], [], None
+
+        def device_alloc(self, nbytes):
+            self.sizes.append(nbytes)
+            return 0x1000 * len(self.sizes)
+
+        def device_free(self, ptr):
+            self.freed.append(ptr)
+            if ptr == self.bad:
+                raise acm.AcmError("free failed")
+
+    ctx = Ctx()
+    with pytest.raises(acm.AcmError, match="free failed"):
+        with Staging(ctx) as s:
+            a, b, c = s.alloc(0), s.alloc(8), s.alloc(3)
+            ctx.bad = a
+            assert s.keep(c) == (c,)
+    assert ctx.sizes == [1, 8, 3] and ctx.freed == [a, b]
+    ctx.freed = []
+    with pytest.raises(ValueError, match="body"):
+        with Staging(ctx) as s:
+            ctx.bad = s.alloc(1)
+            d = s.alloc(1)
+            raise ValueError("body")
+    assert ctx.freed == [ctx.bad, d]
+    s.close()  # a closed staging owns nothing
+    assert ctx.freed == [ctx.bad, d]
